@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- selective-scan fwd+bwd throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -13,8 +13,13 @@ target are quoted on.  Weak scaling: every rank processes its own batch (batch s
 collective); for N > 1 the A_log/D/dt_bias gradients are all-reduced over NCCL each step, as in training.
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the definition of every field.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what its last timed step returned -- out and the gradients of
+every input and parameter (under N GPUs the all-reduced sums the step receives) -- as DIR/<name>.npy in float32.  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -95,6 +100,35 @@ def measured_traffic(workload, kernel, B):
         return None, "kernel not in the capture"
 
 
+OUTPUT_NAMES = ("out", "du", "ddelta", "dz", "dB", "dC", "dA_log", "dD", "ddt_bias")
+DUMP_SAMPLE = 1 << 20   # elements kept of a larger output: nine float32 arrays of at most 4 MiB each, under 64 MB in all
+
+
+def step_outputs(out, grads, flat, by_channels):
+    """{name: tensor} of what one step hands its caller.  Under N GPUs the all-reduced sums in `flat` stand for the rank's
+    own dB, dC (channel sharding) or parameter gradients (batch sharding)."""
+    grads = list(grads)
+    if flat is not None:
+        i = slice(3, 5) if by_channels else slice(5, None)
+        grads[i] = [p.view_as(g) for p, g in zip(flat.split([g.numel() for g in grads[i]]), grads[i])]
+    return dict(zip(OUTPUT_NAMES, [out] + grads))
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as path/<name>.npy in float32.  An array of more than DUMP_SAMPLE elements is reduced to its
+    elements at DUMP_SAMPLE distinct flat indices drawn by numpy.random.default_rng(0), in increasing order: the same
+    indices in every run of the same shape."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach()
+        if a.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.numel(), DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(path, name + ".npy"), a.float().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------ clocks
 class ClockSampler:
     Q = ("clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,"
@@ -108,6 +142,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", f"--id={self.index}", f"--query-gpu={self.Q}",
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)   # the sampler never outlives the benchmark, even one that fails before stop()
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -263,7 +298,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true", help="do not bind the process to the GPU's NUMA node for the e2e leg")
     ap.add_argument("--cpu-budget-s", type=float, default=25.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32; seeded sample of a large output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -337,13 +378,21 @@ def main():
         d = sets[i % nsets]
         out = selective_scan_fn(d["u"], d["delta"], A_log, d["Bm"], d["Cm"], D, z=d["z"], dt_bias=bias)
         grads = torch.autograd.grad(out, (d["u"], d["delta"], d["z"], d["Bm"], d["Cm"], A_log, D, bias), d["dout"])
+        flat = None
         if by_channels:   # channel sharding: dB, dC sum over every rank's channels (2 B L N values); parameters are local
             flat = torch.cat([grads[3].reshape(-1), grads[4].reshape(-1)]).float()
             dist.all_reduce(flat)
         elif world > 1:   # data-parallel training: all-reduce the (tiny) parameter gradients
             flat = torch.cat([g.reshape(-1) for g in grads[5:]])
             dist.all_reduce(flat)
-        return out, grads
+        return out, grads, flat
+
+    last = []   # what the last timed step returned; earlier steps' results are released at once, as in the warm-up
+
+    def timed_step(i):
+        r = step(i)
+        if i == args.steps - 1:
+            last.append(r)
 
     def sync_all():
         if world > 1:
@@ -368,7 +417,7 @@ def main():
     if flush is None:
         e0.record()
         for i in range(args.steps):
-            step(i)
+            timed_step(i)
         e1.record()
         sync_all()
         elapsed_ms = e0.elapsed_time(e1)
@@ -378,7 +427,7 @@ def main():
             flush.fill_(i & 0xFF)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            step(i)
+            timed_step(i)
             b.record()
             torch.cuda.synchronize(dev)
             elapsed_ms += a.elapsed_time(b)
@@ -431,6 +480,10 @@ def main():
                 "step_frac": round((fwd_b + bwd_b) / (ms_per_step * 1e-3) / 1e9 / peak, 4),
                 "note": "selective scan at N=16 is bound by MUFU + FP32 operand delivery on B200, not by HBM (DESIGN.md section 4)"}
     gpu_launches = int(sum(v[1] for v in kern.values()))
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, step_outputs(*last[0], by_channels))
+    last.clear()
 
     # ---- e2e: the same step through the public host-buffer API (gfe_mamba_b200.host_pipeline.HostScanPipeline): pinned HOST
     #      inputs -> H2D, fused fwd+bwd, D2H of out and every activation gradient into pinned HOST outputs, all inside the
@@ -492,4 +545,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True   # the benchmark leaves the tree as the build left it (it may be read-only)
     main()

@@ -1,7 +1,7 @@
 """Generate the golden fixtures under tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference, which does not exist on the
-GPU box):   python tests/golden/make_golden.py
+Needs a checkout of the original GFE-Mamba:
+            GFE_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 The fixtures pin the oracle (tests/test_oracle_golden.py, CPU) and are compared
 with the CUDA path directly (tests/test_gpu_parity.py, GPU).  What is recorded:
@@ -12,7 +12,9 @@ with the CUDA path directly (tests/test_gpu_parity.py, GPU).  What is recorded:
                       autograd gradients, L = 37 (pads to 64) and L = 64
   block_small.npz     one MambaBlock: state dict, forward, gradients of every parameter and of
                       the input, and step() replayed over the same sequence (mamba.py:197-225,342-405)
-  mamba_cfg1.npz      BASELINE config 1: Mamba(d_model=128, n_layers=2), B=8, L=64, fp32
+  mamba_cfg1.npz      BASELINE config 1: Mamba(d_model=128, n_layers=2), B=8, L=64, fp32; the seeded tensors
+                      (state dict, x, dy) as shape + every SAMPLE_STRIDE-th value, redrawn from the seed by
+                      the mamba_cfg1 fixture (tests/conftest.py): whole, the file would be over 1 MB
   block_ln.npz        the same as block_small for jamba's configuration, inner_layernorms=True (mamba.py:169-176,188-195)
   block_odd.npz       the same for d_state=8, d_conv=5: shapes outside the fused kernels (pscan composition, cuDNN conv)
 """
@@ -22,11 +24,14 @@ import sys
 import numpy as np
 import torch
 
-REF = os.environ.get("GFE_REFERENCE", "/root/reference")
+REF = os.environ.get("GFE_REFERENCE", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
+CFG1_SEED, SAMPLE_STRIDE = 404, 17   # a prime stride: samples do not line up with the rows of any parameter
 
 
 def _load_reference():
+    if not REF or not os.path.isdir(os.path.join(REF, "cross_atten")):
+        raise SystemExit("set GFE_REFERENCE to a checkout of the original GFE-Mamba")
     # make sure it is the reference's cross_atten that gets imported, not this repo's drop-in
     sys.path[:] = [p for p in sys.path if os.path.abspath(p or ".") != os.path.abspath(os.path.join(HERE, "..", ".."))]
     sys.path.insert(0, REF)
@@ -111,7 +116,7 @@ def gen_block(ref_mamba, out, seed=303, d_model=16, B=2, L=19, **cfg_kw):
 
 
 def gen_cfg1(ref_mamba, out):
-    torch.manual_seed(404)
+    torch.manual_seed(CFG1_SEED)
     cfg = ref_mamba.MambaConfig(d_model=128, n_layers=2)                 # BASELINE.json configs[0]
     model = ref_mamba.Mamba(cfg)
     B, L = 8, 64
@@ -127,6 +132,17 @@ def gen_cfg1(ref_mamba, out):
     for k, v in model.named_parameters():
         if k.startswith("layers.0.") and any(s in k for s in ("A_log", ".D", "dt_proj", "conv1d", "norm")):
             out[f"grad.{k}"] = np32(v.grad)
+    sample_seeded(out)
+
+
+def sample_seeded(out):
+    """Replaces the tensors drawn from CFG1_SEED (state dict, x, dy) by their shapes and every SAMPLE_STRIDE-th value."""
+    for k in [k for k in out if k.startswith("sd.") or k in ("x", "dy")]:
+        v = out.pop(k)
+        out[f"shape.{k}"] = np.array(v.shape, np.int64)
+        out[f"sample.{k}"] = np.ascontiguousarray(v.reshape(-1)[::SAMPLE_STRIDE])
+    out["seed"] = np.array(CFG1_SEED, np.int64)
+    out["sample_stride"] = np.array(SAMPLE_STRIDE, np.int64)
 
 
 def gen_block_ln(ref_mamba, out):

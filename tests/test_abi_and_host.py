@@ -150,9 +150,9 @@ def test_state_dict_keys_and_seeded_init_match_reference(golden_dir):
     assert blk.A_log._no_weight_decay and blk.D._no_weight_decay
 
 
-def test_mamba_state_dict_layout(golden_dir):
+def test_mamba_state_dict_layout(mamba_cfg1):
     from cross_atten.mamba import Mamba, MambaConfig
-    g = dict(np.load(os.path.join(golden_dir, "mamba_cfg1.npz")))
+    g = mamba_cfg1
     m = Mamba(MambaConfig(d_model=128, n_layers=2, inner_layernorms=False))
     want = {k[3:]: v.shape for k, v in g.items() if k.startswith("sd.")}
     assert {k: tuple(v.shape) for k, v in m.state_dict().items()} == want
@@ -251,6 +251,35 @@ def test_bench_helpers():
             assert bench.measured_traffic("cfgX", "selscan_bwd", 4) == (123, "t")
         finally:
             bench.ROOT = real_root
+
+
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs: float32 files named after the step's outputs, whole when small, the same seeded sample of a large
+    output in every run, and the all-reduced sums in place of a rank's own gradients under N GPUs."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    big = torch.arange(bench.DUMP_SAMPLE + 999, dtype=torch.float32)
+    grads = [torch.ones(2, 3, dtype=torch.bfloat16) * i for i in range(8)]
+    flat = torch.arange(2 * 3 * 3, dtype=torch.float32)
+    arrays = bench.step_outputs(big, grads, flat, by_channels=False)
+    assert list(arrays) == list(bench.OUTPUT_NAMES)
+    assert torch.equal(arrays["dA_log"], flat[:6].view(2, 3)) and torch.equal(arrays["ddt_bias"], flat[12:].view(2, 3))
+    assert torch.equal(arrays["dB"], grads[3])
+    chan = bench.step_outputs(big, grads, flat[:12], by_channels=True)
+    assert torch.equal(chan["dC"], flat[6:12].view(2, 3)) and torch.equal(chan["dD"], grads[6])
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    total = 0
+    for name in bench.OUTPUT_NAMES:
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype == np.float32 and np.array_equal(a, b), name
+        total += a.nbytes
+    out = np.load(tmp_path / "a" / "out.npy")
+    assert out.shape == (bench.DUMP_SAMPLE,) and np.all(np.diff(out) > 0)   # sorted distinct indices of a ramp
+    assert np.array_equal(np.load(tmp_path / "a" / "dz.npy"), grads[2].float().numpy())
+    assert 9 * bench.DUMP_SAMPLE * 4 <= 64e6 and total <= 64e6
 
 
 def test_numa_binding_is_a_no_op_without_topology():

@@ -385,10 +385,10 @@ def test_block_golden_step(golden_dir):
     assert relerr(cache[0], g["h_last"]) < 1e-4 and relerr(cache[1], g["inputs_last"]) < 1e-5
 
 
-def test_mamba_cfg1_golden(golden_dir):
+def test_mamba_cfg1_golden(mamba_cfg1):
     """BASELINE config 1: Mamba(d_model=128, n_layers=2), B=8, L=64, fp32, forward + backward."""
     from cross_atten.mamba import Mamba, MambaConfig
-    g = _load(golden_dir, "mamba_cfg1")
+    g = mamba_cfg1
     d_model, n_layers = int(g["meta"][0]), int(g["meta"][1])
     model = Mamba(MambaConfig(d_model=d_model, n_layers=n_layers))
     model.load_state_dict({k[3:]: torch.from_numpy(v) for k, v in g.items() if k.startswith("sd.")}, strict=True)

@@ -144,9 +144,9 @@ def test_ssm_step(golden_dir):
     assert relerr(inputs, g["inputs_last"]) < 1e-6
 
 
-def test_mamba_cfg1_forward(golden_dir):
+def test_mamba_cfg1_forward(mamba_cfg1):
     """BASELINE config 1 end to end (2 layers, RMSNorm + residual)."""
-    g = _load(golden_dir, "mamba_cfg1")
+    g = mamba_cfg1
     d_model, n_layers, d_state, _, _, dt_rank, _, _ = (int(v) for v in g["meta"])
     sd = {k[3:]: v for k, v in g.items() if k.startswith("sd.")}
     y = orc.mamba_forward(sd, g["x"], n_layers, d_state, dt_rank)

@@ -1,5 +1,6 @@
-"""The reference's own callers of the path, built on the drop-in (CPU, build container only -- /root/reference does not
-exist on the GPU box): cross_atten/mamba_transformer.py:65-66 (Cross_mamba_both -> Mamba(MambaConfig(use_cuda=True))) and
+"""The reference's own callers of the path, built on the drop-in (CPU; needs GFE_REFERENCE, a checkout of the original
+GFE-Mamba, whose caller modules are not part of this repository): cross_atten/mamba_transformer.py:65-66
+(Cross_mamba_both -> Mamba(MambaConfig(use_cuda=True))) and
 cross_atten/jamba.py:9,406 (MambaLayer -> MambaBlock(inner_layernorms=True), RMSNorm).  With this repository ahead of the
 reference on sys.path, `cross_atten.mamba` / `cross_atten.pscan` resolve here and every other module of the namespace
 package to the reference; the models must come out with the same parameter names and shapes as on the reference alone
@@ -8,11 +9,12 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.environ.get("GFE_REFERENCE", "/root/reference")
+REF = os.environ.get("GFE_REFERENCE", "")
 
 PROBE = r"""
 import json, sys
@@ -36,13 +38,15 @@ print("PROBE" + json.dumps(out))
 
 def _probe(pythonpath):
     env = dict(os.environ, PYTHONPATH=os.pathsep.join(pythonpath))
-    r = subprocess.run([sys.executable, "-c", PROBE], capture_output=True, text=True, cwd="/tmp", env=env, timeout=600)
+    r = subprocess.run([sys.executable, "-c", PROBE], capture_output=True, text=True, cwd=tempfile.gettempdir(), env=env,
+                       timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     line = next(l for l in r.stdout.splitlines() if l.startswith("PROBE"))
     return json.loads(line[5:])
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "cross_atten")), reason="reference checkout not present")
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "cross_atten")),
+                    reason="GFE_REFERENCE does not name a checkout of the original GFE-Mamba")
 def test_reference_callers_build_on_the_drop_in():
     ours = _probe([ROOT, REF])
     ref = _probe([REF])
