@@ -34,7 +34,7 @@ static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; 
 constexpr int kNState = 16;     // d_state the fused kernels are compiled for
 constexpr int kChunk = 16;      // time steps per register chunk == checkpoint interval
 constexpr int kMaxSeg = 256;    // max L-split factor (one long sequence sharded over 8 GPUs: 128 channels, 256 segments of 256 steps)
-constexpr int kCkptV2 = 8;      // checkpoint interval of the chained (v2) kernels: halves the register-resident history of backward
+constexpr int kCkptV2 = 8;      // checkpoint interval of the chained kernels: halves the register-resident history of backward
 
 // How one (b, channel) sequence is split along L when B*ED alone cannot fill the GPU.
 struct SegPlan {
@@ -50,11 +50,6 @@ SegPlan plan_segments(int B, int L, int ED);
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
 
-template <typename T> struct DType;
-template <> struct DType<float> { static constexpr int id = GFE_F32; };
-template <> struct DType<__nv_bfloat16> { static constexpr int id = GFE_BF16; };
-template <> struct DType<__half> { static constexpr int id = GFE_F16; };
-
 __device__ __forceinline__ float to_f(float v) { return v; }
 __device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
 __device__ __forceinline__ float to_f(__half v) { return __half2float(v); }
@@ -63,8 +58,6 @@ template <typename T> __device__ __forceinline__ T from_f(float v);
 template <> __device__ __forceinline__ float from_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 from_f<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 template <> __device__ __forceinline__ __half from_f<__half>(float v) { return __float2half_rn(v); }
-
-template <typename T> __device__ __forceinline__ T zero_of() { return from_f<T>(0.0f); }
 
 // streaming (read-once) global load / store: do not pollute L1
 template <typename T> __device__ __forceinline__ T ld_stream(const T *p) { return __ldcs(p); }

@@ -14,13 +14,8 @@
 
 namespace gfe {
 
-#ifndef GFE_CONV_TILE
-#define GFE_CONV_TILE 128
-#endif
-#ifndef GFE_CONV_PREFETCH
-#define GFE_CONV_PREFETCH 1   // the next group's rows are requested before the current group is computed
-#endif
-constexpr int kConvTile = GFE_CONV_TILE;  // time steps per thread (one partial dw|dbias row per tile)
+// time steps per thread (one partial dw|dbias row per tile); 64 and 256 measured, no gain (profiles/r02_chain_variants.txt)
+constexpr int kConvTile = 128;
 
 struct ConvParams {
     const void *xin, *du;
@@ -71,20 +66,21 @@ __global__ void __launch_bounds__(128) conv1d_silu_fwd_kernel(ConvParams p) {
         for (int i = 0; i < V; ++i) win[i][k + 1] = t >= 0 ? xv.get(i) : 0.f;
     }
     constexpr int U = 8;
-    ChanVec<T, V> xn[U];   // rows of the next group, in flight while the current group is computed
+    // rows of the next group, in flight while the current group is computed (measured on both directions: fp32 backward 14 %
+    // faster, 16-bit 3-4 % slower; profiles/r02_chain_variants.txt)
+    ChanVec<T, V> xn[U];
 #pragma unroll
     for (int j = 0; j < U; ++j) xn[j] = ChanVec<T, V>::load(x + (int64_t)min(t0 + j, t1 - 1) * p.x_rs);
     for (int tb = t0; tb < t1; tb += U) {
         ChanVec<T, V> xr[U];
 #pragma unroll
         for (int j = 0; j < U; ++j) xr[j] = xn[j];
-        if (GFE_CONV_PREFETCH && tb + U < t1) {
+        if (tb + U < t1) {
 #pragma unroll
             for (int j = 0; j < U; ++j) xn[j] = ChanVec<T, V>::load(x + (int64_t)min(tb + U + j, t1 - 1) * p.x_rs);
         }
 #pragma unroll
         for (int j = 0; j < U; ++j) {
-            if (!GFE_CONV_PREFETCH && tb > t0) xr[j] = ChanVec<T, V>::load(x + (int64_t)min(tb + j, t1 - 1) * p.x_rs);
             if (tb + j < t1) {
                 ChanVec<T, V> o;
 #pragma unroll
@@ -148,7 +144,7 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_kernel(ConvParams p) {
         ChanVec<T, V> xr[U], gr[U];
 #pragma unroll
         for (int j = 0; j < U; ++j) { xr[j] = xn[j]; gr[j] = gn[j]; }
-        if (GFE_CONV_PREFETCH && tb + U < tend) {
+        if (tb + U < tend) {
 #pragma unroll
             for (int j = 0; j < U; ++j) {
                 const int t = min(tb + U + j, p.L - 1);
@@ -159,10 +155,6 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_kernel(ConvParams p) {
 #pragma unroll
         for (int j = 0; j < U; ++j) {
             const int t = tb + j;
-            if (!GFE_CONV_PREFETCH && tb > t0) {
-                xr[j] = ChanVec<T, V>::load(x + (int64_t)min(t, p.L - 1) * p.x_rs);
-                gr[j] = ChanVec<T, V>::load(du + (int64_t)min(t, p.L - 1) * p.du_rs);
-            }
             if (t < tend) {
                 const int s_out = t - (K - 1);   // dxin[s] = sum_k w[k] dv[s + K-1 - k]
                 ChanVec<T, V> o;
@@ -471,17 +463,10 @@ static int conv_bwd_launch(ConvParams &p, cudaStream_t st) {
     const int v = conv_vec<T>(p, true);
     const dim3 block(128), grid((p.ED / v + 127) / 128, p.ntiles, p.B);
     { ScopedKernelTimer tm(K_CONV_BWD, st);
-#ifndef GFE_CONV_BWD_NP16
-#define GFE_CONV_BWD_NP16 1   // channel pairs per lane of the 16-bit backward (1: 4-byte accesses, 94 registers, +5 %; 2: 8-byte accesses, 166 registers)
-#endif
-      if (v == V) {
-          if constexpr (sizeof(T) == 2 && GFE_CONV_BWD_NP16 == 1) {
-              const dim3 grid1((p.ED / 2 + 127) / 128, p.ntiles, p.B);
-              conv1d_silu_bwd_pk_kernel<T, K, 1><<<grid1, block, 0, st>>>(p);
-          } else {
-              conv1d_silu_bwd_pk_kernel<T, K, V / 2><<<grid, block, 0, st>>>(p);
-          }
-      } else conv1d_silu_bwd_kernel<T, K, 1><<<grid, block, 0, st>>>(p); }
+      // packed backward: one channel pair per lane for every dtype (16-bit: 4-byte accesses, 94 registers, 5 % faster than
+      // two pairs with 8-byte accesses and 166 registers)
+      if (v == V) conv1d_silu_bwd_pk_kernel<T, K, 1><<<dim3((p.ED / 2 + 127) / 128, p.ntiles, p.B), block, 0, st>>>(p);
+      else conv1d_silu_bwd_kernel<T, K, 1><<<grid, block, 0, st>>>(p); }
     int rc = check_launch("conv1d_silu_bwd");
     if (rc != GFE_OK) return rc;
     { ScopedKernelTimer tm(K_CONV_BWD_FIN, st);

@@ -13,9 +13,6 @@
 // paying a second pass.  Only when even
 // that cannot fill the GPU (B*D*N below ~25 k elements, e.g. one long sequence with few channels) is L split into segments:
 // pass 1 reduces each segment to its (product of A, local end state) pair, pass 2 starts each segment from the combined carry.
-#include <stdio.h>
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace gfe {
@@ -31,10 +28,7 @@ struct PscanPlan {
 // fewer steps, so it keeps the wider vectors longer (measured at B=8, L=1024, D=1024: (4, 8) 98 % of the HBM peak, (2, 16) 88 %).
 static PscanPlan pscan_plan(int B, int L, int64_t DN, int nloads) {
     PscanPlan p;
-    double target = 12e6 * sm_count() / 148.0;                  // bytes in flight that saturate HBM (Little: ~6.5 TB/s x ~1.5 us)
-#ifdef GFE_EXPERIMENTS
-    if (const char *e = getenv("GFE_PSCAN_TARGET_MB")) target = atof(e) * 1e6;   // A/B measurements only
-#endif
+    const double target = 12e6 * sm_count() / 148.0;            // bytes in flight that saturate HBM (Little: ~6.5 TB/s x ~1.5 us)
     const double per_u = (double)B * (double)DN * 4.0 * nloads;  // bytes requested per unrolled step
     if (nloads == 2) {   // forward: (4, 16) when that alone fills the pipe, else the narrowest vectors and the deepest unroll
         p.V = 4; p.U = 16;
@@ -44,9 +38,6 @@ static PscanPlan pscan_plan(int B, int L, int64_t DN, int nloads) {
         if (DN % 4 != 0 || per_u * 8 < target) { p.V = 2; p.U = 16; }
         if (DN % 2 != 0 || per_u * 16 < target) { p.V = 1; p.U = 32; }
     }
-#ifdef GFE_EXPERIMENTS
-    if (const char *e = getenv("GFE_PSCAN_VU")) { int v = 0, u = 0; if (sscanf(e, "%d,%d", &v, &u) == 2 && nloads == 2) { p.V = v; p.U = u; } }
-#endif
     int S = 1;
     if (per_u * p.U * 2 < target) {   // still less than half of it: split L (re-reads A and X once more)
         S = (int)(target / (per_u * p.U));
@@ -353,17 +344,12 @@ __global__ void __launch_bounds__(32 * W) pscan_bwd_chain_kernel(PscanParams p) 
     }
 }
 
-#ifndef GFE_PSCAN_CHAIN
-#define GFE_PSCAN_CHAIN 1
-#endif
-#ifndef GFE_PSCAN_FW
-#define GFE_PSCAN_FW 8   // warps per CTA (batches in flight per column), forward
-#endif
-#ifndef GFE_PSCAN_BW
-#define GFE_PSCAN_BW 4   // backward
-#endif
+// warps per CTA of the warp-chained kernels (batches in flight per column): forward 8, backward 4 (4 / 8 / 16 forward against
+// 8 / 4 / 2 backward measured on three shapes, profiles/r02_chain_variants.txt)
+constexpr int kPsChainFW = 8;
+constexpr int kPsChainBW = 4;
 constexpr int kPsChainU = 8;
-static bool pscan_use_chain(int L, int nseg) { return GFE_PSCAN_CHAIN && nseg == 1 && L >= 4 * kPsChainU; }
+static bool pscan_use_chain(int L, int nseg) { return nseg == 1 && L >= 4 * kPsChainU; }
 
 static bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
@@ -418,8 +404,8 @@ GFE_API int gfe_pscan_fwd(const float *A, const float *X, float *H, int B, int L
         const int Vc = (al && DN % 4 == 0) ? 4 : 1;
         const dim3 gridc((unsigned)ceil_div64(DN / Vc, 32), 1, B);
         ScopedKernelTimer tm(K_PSCAN_FWD, st);
-        if (Vc == 4) pscan_fwd_chain_kernel<4, kPsChainU, GFE_PSCAN_FW><<<gridc, 32 * GFE_PSCAN_FW, 0, st>>>(p);
-        else pscan_fwd_chain_kernel<1, kPsChainU, GFE_PSCAN_FW><<<gridc, 32 * GFE_PSCAN_FW, 0, st>>>(p);
+        if (Vc == 4) pscan_fwd_chain_kernel<4, kPsChainU, kPsChainFW><<<gridc, 32 * kPsChainFW, 0, st>>>(p);
+        else pscan_fwd_chain_kernel<1, kPsChainU, kPsChainFW><<<gridc, 32 * kPsChainFW, 0, st>>>(p);
         return check_launch("pscan_fwd (chained)");
     }
     { ScopedKernelTimer tm(K_PSCAN_FWD, st);
@@ -462,8 +448,8 @@ GFE_API int gfe_pscan_bwd(const float *A, const float *H, const float *dH, float
         const int Vc = (al && DN % 4 == 0) ? 4 : 1;
         const dim3 gridc((unsigned)ceil_div64(DN / Vc, 32), 1, B);
         ScopedKernelTimer tm(K_PSCAN_BWD, st);
-        if (Vc == 4) pscan_bwd_chain_kernel<4, kPsChainU, GFE_PSCAN_BW><<<gridc, 32 * GFE_PSCAN_BW, 0, st>>>(p);
-        else pscan_bwd_chain_kernel<1, kPsChainU, GFE_PSCAN_BW><<<gridc, 32 * GFE_PSCAN_BW, 0, st>>>(p);
+        if (Vc == 4) pscan_bwd_chain_kernel<4, kPsChainU, kPsChainBW><<<gridc, 32 * kPsChainBW, 0, st>>>(p);
+        else pscan_bwd_chain_kernel<1, kPsChainU, kPsChainBW><<<gridc, 32 * kPsChainBW, 0, st>>>(p);
         return check_launch("pscan_bwd (chained)");
     }
     const dim3 grid((unsigned)ceil_div64(nvec, 128), pl.nseg, B);

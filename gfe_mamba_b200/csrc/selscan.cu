@@ -21,9 +21,6 @@
 // 64 values), per-warp partial rows in the workspace, one small finalize kernel.  Parameter gradients
 // (dA_log, dD, ddt_bias) are accumulated per lane over its whole segment, then reduced over (b, seg)
 // by the second finalize kernel.  Everything is deterministic (no atomics).
-#include <stdlib.h>
-#include <string.h>
-
 #include "common.cuh"
 #include "selscan_shared.cuh"
 
@@ -582,8 +579,7 @@ __global__ void __launch_bounds__(256) selscan_bwd_finalize_bc_kernel(ScanParams
     const int n = (int)(idx & 31);
     float acc = 0.f;
     const int64_t rbase = idx & ~(int64_t)31;
-    const float *src = p.part_bc + (p.bc_interleaved == 2 ? rbase + ((n >> 4) * 2 + (n & 1)) * 8 + ((n & 15) >> 1)   // v3: [dB even | dB odd | dC even | dC odd]
-                                    : p.bc_interleaved ? rbase + 2 * (n & 15) + (n >> 4) : idx);
+    const float *src = p.part_bc + (p.bc_interleaved ? rbase + 2 * (n & 15) + (n >> 4) : idx);
     for (int g = 0; g < p.G; ++g) acc += __ldcs(src + (size_t)g * rows * 32);
     const int64_t b = row / p.L, t = row % p.L;
     if (n < 16)
@@ -612,8 +608,6 @@ __global__ void __launch_bounds__(128) selscan_bwd_finalize_par_kernel(ScanParam
 // =====================================================================================================
 // Host side
 // =====================================================================================================
-
-static int warps_per_cta() { return 1; }
 
 struct WsLayout {
     size_t seg_h, seg_sd, part_bc, part_par, total;
@@ -707,17 +701,16 @@ static int launch_fwd(const gfe_selscan_args *a, cudaStream_t st) {
     p.seg_h = reinterpret_cast<float2 *>(ws + wl.seg_h);
     p.seg_sd = reinterpret_cast<float *>(ws + wl.seg_sd);
 
-    const int W = warps_per_cta();
-    const dim3 block(32 * W);
-    const dim3 grid((p.G + W - 1) / W, sp.nseg, a->batch);
+    const dim3 block(32);   // one warp per CTA
+    const dim3 grid(p.G, sp.nseg, a->batch);
     if (sp.nseg > 1) {
         { ScopedKernelTimer tm(K_SELSCAN_FWD_SUMMARY, st);
-          selscan_fwd_summary_kernel<T><<<grid, block, W * kChunk * 32 * sizeof(float), st>>>(p); }
+          selscan_fwd_summary_kernel<T><<<grid, block, kChunk * 32 * sizeof(float), st>>>(p); }
         int rc = check_launch("selscan_fwd_summary");
         if (rc != GFE_OK) return rc;
     }
     {
-        const size_t smem = (size_t)W * 2 * kChunk * 32 * sizeof(float);
+        const size_t smem = 2 * kChunk * 32 * sizeof(float);
         ScopedKernelTimer tm(K_SELSCAN_FWD, st);
         if (a->z != nullptr) selscan_fwd_kernel<T, true><<<grid, block, smem, st>>>(p);
         else selscan_fwd_kernel<T, false><<<grid, block, smem, st>>>(p);
@@ -730,18 +723,17 @@ static int launch_finalize_t(const gfe_selscan_args *a, ScanParams &p, cudaStrea
 
 template <typename T, bool HAS_Z>
 static int launch_bwd_z(const gfe_selscan_args *a, ScanParams &p, const SegPlan &sp, cudaStream_t st) {
-    const int W = warps_per_cta();
-    const dim3 block(32 * W);
+    const dim3 block(32);   // one warp per CTA
     if (sp.nseg > 1) {
-        const dim3 grid((p.G + W - 1) / W, sp.nseg - 1, a->batch);
+        const dim3 grid(p.G, sp.nseg - 1, a->batch);
         { ScopedKernelTimer tm(K_SELSCAN_BWD_SUMMARY, st);
-          selscan_bwd_summary_kernel<T, HAS_Z><<<grid, block, W * kChunk * 32 * sizeof(float), st>>>(p); }
+          selscan_bwd_summary_kernel<T, HAS_Z><<<grid, block, kChunk * 32 * sizeof(float), st>>>(p); }
         int rc = check_launch("selscan_bwd_summary");
         if (rc != GFE_OK) return rc;
     }
-    const dim3 grid((p.G + W - 1) / W, sp.nseg, a->batch);
+    const dim3 grid(p.G, sp.nseg, a->batch);
     {
-        const size_t smem = (size_t)W * kBwdSmemFloats * sizeof(float);
+        const size_t smem = kBwdSmemFloats * sizeof(float);
         ScopedKernelTimer tm(K_SELSCAN_BWD, st);
         launch_fast(selscan_bwd_kernel<T, HAS_Z>, grid, block, smem, st, p);
     }
@@ -750,7 +742,7 @@ static int launch_bwd_z(const gfe_selscan_args *a, ScanParams &p, const SegPlan 
     return launch_finalize_t<T>(a, p, st);
 }
 
-// dB|dC and parameter-gradient finalize kernels, shared with the v2 backward (selscan_v2_bwd.cu)
+// dB|dC and parameter-gradient finalize kernels, shared with the chained backward (selscan_chain_bwd.cu)
 template <typename T>
 static int launch_finalize_t(const gfe_selscan_args *a, ScanParams &p, cudaStream_t st) {
     const int64_t nbc = (int64_t)a->batch * a->seqlen * 32;

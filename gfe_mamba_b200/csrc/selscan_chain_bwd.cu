@@ -3,10 +3,10 @@
 //
 // Same lane layout as the forward kernel (selscan_v4_fwd.cu): a CTA of 2 * CPC threads serves CPC adjacent channels of
 // one batch row; lane (pair, quad) owns the states 4q..4q+3 of channels 2p and 2p + 1 as four float2 pairs.  Against the
-// first chained backward (one channel per lane, experiments/selscan_v2_bwd.cu) every B|C quad fetched from shared memory
-// feeds eight state-steps instead of four, the first level of the cross-channel dB|dC sums is an FFMA in the lane, the
-// shuffle reduction runs over half as many values, and the per-(t, channel) sums over states leave the lane as ONE
-// 16-byte store.  Per lane and step (8 state-steps): 6 LDS + 48 packed FP32 + 16 exp2 + 7 SHFL + 1 STS.128.
+// first chained backward (one channel x four states per lane, profiles/r02_chain_variants.txt) every B|C quad fetched from
+// shared memory feeds eight state-steps instead of four, the first level of the cross-channel dB|dC sums is an FFMA in the
+// lane, the shuffle reduction runs over half as many values, and the per-(t, channel) sums over states leave the lane as
+// ONE 16-byte store.  Per lane and step (8 state-steps): 6 LDS + 48 packed FP32 + 16 exp2 + 7 SHFL + 1 STS.128.
 //
 // Per unit = (L-segment, batch row, channel block), segments walked last to first (ChainSched, see selscan_shared.cuh; the
 // segments are either chained through flags or independent, their carries then coming from selscan_seg.cu):
@@ -73,7 +73,7 @@ __device__ unsigned long long g_bwd_phase_clk[8];
 #endif
 
 template <typename T, bool HAS_Z, int CPB, int CPC>
-__global__ void __launch_bounds__(2 * CPC, GFE_CBWD_MINB * (64 / CPC)) selscan_bwd_chain_kernel(ScanParams p, ChainSched cs) {
+__global__ void __launch_bounds__(2 * CPC, kBwdMinBlocks * (64 / CPC)) selscan_bwd_chain_kernel(ScanParams p, ChainSched cs) {
 #ifdef GFE_PHASE_CLOCKS
     long long clk_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, clk_last = clock64();
 #endif
@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(2 * CPC, GFE_CBWD_MINB * (64 / CPC)) selscan_b
 #pragma unroll
                     for (int q = 0; q < CKP; ++q) {   // piece tid + q NT of [half][c][16]
                         constexpr int QH = PH / NT;    // pieces per thread and half
-                        if (q / QH < nhalf) cp_async<16>(dst_ck + so + q * NT * 16, sck + (size_t)(q / QH) * ck_step + (q % QH) * NT * 16);
+                        if (q / QH < nhalf) cp_async16(dst_ck + so + q * NT * 16, sck + (size_t)(q / QH) * ck_step + (q % QH) * NT * 16);
                         else *reinterpret_cast<float4 *>(smem + so + SM::kOffCk + (tid + q * NT) * 16) = make_float4(0.f, 0.f, 0.f, 0.f);   // identity half
                     }
                     sck -= 2 * ck_step;
@@ -195,18 +195,18 @@ __global__ void __launch_bounds__(2 * CPC, GFE_CBWD_MINB * (64 / CPC)) selscan_b
                     if (srow < nrows) {
 #pragma unroll
                         for (int q = 0; q < PPT; ++q) {
-                            cp_async<16>(dst_act + so + q * 16, su + q * 16);
-                            cp_async<16>(dst_act + so + SM::kTile + q * 16, sd + q * 16);
-                            cp_async<16>(dst_act + so + 2 * SM::kTile + q * 16, sg_ + q * 16);
+                            cp_async16(dst_act + so + q * 16, su + q * 16);
+                            cp_async16(dst_act + so + SM::kTile + q * 16, sd + q * 16);
+                            cp_async16(dst_act + so + 2 * SM::kTile + q * 16, sg_ + q * 16);
                             if (HAS_Z) {
-                                cp_async<16>(dst_act + so + 3 * SM::kTile + q * 16, sy + q * 16);
-                                cp_async<16>(dst_act + so + 4 * SM::kTile + q * 16, sz + q * 16);
+                                cp_async16(dst_act + so + 3 * SM::kTile + q * 16, sy + q * 16);
+                                cp_async16(dst_act + so + 4 * SM::kTile + q * 16, sz + q * 16);
                             }
                         }
                     }
 #pragma unroll
                     for (int q = 0; q < BCI; ++q)
-                        if (tid + q * NT < 2 * BCP && bcrow[q] < nrows) cp_async<16>(dst_bc + so + q * NT * 16, sbc[q]);
+                        if (tid + q * NT < 2 * BCP && bcrow[q] < nrows) cp_async16(dst_bc + so + q * NT * 16, sbc[q]);
                     constexpr int64_t sz_t = (int64_t)sizeof(T) * kChunk;
                     su -= p.u_rs * sz_t; sd -= p.d_rs * sz_t; sg_ -= p.do_rs * sz_t;
                     if (HAS_Z) { sy -= (int64_t)p.ED * sz_t; sz -= p.z_rs * sz_t; }
@@ -214,16 +214,16 @@ __global__ void __launch_bounds__(2 * CPC, GFE_CBWD_MINB * (64 / CPC)) selscan_b
                     for (int q = 0; q < BCI; ++q) sbc[q] -= ((tid + q * NT) / BCP ? p.C_rs : p.B_rs) * sz_t;
                 } else {
                     unsigned char *s = smem + so;
-                    stage_tile<T, 0, CPC, NT>(s, ub + (int64_t)tb * p.u_rs, p.u_rs, nrows, tid);
-                    stage_tile<T, 0, CPC, NT>(s + SM::kTile, db + (int64_t)tb * p.d_rs, p.d_rs, nrows, tid);
-                    stage_tile<T, 0, CPC, NT>(s + 2 * SM::kTile, gb + (int64_t)tb * p.do_rs, p.do_rs, nrows, tid);
+                    stage_tile<T, CPC, NT>(s, ub + (int64_t)tb * p.u_rs, p.u_rs, nrows, tid);
+                    stage_tile<T, CPC, NT>(s + SM::kTile, db + (int64_t)tb * p.d_rs, p.d_rs, nrows, tid);
+                    stage_tile<T, CPC, NT>(s + 2 * SM::kTile, gb + (int64_t)tb * p.do_rs, p.do_rs, nrows, tid);
                     if (HAS_Z) {
-                        stage_tile<T, 0, CPC, NT>(s + 3 * SM::kTile, yb + (int64_t)tb * p.ED, p.ED, nrows, tid);
-                        stage_tile<T, 0, CPC, NT>(s + 4 * SM::kTile, zb + (int64_t)tb * p.z_rs, p.z_rs, nrows, tid);
+                        stage_tile<T, CPC, NT>(s + 3 * SM::kTile, yb + (int64_t)tb * p.ED, p.ED, nrows, tid);
+                        stage_tile<T, CPC, NT>(s + 4 * SM::kTile, zb + (int64_t)tb * p.z_rs, p.z_rs, nrows, tid);
                     }
                     unsigned char *sb = s + NTILE * SM::kTile;
-                    stage_tile<T, 0, kNState, NT>(sb, Bb + (int64_t)tb * p.B_rs, p.B_rs, nrows, tid);
-                    stage_tile<T, 0, kNState, NT>(sb + SM::kBCRaw, Cb + (int64_t)tb * p.C_rs, p.C_rs, nrows, tid);
+                    stage_tile<T, kNState, NT>(sb, Bb + (int64_t)tb * p.B_rs, p.B_rs, nrows, tid);
+                    stage_tile<T, kNState, NT>(sb + SM::kBCRaw, Cb + (int64_t)tb * p.C_rs, p.C_rs, nrows, tid);
                 }
             }
             cp_async_commit();

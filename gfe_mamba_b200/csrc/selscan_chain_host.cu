@@ -2,9 +2,6 @@
 // the launch plan (channel-block width, L-segments), the workspace layout of the chain scheduler, argument checks and
 // the forward dispatch.  Everything here is a pure function of the shape and the current device, so the size queries of
 // the C ABI and the launches always agree.
-#include <stdlib.h>
-#include <string.h>
-
 #include "common.cuh"
 #include "selscan_shared.cuh"
 
@@ -18,13 +15,10 @@ int seg_launch_carries(const ScanParams &p, const ChainSched &cs, int dtype, int
 // L is cut into chained segments, ~12 units per resident CTA: the units of a chain interleave with those of the others and
 // hop between SMs, which evens out SMs that host 2 and 3 working CTAs (measured on cfg3, profiles/r02_chain_variants.txt:
 // 10-16 segments beat 1, 4 and 32 by 2-4 %).  Independent segments (too few chains to fill the GPU) only need enough units
-// for the dynamic scheduler to balance the resident CTAs: ~3 per CTA.
+// for the dynamic scheduler to balance the resident CTAs: 2 per CTA (2 / 3 / 6 measured on cfg4, 2 fastest by 1-3 %).
 static void chain_plan(int B, int L, int nblk, int ctas_per_sm, bool independent, int &nseg, int &seg_len) {
     const int64_t slots = (int64_t)sm_count() * ctas_per_sm;
-    int64_t want = ceil_div64((independent ? GFE_SEG_UNITS_PER_CTA : 12) * slots, (int64_t)B * nblk);
-#ifdef GFE_EXPERIMENTS
-    if (const char *e = getenv("GFE_CHAIN_NSEG")) want = atoi(e);   // A/B measurements only
-#endif
+    int64_t want = ceil_div64((independent ? 2 : 12) * slots, (int64_t)B * nblk);
     const int64_t max_by_len = L / (8 * kChunk) > 0 ? L / (8 * kChunk) : 1;   // >= 128 steps per segment
     if (want > max_by_len) want = max_by_len;
     if (want > kMaxSeg) want = kMaxSeg;
@@ -33,53 +27,28 @@ static void chain_plan(int B, int L, int nblk, int ctas_per_sm, bool independent
     nseg = (L + seg_len - 1) / seg_len;
 }
 
-// Channel-block width: 64 when it divides ED, else 32 (16 / 32 / 64 measured on cfg3 and cfg5: 64 is never slower,
-// profiles/r02_chain_variants.txt).
-static int fwd_cpc(int ED) {
-#ifdef GFE_EXPERIMENTS
-    if (const char *e = getenv("GFE_FWD_CPC")) {   // A/B measurements only
-        const int v = atoi(e);
-        if ((v == 32 || v == 64) && ED % v == 0) return v;
-    }
-#endif
-    return ED % GFE_FWD_CPC_DEFAULT == 0 ? GFE_FWD_CPC_DEFAULT : 32;
-}
-static int bwd_cpc(int ED) {
-#ifdef GFE_EXPERIMENTS
-    if (const char *e = getenv("GFE_BWD_CPC")) {
-        const int v = atoi(e);
-        if ((v == 32 || v == 64) && ED % v == 0) return v;
-    }
-#endif
-    return ED % GFE_BWD_CPC_DEFAULT == 0 ? GFE_BWD_CPC_DEFAULT : 32;
-}
+// Channel-block width of both directions: 64 when it divides ED, else 32 (16 / 32 / 64 measured on cfg3 and cfg5: 64 is
+// never slower, profiles/r02_chain_variants.txt).
+static int chain_cpc(int ED) { return ED % 64 == 0 ? 64 : 32; }
 
 // Chains wait for their predecessor segment when B * ED alone fills the GPU (plan_segments: at least half the schedulers
 // get a warp without splitting L); otherwise the segments are made independent by a summary + combine pass.
-static bool chain_independent(int B, int L, int ED) {
-#ifdef GFE_EXPERIMENTS
-    if (const char *e = getenv("GFE_SELSCAN_CHAIN")) {   // A/B measurements only: 1 = always wait, 2 = always independent
-        if (e[0] == '1') return false;
-        if (e[0] == '2') return true;
-    }
-#endif
-    return plan_segments(B, L, ED).nseg > 1;
-}
+static bool chain_independent(int B, int L, int ED) { return plan_segments(B, L, ED).nseg > 1; }
 
 ChainPlan chain_fwd_plan(int B, int L, int ED) {
     ChainPlan pl{};
-    pl.cpc = fwd_cpc(ED);
+    pl.cpc = chain_cpc(ED);
     pl.nblk = ED / pl.cpc;
     pl.independent = chain_independent(B, L, ED) ? 1 : 0;
-    chain_plan(B, L, pl.nblk, 3 * (64 / pl.cpc), pl.independent, pl.nseg, pl.seg_len);
+    chain_plan(B, L, pl.nblk, kFwdMinBlocks * (64 / pl.cpc), pl.independent, pl.nseg, pl.seg_len);
     return pl;
 }
 ChainPlan chain_bwd_plan(int B, int L, int ED) {
     ChainPlan pl{};
-    pl.cpc = bwd_cpc(ED);
+    pl.cpc = chain_cpc(ED);
     pl.nblk = ED / pl.cpc;
     pl.independent = chain_independent(B, L, ED) ? 1 : 0;
-    chain_plan(B, L, pl.nblk, GFE_CBWD_MINB * (64 / pl.cpc), pl.independent, pl.nseg, pl.seg_len);
+    chain_plan(B, L, pl.nblk, kBwdMinBlocks * (64 / pl.cpc), pl.independent, pl.nseg, pl.seg_len);
     return pl;
 }
 
@@ -145,7 +114,7 @@ int chain_check_alignment(const gfe_selscan_args *a) {
 }
 
 size_t chain_ckpt_state_bytes(int B, int L, int ED, int dtype) {   // [b][t / 8][c][16], fp32 (bf16 for bf16 activations), 256-byte padded
-    const size_t el = (GFE_CKPT_BF16 && dtype == GFE_BF16) ? 2 : 4;
+    const size_t el = dtype == GFE_BF16 ? 2 : 4;
     return align_up((size_t)B * ((L + kCkptV2 - 1) / kCkptV2) * ED * kNState * el, 256);
 }
 
@@ -172,10 +141,6 @@ int chain_cpb(const gfe_selscan_args *a, bool bwd) {
     for (const void *q : ptrs) ok &= (reinterpret_cast<uintptr_t>(q) & 15) == 0;
     for (int64_t stv : strides) ok &= (stv * s) % 16 == 0;
     if (a->ckpt) ok &= (reinterpret_cast<uintptr_t>(a->ckpt) & 15) == 0;
-#ifdef GFE_EXPERIMENTS
-    if (const char *e = getenv("GFE_SELSCAN_PATH"))
-        if (!strcmp(e, "plain")) ok = false;
-#endif
     return ok ? 16 : 0;
 }
 

@@ -17,16 +17,9 @@
 
 namespace gfe {
 
-#ifndef GFE_SEG_STAGES
-#define GFE_SEG_STAGES 3
-#endif
-#ifndef GFE_SEG_POLY
-#define GFE_SEG_POLY 1   // exp2 pairs (of 4 per lane and step) evaluated on the FMA pipe
-#endif
-
 template <typename T, bool HAS_Z, int CPC>
 struct SegSumSmem {
-    static constexpr int kStages = GFE_SEG_STAGES;                       // (2, 3 and 4 stages measure the same)
+    static constexpr int kStages = 3;                                    // (2, 3 and 4 stages measure the same)
     static constexpr int kNTile = HAS_Z ? 3 : 2;                         // x (u forward | dout reverse), delta, [z]
     static constexpr int kTile = kChunk * CPC * (int)sizeof(T);
     static constexpr int kBCRaw = kChunk * kNState * (int)sizeof(T);     // B rows (forward) | C rows (reverse)
@@ -93,23 +86,23 @@ __global__ void __launch_bounds__(2 * CPC, 4 * (64 / CPC)) selscan_seg_summary_k
                         const char *sd = reinterpret_cast<const char *>(db + (int64_t)(tb + srow) * p.d_rs) + spiece * 16;
 #pragma unroll
                         for (int q = 0; q < PPT; ++q) {
-                            cp_async<16>(dst_act + so + q * 16, su + q * 16);
-                            cp_async<16>(dst_act + so + SM::kTile + q * 16, sd + q * 16);
+                            cp_async16(dst_act + so + q * 16, su + q * 16);
+                            cp_async16(dst_act + so + SM::kTile + q * 16, sd + q * 16);
                         }
                         if (HAS_Z) {
                             const char *sz = reinterpret_cast<const char *>(zb + (int64_t)(tb + srow) * p.z_rs) + spiece * 16;
 #pragma unroll
-                            for (int q = 0; q < PPT; ++q) cp_async<16>(dst_act + so + 2 * SM::kTile + q * 16, sz + q * 16);
+                            for (int q = 0; q < PPT; ++q) cp_async16(dst_act + so + 2 * SM::kTile + q * 16, sz + q * 16);
                         }
                     }
                     if (tid < BCP && bcrow < nrows)
-                        cp_async<16>(dst_bc + so, reinterpret_cast<const char *>(BCb + (int64_t)(tb + bcrow) * bc_rs) + bcpiece * 16);
+                        cp_async16(dst_bc + so, reinterpret_cast<const char *>(BCb + (int64_t)(tb + bcrow) * bc_rs) + bcpiece * 16);
                 } else {
                     unsigned char *s = smem + so;
-                    stage_tile<T, 0, CPC, NT>(s, xb + (int64_t)tb * x_rs, x_rs, nrows, tid);
-                    stage_tile<T, 0, CPC, NT>(s + SM::kTile, db + (int64_t)tb * p.d_rs, p.d_rs, nrows, tid);
-                    if (HAS_Z) stage_tile<T, 0, CPC, NT>(s + 2 * SM::kTile, zb + (int64_t)tb * p.z_rs, p.z_rs, nrows, tid);
-                    stage_tile<T, 0, kNState, NT>(s + NTILE * SM::kTile, BCb + (int64_t)tb * bc_rs, bc_rs, nrows, tid);
+                    stage_tile<T, CPC, NT>(s, xb + (int64_t)tb * x_rs, x_rs, nrows, tid);
+                    stage_tile<T, CPC, NT>(s + SM::kTile, db + (int64_t)tb * p.d_rs, p.d_rs, nrows, tid);
+                    if (HAS_Z) stage_tile<T, CPC, NT>(s + 2 * SM::kTile, zb + (int64_t)tb * p.z_rs, p.z_rs, nrows, tid);
+                    stage_tile<T, kNState, NT>(s + NTILE * SM::kTile, BCb + (int64_t)tb * bc_rs, bc_rs, nrows, tid);
                 }
             }
             cp_async_commit();
@@ -188,8 +181,9 @@ __global__ void __launch_bounds__(2 * CPC, 4 * (64 / CPC)) selscan_seg_summary_k
                 for (int ch = 0; ch < 2; ++ch) {
                     const float dl = ch ? dd.z : dd.x, v = ch ? dd.w : dd.y;
                     const float2 x0 = fmul2(splat2(dl), A2[ch][0]), x1 = fmul2(splat2(dl), A2[ch][1]);
-                    const float2 a0 = (GFE_SEG_POLY >= 1 && ch == 0) ? ex2_poly2(x0) : ex2_2(x0);
-                    const float2 a1 = (GFE_SEG_POLY >= 2 && ch == 1) ? ex2_poly2(x1) : ex2_2(x1);
+                    // one exp2 pair of 4 on the FMA pipe (0 / 1 / 2 pairs measured on cfg4: 1 fastest, profiles/r02_chain_variants.txt)
+                    const float2 a0 = ch == 0 ? ex2_poly2(x0) : ex2_2(x0);
+                    const float2 a1 = ex2_2(x1);
                     if (REV) {
                         h[ch][0] = fmul2(a0, ffma2(B01, splat2(v), h[ch][0]));
                         h[ch][1] = fmul2(a1, ffma2(B23, splat2(v), h[ch][1]));

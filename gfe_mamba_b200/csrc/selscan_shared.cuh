@@ -4,10 +4,6 @@
 
 #include "common.cuh"
 
-#ifndef GFE_CKPT_BF16
-#define GFE_CKPT_BF16 1        // chained kernels: bf16 activations keep their 8-step state checkpoints in bf16 (half the checkpoint stream)
-#endif
-
 namespace gfe {
 
 struct ScanParams {
@@ -21,7 +17,7 @@ struct ScanParams {
     int64_t o_bs, o_rs;
     float *last_state;
     float2 *ckpt;   // [B][nchunks][8][ED]
-    void *ysave;    // [B][L][ED] activation dtype: y before the gate (fast kernels), lives behind ckpt
+    void *ysave;    // [B][L][ED] activation dtype: y before the gate, lives behind ckpt (written by the chained kernels only)
     float2 *seg_h;  // [B][nseg][8][ED]  segment-local end state (fwd) / start carry (bwd)
     float *seg_sd;  // [B][nseg][ED]     sum of delta over the segment
     // backward
@@ -33,13 +29,13 @@ struct ScanParams {
     float *part_bc;   // [G][B][L][32]   per-warp dB|dC rows
     float *part_par;  // [B][nseg][18][ED]
     int G;            // ceil(ED / 32)
-    int bc_interleaved;   // part_bc rows are {dB[n], dC[n]} pairs (v2 backward) instead of dB[16] | dC[16]
+    int bc_interleaved;   // part_bc rows: 1 = {dB[n], dC[n]} pairs (chained backward), 0 = dB[16] | dC[16] (generic backward)
 };
 
 constexpr int kPairs = kNState / 2;
 constexpr int kRedStride = 34;  // padded row of the reduced dB|dC tile (bank-conflict free float2 writes)
 
-// Dynamic chaining of L-segments (v2 kernels): persistent CTAs draw (segment, batch row, channel block) units from an
+// Dynamic chaining of L-segments (chained kernels): persistent CTAs draw (segment, batch row, channel block) units from an
 // atomic counter in segment-major order; a unit waits for the flag of its predecessor segment, reads the carried
 // state, and publishes its own.  Units are drawn in dependency order, so a waiting CTA only ever waits on a unit that
 // is already running or finished: no deadlock, no tail quantisation, no recomputation.
@@ -60,32 +56,13 @@ struct ChainSched {
 // ---- cp.async helpers -------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-template <int BYTES>
-__device__ __forceinline__ void cp_async(uint32_t dst, const void *src) {
-    if constexpr (BYTES == 16) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-    else if constexpr (BYTES == 8) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(src) : "memory");
-    else asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
+// one 16-byte piece, global -> shared, bypassing L1
+__device__ __forceinline__ void cp_async16(uint32_t dst, const void *src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-// Copy up to kChunk rows of ROW_ELEMS contiguous elements (row stride rs elements) into a dense shared tile.
-template <typename T, int CPB, int ROW_ELEMS>
-__device__ __forceinline__ void tile_issue(uint32_t dst, const T *src, int64_t rs, int nrows, int lane, int dst_row_bytes,
-                                           int dst_col_byte_off) {
-    constexpr int RB = ROW_ELEMS * (int)sizeof(T);   // bytes per source row
-    constexpr int PPR = RB / CPB;                     // pieces per row
-    constexpr int TOTAL = kChunk * PPR;
-    const char *s = reinterpret_cast<const char *>(src);
-#pragma unroll
-    for (int i0 = 0; i0 < TOTAL; i0 += 32) {
-        const int i = i0 + lane;
-        const int row = i / PPR, piece = i % PPR;
-        if ((TOTAL % 32 == 0 || i < TOTAL) && row < nrows)
-            cp_async<CPB>(dst + row * dst_row_bytes + dst_col_byte_off + piece * CPB, s + (int64_t)row * rs * (int64_t)sizeof(T) + piece * CPB);
-    }
-}
 
 // exp2 of two non-positive arguments on the FMA pipe: Cody-Waite split + degree-5 minimax with p(0) = 1 exactly (max rel err 2.4e-7
 // in fp32, same class as ex2.approx), exponent inserted with integer adds.
@@ -106,73 +83,13 @@ __device__ __forceinline__ float2 ex2_poly2(float2 x) {
                        __int_as_float(__float_as_int(p.y) + (__float_as_int(t.y) << 23)));
 }
 
-// log1p(e) for 0 <= e < 0.5 via 2 atanh(e / (2 + e))
-__device__ __forceinline__ float log1p_small(float e) {
-    const float s = e * rcp_approx(2.0f + e);
-    const float s2 = s * s;
-    float p = fmaf(s2, 1.0f / 9.0f, 1.0f / 7.0f);
-    p = fmaf(s2, p, 1.0f / 5.0f);
-    p = fmaf(s2, p, 1.0f / 3.0f);
-    p = fmaf(s2, p, 1.0f);
-    return 2.0f * s * p;
-}
-
-// softplus for a group of G steps, branch-free per lane; the log1p formulation is chosen by a warp-uniform vote.
-// x[i] -> dl[i]; optionally sig[i] = sigmoid(x[i]).
-template <int G, bool WANT_SIG>
-__device__ __forceinline__ void softplus_group(const float (&x)[G], float (&dl)[G], float (&sig)[G]) {
-    float e[G];
-    bool any_big = false;
-#pragma unroll
-    for (int i = 0; i < G; ++i) {
-        e[i] = ex2_approx(fminf(x[i], 30.0f) * kLog2e);
-        any_big |= e[i] >= 0.5f;
-    }
-#pragma unroll
-    for (int i = 0; i < G; ++i) dl[i] = log1p_small(fminf(e[i], 0.5f));
-    if (__any_sync(0xffffffffu, any_big)) {
-#pragma unroll
-        for (int i = 0; i < G; ++i) {
-            const float big = kLn2 * lg2_approx(1.0f + e[i]);
-            dl[i] = e[i] >= 0.5f ? big : dl[i];
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < G; ++i) {
-        if (WANT_SIG) sig[i] = x[i] > 20.0f ? 1.0f : e[i] * rcp_approx(1.0f + e[i]);
-        dl[i] = x[i] > 20.0f ? x[i] : dl[i];
-    }
-}
-
-
-// Branch-free softplus of two values (no vote, no second formulation, so it can be interleaved with other work):
-// softplus(x) = max(x, 0) + log1p(w), w = exp(-|x|) in (0, 1], log1p(w) = 2 atanh(w / (2 + w)) with six odd terms
-// (s^2 <= 1/9: relative error < 1e-6 for every x; x > 20 returns x to fp32 rounding, the torch threshold).
-// Optionally sig = sigmoid(x) = d softplus / dx.
+// Branch-free softplus of two values (one formulation for every x, so it can be interleaved with other work):
+// softplus(x) = max(x, 0) + log1p(w), w = exp(-|x|) in (0, 1], with log1p(w) = ln2 * lg2(1 + w) on the MUFU pipe: 1 + w is in
+// [1, 2], where lg2.approx is accurate to 2^-22.6 ABSOLUTE, i.e. softplus to ~1.2e-7 absolute -- what the max-normalised
+// tolerances of the path need -- for 6 instead of the 15 FP32-pipe instructions per pair of a 2 atanh(w / (2 + w)) series
+// (the item phases are issue-bound, not MUFU-bound).  Optionally sig = sigmoid(x) = d softplus / dx.
 template <bool WANT_SIG>
-__device__ __forceinline__ float2 softplus2(float2 x, float2 &sig) {
-    const float2 w = ex2_2(make_float2(fabsf(x.x) * -kLog2e, fabsf(x.y) * -kLog2e));
-    const float2 d = fadd2(w, splat2(2.0f));
-    const float2 s = fmul2(w, make_float2(rcp_approx(d.x), rcp_approx(d.y)));
-    const float2 s2 = fmul2(s, s);
-    float2 p = ffma2(s2, splat2(2.0f / 11.0f), splat2(2.0f / 9.0f));
-    p = ffma2(p, s2, splat2(2.0f / 7.0f));
-    p = ffma2(p, s2, splat2(2.0f / 5.0f));
-    p = ffma2(p, s2, splat2(2.0f / 3.0f));
-    p = ffma2(p, s2, splat2(2.0f));
-    const float2 r = fmul2(s, p);
-    if (WANT_SIG) {
-        const float2 q = make_float2(rcp_approx(1.0f + w.x), rcp_approx(1.0f + w.y));   // sigmoid(|x|)
-        sig = make_float2(x.x >= 0.f ? q.x : w.x * q.x, x.y >= 0.f ? q.y : w.y * q.y);
-    }
-    return make_float2(fmaxf(x.x, 0.f) + r.x, fmaxf(x.y, 0.f) + r.y);
-}
-
-// The same with log1p(w) = ln2 * lg2(1 + w) on the MUFU pipe: 1 + w is in [1, 2], where lg2.approx is accurate to 2^-22.6
-// ABSOLUTE, i.e. softplus to ~1.2e-7 absolute -- what the max-normalised tolerances of the path need -- for 6 instead of 15
-// FP32-pipe instructions per pair (the item phases are issue-bound, not MUFU-bound).
-template <bool WANT_SIG>
-__device__ __forceinline__ float2 softplus2_lg(float2 x, float2 &sig) {
+__device__ __forceinline__ float2 softplus_pair(float2 x, float2 &sig) {
     const float2 w = ex2_2(make_float2(fabsf(x.x) * -kLog2e, fabsf(x.y) * -kLog2e));
     const float2 d = fadd2(w, splat2(1.0f));
     if (WANT_SIG) {
@@ -181,25 +98,12 @@ __device__ __forceinline__ float2 softplus2_lg(float2 x, float2 &sig) {
     }
     return make_float2(fmaf(kLn2, lg2_approx(d.x), fmaxf(x.x, 0.f)), fmaf(kLn2, lg2_approx(d.y), fmaxf(x.y, 0.f)));
 }
-#ifndef GFE_SOFTPLUS_LG2
-#define GFE_SOFTPLUS_LG2 1
-#endif
-template <bool WANT_SIG>
-__device__ __forceinline__ float2 softplus_pair(float2 x, float2 &sig) {
-#if GFE_SOFTPLUS_LG2
-    return softplus2_lg<WANT_SIG>(x, sig);
-#else
-    return softplus2<WANT_SIG>(x, sig);
-#endif
-}
 
-// Element type of the chained kernels' state checkpoints: fp32, except bf16 for bf16 activations (the recomputed states then
-// carry a 2^-9 relative error, well inside the 2e-2 tolerance of that dtype; fp16 keeps fp32 checkpoints: states can exceed
-// its range).
+// Element type of the chained kernels' state checkpoints: fp32, except bf16 for bf16 activations (half the checkpoint
+// stream; the recomputed states then carry a 2^-9 relative error, well inside the 2e-2 tolerance of that dtype; fp16 keeps
+// fp32 checkpoints: states can exceed its range).
 template <typename T> struct CkptOf { using type = float; };
-#if GFE_CKPT_BF16
 template <> struct CkptOf<__nv_bfloat16> { using type = __nv_bfloat16; };
-#endif
 __device__ __forceinline__ void ckpt_store(float *dst, float4 v) { __stcs(reinterpret_cast<float4 *>(dst), v); }
 __device__ __forceinline__ void ckpt_store(__nv_bfloat16 *dst, float4 v) {
     const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
@@ -222,7 +126,7 @@ __device__ __forceinline__ void st_release(int *p, int v) {
     asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
-// ---- two adjacent channels at a time (item phases of the v2 kernels) -----------------------------------------
+// ---- two adjacent channels at a time (item phases of the chained kernels) ------------------------------------
 template <typename T> struct Pair;
 template <> struct Pair<float> { using type = float2; };
 template <> struct Pair<__nv_bfloat16> { using type = __nv_bfloat162; };
@@ -257,41 +161,15 @@ template <typename T> __device__ __forceinline__ void stg_pair(T *dst, float a, 
     }
 }
 
-// Copy nrows rows of ROW_ELEMS contiguous elements (row stride rs elements) into a dense shared tile, all NT threads
-// of the CTA taking part.  CPB = 16: cp.async 16-byte pieces (bases and strides 16-byte aligned); CPB = 0: plain loads.
-template <typename T, int CPB, int ROW_ELEMS, int NT>
+// Copy nrows rows of ROW_ELEMS contiguous elements (row stride rs elements) into a dense shared tile with plain loads, all
+// NT threads of the CTA taking part: the staging path of tensors whose bases or strides rule out 16-byte cp.async pieces.
+template <typename T, int ROW_ELEMS, int NT>
 __device__ __forceinline__ void stage_tile(unsigned char *dst, const T *src, int64_t rs, int nrows, int tid) {
-    constexpr int RB = ROW_ELEMS * (int)sizeof(T);
-    if constexpr (CPB == 16) {
-        constexpr int PPR = RB / 16;
-        const int total = nrows * PPR;
-        const uint32_t d = smem_u32(dst);
-        const char *s = reinterpret_cast<const char *>(src);
-        for (int i = tid; i < total; i += NT) {
-            const int row = i / PPR, piece = i % PPR;
-            cp_async<16>(d + row * RB + piece * 16, s + (int64_t)row * rs * (int64_t)sizeof(T) + piece * 16);
-        }
-    } else {
-        const int total = nrows * ROW_ELEMS;
-        T *d = reinterpret_cast<T *>(dst);
-        for (int i = tid; i < total; i += NT) {
-            const int row = i / ROW_ELEMS, col = i % ROW_ELEMS;
-            d[i] = src[(int64_t)row * rs + col];
-        }
-    }
-}
-// One 16-row tile whose 16 * ROW_ELEMS * sizeof(T) / 16 pieces are at most NT: every thread moves at most ONE 16-byte
-// piece, no loop, row stride taken from the (uniform) kernel parameters.  Falls back to stage_tile for plain loads.
-template <typename T, int CPB, int ROW_ELEMS, int NT>
-__device__ __forceinline__ void stage_tile1(unsigned char *dst, const T *src, int64_t rs, int nrows, int tid) {
-    constexpr int RB = ROW_ELEMS * (int)sizeof(T);
-    constexpr int PPR = RB / 16;
-    if constexpr (CPB == 16 && kChunk * PPR <= NT) {
-        const int row = tid / PPR, piece = tid % PPR;
-        if (tid < kChunk * PPR && row < nrows)
-            cp_async<16>(smem_u32(dst) + tid * 16, reinterpret_cast<const char *>(src + (int64_t)row * rs) + piece * 16);
-    } else {
-        stage_tile<T, CPB, ROW_ELEMS, NT>(dst, src, rs, nrows, tid);
+    const int total = nrows * ROW_ELEMS;
+    T *d = reinterpret_cast<T *>(dst);
+    for (int i = tid; i < total; i += NT) {
+        const int row = i / ROW_ELEMS, col = i % ROW_ELEMS;
+        d[i] = src[(int64_t)row * rs + col];
     }
 }
 #endif  // __CUDACC__
@@ -321,18 +199,11 @@ static int persistent_grid(int nt, size_t smem, int total) {
 #endif
 
 // host side of the chained kernels (selscan_chain_host.cu, selscan_chain_bwd.cu)
-#ifndef GFE_FWD_CPC_DEFAULT
-#define GFE_FWD_CPC_DEFAULT 64   // channel-block width of the forward kernel when ED allows it
-#endif
-#ifndef GFE_BWD_CPC_DEFAULT
-#define GFE_BWD_CPC_DEFAULT 64
-#endif
-#ifndef GFE_CBWD_MINB
-#define GFE_CBWD_MINB 2        // backward: CTAs of 128 threads per SM the register budget is set for (2: 255 registers, 3: 168)
-#endif
-#ifndef GFE_SEG_UNITS_PER_CTA
-#define GFE_SEG_UNITS_PER_CTA 2   // independent segments: units per resident CTA the plan aims for
-#endif
+// CTAs of 128 threads per SM that the chained kernels' register budgets (__launch_bounds__) and the launch plans are set for.
+// Forward 3: 4 (126 registers) measured 2-8 % slower on cfg3 and cfg5.  Backward 2: 255 registers without spills; 3 caps
+// it at 168 registers with spills and measured slower on both (profiles/r02_chain_variants.txt).
+constexpr int kFwdMinBlocks = 3;
+constexpr int kBwdMinBlocks = 2;
 struct ChainPlan {
     int cpc, nblk;          // channel-block width and count
     int nseg, seg_len;      // L-segments (seg_len a multiple of kChunk)

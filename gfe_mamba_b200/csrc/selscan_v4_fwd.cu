@@ -1,16 +1,17 @@
 // selscan_v4_fwd.cu -- fused selective-scan forward, "v4": two channels x four states per lane.
 // Replaces mamba.py:255-256, 275-284, 220-222 of the reference (softplus -> discretise -> scan -> C.h -> D skip -> gate).
 //
-// What the v2 profile said (profiles/r01_ab_*): the forward was bound by the shared-memory data pipe and by issue slots,
-// not by HBM.  An LDS.128 costs ~2 pipe clocks whatever its address pattern (tools/microbench_lds.cu), so the number
-// of LDS per state-step is what matters, and half of v2's instructions were spent outside the recurrence.  Here
+// What the profile of the first chained forward (one channel x four states per lane, profiles/r01_ab_*) said: it was bound by
+// the shared-memory data pipe and by issue slots, not by HBM.  An LDS.128 costs ~2 pipe clocks whatever its address pattern
+// (tools/microbench_lds.cu), so the number of LDS per state-step is what matters, and half of its instructions were spent
+// outside the recurrence.  Here
 //   * a lane owns the states 4q..4q+3 of TWO adjacent channels: the B and C quads it fetches feed eight state-steps
 //     instead of four, and {delta, delta*u} of both channels arrive in one LDS.128 (no splatted copies: ptxas folds a
 //     scalar operand of FFMA2/FMUL2 into the R.F32 broadcast form);
 //   * a CTA of 128 threads serves 64 channels; every thread stages exactly one 16-byte piece per tile with offsets
 //     computed once per unit, and the per-(t, channel pair) scalar work runs once per pair in the item mapping;
 //   * per lane and step: 3 LDS.128 + 16 packed FP32 ops + 8 exp2 (every other step 2 of them on the FMA pipe) + 1 STS.64 for 8
-//     state-steps (v2: 3 LDS.128 + 8 + 4 + 1 for 4); the slot loads run two steps ahead of their use;
+//     state-steps (one channel per lane: 3 LDS.128 + 8 + 4 + 1 for 4); the slot loads run two steps ahead of their use;
 //   * the item phases work on packed FP32 over the channel pair, slots are laid out in pair order {dl0, dl1, dl0 u0, dl1 u1},
 //     rows are masked only in a ragged last chunk, paired stores are a compile-time property of the cp.async instantiation.
 // Segments are chained (ChainSched) or independent (carries from selscan_seg.cu); checkpoints [b][t/8][c][16] (fp32, bf16 for bf16 activations) and the saved y are what
@@ -22,20 +23,7 @@
 
 namespace gfe {
 
-// CPC = channels per CTA (64, 32 or 16); 2 * CPC threads: lane (pair, quad) owns 2 channels x 4 states.  With CPC = 16 a
-// CTA is a single warp and every __syncthreads below is a warp barrier: the warps of an SM then run fully decoupled.
-#ifndef GFE_SOFTPLUS2
-#define GFE_SOFTPLUS2 1
-#endif
-#ifndef GFE_V4_PREFETCH
-#define GFE_V4_PREFETCH 2
-#endif
-#ifndef GFE_V4_POLY
-#define GFE_V4_POLY 1
-#endif
-#ifndef GFE_V4_MINB
-#define GFE_V4_MINB 3
-#endif
+// CPC = channels per CTA (64 or 32); 2 * CPC threads: lane (pair, quad) owns 2 channels x 4 states.
 template <typename T, bool HAS_Z, int CPC>
 struct FwdV4Smem {
     static constexpr int kV4CPC = CPC;
@@ -59,7 +47,9 @@ __device__ __forceinline__ void v4_recur_chunk(const float4 *__restrict__ dd_r, 
                                                float2 *__restrict__ y_w, const float2 (&A2)[2][2], float2 (&h)[2][2],
                                                CK *__restrict__ ckq, size_t ck_step, int tb, int t1) {
     constexpr int kV4YPlane = CPC / 2 + 4;
-    constexpr int PF = GFE_V4_PREFETCH;   // slot loads are issued PF steps ahead of their use, BEFORE the stores of the steps between
+    // slot loads are issued PF steps ahead of their use, BEFORE the stores of the steps between (1 / 2 / 3 / 4 steps measured on
+    // cfg3 and cfg5: 2 within 1 % of the best on both, profiles/r02_chain_variants.txt)
+    constexpr int PF = 2;
     float4 dd_q[PF + 1], B_q[PF + 1], C_q[PF + 1];
 #pragma unroll
     for (int i = 0; i < PF; ++i) { dd_q[i] = dd_r[i * (CPC / 2)]; B_q[i] = bc_r[i * 8]; C_q[i] = bc_r[i * 8 + 4]; }
@@ -85,9 +75,10 @@ __device__ __forceinline__ void v4_recur_chunk(const float4 *__restrict__ dd_r, 
         for (int ch = 0; ch < 2; ++ch) {
             const float dl = ch ? dd.y : dd.x, du = ch ? dd.w : dd.z;
             const float2 x0 = fmul2(splat2(dl), A2[ch][0]), x1 = fmul2(splat2(dl), A2[ch][1]);
-            // GFE_V4_POLY of every 8 exps of a step run as a polynomial on the FMA pipe instead of MUFU.EX2
-            const float2 a0 = (GFE_V4_POLY >= 1 && ch == 0 && (j & 1)) ? ex2_poly2(x0) : ex2_2(x0);
-            const float2 a1 = (GFE_V4_POLY >= 2 && ch == 1 && !(j & 1)) ? ex2_poly2(x1) : ex2_2(x1);
+            // on odd steps one exp2 pair of 4 runs as a polynomial on the FMA pipe instead of MUFU.EX2 (0 / 1 / 2 pairs measured
+            // on cfg3: 1 fastest, profiles/r02_chain_variants.txt)
+            const float2 a0 = (ch == 0 && (j & 1)) ? ex2_poly2(x0) : ex2_2(x0);
+            const float2 a1 = ex2_2(x1);
             h[ch][0] = ffma2(a0, h[ch][0], fmul2(splat2(du), B01));
             h[ch][1] = ffma2(a1, h[ch][1], fmul2(splat2(du), B23));
             const float2 y2 = ffma2(h[ch][1], C23, fmul2(h[ch][0], C01));
@@ -105,7 +96,7 @@ __device__ unsigned long long g_fwd_phase_clk[8];
 #endif
 
 template <typename T, bool HAS_Z, int CPB, int CPC>
-__global__ void __launch_bounds__(2 * CPC, GFE_V4_MINB * (64 / CPC)) selscan_fwd_v4_kernel(ScanParams p, ChainSched cs) {
+__global__ void __launch_bounds__(2 * CPC, kFwdMinBlocks * (64 / CPC)) selscan_fwd_v4_kernel(ScanParams p, ChainSched cs) {
 #ifdef GFE_PHASE_CLOCKS
     long long clk_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}, clk_last = clock64();
 #endif
@@ -189,14 +180,14 @@ __global__ void __launch_bounds__(2 * CPC, GFE_V4_MINB * (64 / CPC)) selscan_fwd
                     if (srow < nrows) {
 #pragma unroll
                         for (int i = 0; i < PPT; ++i) {
-                            cp_async<16>(dst_act + so + i * 16, su + i * 16);
-                            cp_async<16>(dst_act + so + SM::kTile + i * 16, sd + i * 16);
-                            if (HAS_Z) cp_async<16>(dst_act + so + 2 * SM::kTile + i * 16, sz + i * 16);
+                            cp_async16(dst_act + so + i * 16, su + i * 16);
+                            cp_async16(dst_act + so + SM::kTile + i * 16, sd + i * 16);
+                            if (HAS_Z) cp_async16(dst_act + so + 2 * SM::kTile + i * 16, sz + i * 16);
                         }
                     }
 #pragma unroll
                     for (int i = 0; i < BCI; ++i)
-                        if (tid + i * NT < 2 * BCP && bcrow[i] < nrows) cp_async<16>(dst_bc + so + i * NT * 16, sbc[i]);
+                        if (tid + i * NT < 2 * BCP && bcrow[i] < nrows) cp_async16(dst_bc + so + i * NT * 16, sbc[i]);
                     constexpr int64_t sz_t = (int64_t)sizeof(T) * kChunk;
                     su += p.u_rs * sz_t; sd += p.d_rs * sz_t;
                     if (HAS_Z) sz += p.z_rs * sz_t;
@@ -204,11 +195,11 @@ __global__ void __launch_bounds__(2 * CPC, GFE_V4_MINB * (64 / CPC)) selscan_fwd
                     for (int i = 0; i < BCI; ++i) sbc[i] += ((tid + i * NT) / BCP ? p.C_rs : p.B_rs) * sz_t;
                 } else {
                     unsigned char *s = smem + so;
-                    stage_tile<T, 0, CPC, NT>(s, ub + (int64_t)tb * p.u_rs, p.u_rs, nrows, tid);
-                    stage_tile<T, 0, CPC, NT>(s + SM::kTile, db + (int64_t)tb * p.d_rs, p.d_rs, nrows, tid);
-                    if (HAS_Z) stage_tile<T, 0, CPC, NT>(s + 2 * SM::kTile, zb + (int64_t)tb * p.z_rs, p.z_rs, nrows, tid);
-                    stage_tile<T, 0, kNState, NT>(s + NTILE * SM::kTile, Bb + (int64_t)tb * p.B_rs, p.B_rs, nrows, tid);
-                    stage_tile<T, 0, kNState, NT>(s + NTILE * SM::kTile + SM::kBCRaw, Cb + (int64_t)tb * p.C_rs, p.C_rs, nrows, tid);
+                    stage_tile<T, CPC, NT>(s, ub + (int64_t)tb * p.u_rs, p.u_rs, nrows, tid);
+                    stage_tile<T, CPC, NT>(s + SM::kTile, db + (int64_t)tb * p.d_rs, p.d_rs, nrows, tid);
+                    if (HAS_Z) stage_tile<T, CPC, NT>(s + 2 * SM::kTile, zb + (int64_t)tb * p.z_rs, p.z_rs, nrows, tid);
+                    stage_tile<T, kNState, NT>(s + NTILE * SM::kTile, Bb + (int64_t)tb * p.B_rs, p.B_rs, nrows, tid);
+                    stage_tile<T, kNState, NT>(s + NTILE * SM::kTile + SM::kBCRaw, Cb + (int64_t)tb * p.C_rs, p.C_rs, nrows, tid);
                 }
             }
             cp_async_commit();
@@ -401,7 +392,7 @@ static void launch_fwd_v4_cpc(const ScanParams &p, const ChainSched &cs, bool ha
     }
 }
 
-// called by the chained-kernel dispatch (selscan_v2_fwd.cu) with cpc = cs.nblk's channel-block width
+// called by the chained-kernel dispatch (selscan_chain_host.cu) with cpc = cs.nblk's channel-block width
 template <typename T>
 void v4_launch_fwd_kernel(const ScanParams &p, const ChainSched &cs, int cpc, bool has_z, int cpb, cudaStream_t st) {
     if (cpc == 64) launch_fwd_v4_cpc<T, 64>(p, cs, has_z, cpb, st);

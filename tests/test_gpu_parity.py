@@ -136,7 +136,8 @@ def test_pscan_does_not_mutate_inputs_and_is_linear_in_x():
 
 # --------------------------------------------------------------------------------------- fused selective scan
 @pytest.mark.parametrize("B,L,ED", [(2, 1, 32), (1, 5, 40), (2, 16, 64), (2, 17, 32), (3, 37, 96), (2, 64, 33),
-                                    (2, 300, 64), (2, 1858, 64)])
+                                    (2, 300, 64), (2, 1858, 64),
+                                    (1, 2100, 40), (2, 1858, 1000)])   # ED % 32 != 0 with few warps: generic kernels split L
 def test_selscan_fp32_vs_oracle(B, L, ED):
     d = make_scan_inputs(B, L, ED, seed=B * 1000 + L)
     compare(run_fused(d, torch.float32), oracle_fused(d, torch.float32), TOL[torch.float32])
@@ -160,12 +161,13 @@ def test_selscan_half_precision(dtype):
     compare(run_fused(d, dtype), oracle_fused(d, dtype), TOL[dtype])
 
 
-# ---- the chained kernels (selscan_v4_fwd / selscan_v2_{fwd,bwd}): selected when B * ED / 32 >= 296 warps -----------------
+# ---- the chained kernels (selscan_v4_fwd.cu / selscan_chain_bwd.cu), serving ED % 32 == 0; their L-segments wait on each
+# ---- other when B * ED / 32 >= 296 warps ------------------------------------------------------------------------------------
 @pytest.mark.parametrize("B,L,ED", [(24, 203, 512),    # ragged L (not a multiple of 8 / 16), one segment
                                     (20, 1000, 512),   # every chain has a CTA of its own: one unit per chain, ragged tail
                                     (40, 400, 1024),   # more chains (640) than resident CTAs: three chained L-segments
                                     (10, 1170, 4096),  # same, 64-channel blocks on both sides, ragged last segment
-                                    (24, 203, 480),    # ED % 64 == 32: v2 forward (32-channel blocks)
+                                    (24, 203, 480),    # ED % 64 == 32: 32-channel blocks on both sides
                                     (40, 16, 256), (40, 1, 256), (40, 9, 256)])   # shorter than one chunk
 def test_selscan_chained_fp32_vs_oracle(B, L, ED):
     d = make_scan_inputs(B, L, ED, seed=B + L + ED)
@@ -209,7 +211,8 @@ def test_selscan_chained_strided_views_and_inference():
 
 
 def test_selscan_l_split_path():
-    """Few channels, long L -> plan_segments() splits L; carries are combined from segment summaries."""
+    """Few channels, long L -> the chained kernels run independent L-segments whose carries come from the summary and
+    combine passes."""
     d = make_scan_inputs(1, 4096, 64, seed=3)
     compare(run_fused(d, torch.float32), oracle_fused(d, torch.float32), TOL[torch.float32])
     d = make_scan_inputs(2, 1858, 32, seed=4)   # production-like L, ragged last chunk, split
