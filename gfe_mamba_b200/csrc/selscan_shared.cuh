@@ -84,19 +84,29 @@ __device__ __forceinline__ float2 ex2_poly2(float2 x) {
 }
 
 // Branch-free softplus of two values (one formulation for every x, so it can be interleaved with other work):
-// softplus(x) = max(x, 0) + log1p(w), w = exp(-|x|) in (0, 1], with log1p(w) = ln2 * lg2(1 + w) on the MUFU pipe: 1 + w is in
-// [1, 2], where lg2.approx is accurate to 2^-22.6 ABSOLUTE, i.e. softplus to ~1.2e-7 absolute -- what the max-normalised
-// tolerances of the path need -- for 6 instead of the 15 FP32-pipe instructions per pair of a 2 atanh(w / (2 + w)) series
-// (the item phases are issue-bound, not MUFU-bound).  Optionally sig = sigmoid(x) = d softplus / dx.
+// softplus(x) = max(x, 0) + log1p(w), w = exp(-|x|) in (0, 1], log1p(w) = 2 atanh(w / (2 + w)) with six odd terms
+// (s^2 <= 1/9: relative error < 1e-6 for every x; x > 20 returns x to fp32 rounding, the torch threshold).
+// Not ln2 * lg2(1 + w): for x < 0 that rounds 1 + w to fp32 before the logarithm and lg2.approx is accurate to 2^-22.6 only
+// in ABSOLUTE terms, so delta = softplus(x) loses all relative accuracy below x ~ -10 (100 % below -16.6) -- the step sizes
+// of long-memory channels, where the generic and decode kernels (softplus_only, the same series) stay exact.
+// Optionally sig = sigmoid(x) = d softplus / dx.
 template <bool WANT_SIG>
 __device__ __forceinline__ float2 softplus_pair(float2 x, float2 &sig) {
     const float2 w = ex2_2(make_float2(fabsf(x.x) * -kLog2e, fabsf(x.y) * -kLog2e));
-    const float2 d = fadd2(w, splat2(1.0f));
+    const float2 d = fadd2(w, splat2(2.0f));
+    const float2 s = fmul2(w, make_float2(rcp_approx(d.x), rcp_approx(d.y)));
+    const float2 s2 = fmul2(s, s);
+    float2 p = ffma2(s2, splat2(2.0f / 11.0f), splat2(2.0f / 9.0f));
+    p = ffma2(p, s2, splat2(2.0f / 7.0f));
+    p = ffma2(p, s2, splat2(2.0f / 5.0f));
+    p = ffma2(p, s2, splat2(2.0f / 3.0f));
+    p = ffma2(p, s2, splat2(2.0f));
+    const float2 r = fmul2(s, p);
     if (WANT_SIG) {
-        const float2 q = make_float2(rcp_approx(d.x), rcp_approx(d.y));   // sigmoid(|x|)
+        const float2 q = make_float2(rcp_approx(1.0f + w.x), rcp_approx(1.0f + w.y));   // sigmoid(|x|)
         sig = make_float2(x.x >= 0.f ? q.x : w.x * q.x, x.y >= 0.f ? q.y : w.y * q.y);
     }
-    return make_float2(fmaf(kLn2, lg2_approx(d.x), fmaxf(x.x, 0.f)), fmaf(kLn2, lg2_approx(d.y), fmaxf(x.y, 0.f)));
+    return make_float2(fmaxf(x.x, 0.f) + r.x, fmaxf(x.y, 0.f) + r.y);
 }
 
 // Element type of the chained kernels' state checkpoints: fp32, except bf16 for bf16 activations (half the checkpoint
