@@ -74,6 +74,8 @@ SIGNATURES = {
     "gfe_add_mean_pool_workspace_bytes": (c_sz, [ctypes.c_int] * 3),
     "gfe_add_mean_pool_fwd": (ctypes.c_int, [c_vp, c_vp, c_vp] + [ctypes.c_int] * 4 + [c_vp, c_sz, c_vp]),
     "gfe_mean_pool_bwd": (ctypes.c_int, [c_vp, c_vp] + [ctypes.c_int] * 4 + [c_vp]),
+    "gfe_add_mean_pool_fwd_mixed": (ctypes.c_int, [c_vp, c_vp, c_vp] + [ctypes.c_int] * 5 + [c_vp, c_sz, c_vp]),
+    "gfe_mean_pool_bwd_mixed": (ctypes.c_int, [c_vp, c_vp, c_vp] + [ctypes.c_int] * 5 + [c_vp]),
     "gfe_clip_adam_chunk_elems": (ctypes.c_int, []),
     "gfe_clip_adam_step": (ctypes.c_int, [c_vp] * 11 + [ctypes.c_int] * 2 + [ctypes.c_float] * 5 + [ctypes.c_int] * 2 + [c_vp]),
     "gfe_timing_enable": (ctypes.c_int, [ctypes.c_int]),

@@ -5,8 +5,11 @@
 // and the stack's last operation is the residual add of its last layer (mamba.py:103).  Unfused that is one pass writing the
 // (B, L, D) sum and one pass reading it back; here the two (B, L, D) operands are read once and only (B, D) is written:
 //   fwd   out[b, d] = (1 / L) * sum_t (a[b, t, d] + r[b, t, d])          reads 2 B L D, writes B D
-//   bwd   da[b, t, d] = dr[b, t, d] = dout[b, d] / L                      writes B L D once (both operands share it)
+//   bwd   da[b, t, d] = dr[b, t, d] = dout[b, d] / L                      writes B L D per operand that needs it
 // Deterministic: per-(row tile) partial sums in fp32, added in tile order by a second tiny kernel.
+// The operands may differ in element type the way addnorm.cu's do: under autocast the last branch (out_proj's output) is
+// 16-bit and the residual stream fp32.  Then out and dout are fp32, as torch promotes a + r, every element is read in its own
+// type (no cast pass over (B, L, D)), and backward writes each operand's gradient in its own type in the same pass.
 #include "common.cuh"
 
 namespace gfe {
@@ -14,15 +17,19 @@ namespace gfe {
 constexpr int kPoolTile = 64;   // rows per partial sum
 constexpr int kPoolNT = 128;
 
-template <typename T>
-__global__ void __launch_bounds__(kPoolNT) add_mean_pool_partial_kernel(const T *__restrict__ a, const T *__restrict__ r, float *__restrict__ part,
-                                                                         int L, int D, int ntile) {
+// element type of out / dout: the operands' when they agree, else fp32 (the other one is 16-bit)
+template <typename TA, typename TR> struct PoolOut { using type = float; };
+template <typename T> struct PoolOut<T, T> { using type = T; };
+
+template <typename TA, typename TR>
+__global__ void __launch_bounds__(kPoolNT) add_mean_pool_partial_kernel(const TA *__restrict__ a, const TR *__restrict__ r,
+                                                                         float *__restrict__ part, int L, int D, int ntile) {
     const int d = blockIdx.x * kPoolNT + threadIdx.x;
     const int tile = blockIdx.y, b = blockIdx.z;
     if (d >= D) return;
     const int t0 = tile * kPoolTile, t1 = min(L, t0 + kPoolTile);
-    const T *pa = a + ((size_t)b * L + t0) * D + d;
-    const T *pr = r ? r + ((size_t)b * L + t0) * D + d : nullptr;
+    const TA *pa = a + ((size_t)b * L + t0) * D + d;
+    const TR *pr = r ? r + ((size_t)b * L + t0) * D + d : nullptr;
     float acc0 = 0.f, acc1 = 0.f;
     int t = t0;
     for (; t + 1 < t1; t += 2) {   // two independent chains: the loads of both rows are in flight together
@@ -44,33 +51,47 @@ __global__ void __launch_bounds__(kPoolNT) add_mean_pool_final_kernel(const floa
     out[(size_t)b * D + d] = from_f<T>(acc / (float)L);
 }
 
-template <typename T>
-__global__ void __launch_bounds__(kPoolNT) mean_pool_bwd_kernel(const T *__restrict__ dout, T *__restrict__ da, int L, int D) {
+// dout / L rounded once per operand type; dr == nullptr: only a's gradient (no r, or r needs none, or the caller shares da)
+template <typename TA, typename TR>
+__global__ void __launch_bounds__(kPoolNT) mean_pool_bwd_kernel(const typename PoolOut<TA, TR>::type *__restrict__ dout,
+                                                                TA *__restrict__ da, TR *__restrict__ dr, int L, int D) {
     const int d = blockIdx.x * kPoolNT + threadIdx.x;
     const int tile = blockIdx.y, b = blockIdx.z;
     if (d >= D) return;
-    const T v = from_f<T>(to_f(dout[(size_t)b * D + d]) / (float)L);
+    const float g = to_f(dout[(size_t)b * D + d]) / (float)L;
+    const TA va = from_f<TA>(g);
+    const TR vr = from_f<TR>(g);
     const int t0 = tile * kPoolTile, t1 = min(L, t0 + kPoolTile);
-    T *p = da + ((size_t)b * L + t0) * D + d;
-    for (int t = t0; t < t1; ++t, p += D) st_stream(p, v);
+    const size_t o = ((size_t)b * L + t0) * D + d;
+    TA *p = da + o;
+    for (int t = t0; t < t1; ++t, p += D) st_stream(p, va);
+    if (dr != nullptr) {
+        TR *q = dr + o;
+        for (int t = t0; t < t1; ++t, q += D) st_stream(q, vr);
+    }
 }
 
-template <typename T>
-static int pool_fwd_t(const void *a, const void *r, void *out, int B, int L, int D, float *part, cudaStream_t st) {
-    const int ntile = (L + kPoolTile - 1) / kPoolTile;
-    { ScopedKernelTimer tm(K_POOL_FWD, st);
-      add_mean_pool_partial_kernel<T><<<dim3((D + kPoolNT - 1) / kPoolNT, ntile, B), kPoolNT, 0, st>>>(
-          reinterpret_cast<const T *>(a), reinterpret_cast<const T *>(r), part, L, D, ntile);
-      add_mean_pool_final_kernel<T><<<dim3((D + kPoolNT - 1) / kPoolNT, B), kPoolNT, 0, st>>>(part, reinterpret_cast<T *>(out), L, D, ntile); }
-    return check_launch("add_mean_pool_fwd");
-}
+template <typename T> struct PoolTag { using type = T; };
 
-template <typename T>
-static int pool_bwd_t(const void *dout, void *da, int B, int L, int D, cudaStream_t st) {
-    const int ntile = (L + kPoolTile - 1) / kPoolTile;
-    { ScopedKernelTimer tm(K_POOL_BWD, st);
-      mean_pool_bwd_kernel<T><<<dim3((D + kPoolNT - 1) / kPoolNT, ntile, B), kPoolNT, 0, st>>>(reinterpret_cast<const T *>(dout), reinterpret_cast<T *>(da), L, D); }
-    return check_launch("mean_pool_bwd");
+// (a, r) element types the kernels are compiled for: equal, or fp32 next to a 16-bit type in either order
+template <typename F>
+static int pool_dispatch(int a_dtype, int r_dtype, const char *what, F &&f) {
+    if (a_dtype == r_dtype) {
+        switch (a_dtype) {
+            case GFE_F32: return f(PoolTag<float>{}, PoolTag<float>{});
+            case GFE_BF16: return f(PoolTag<__nv_bfloat16>{}, PoolTag<__nv_bfloat16>{});
+            case GFE_F16: return f(PoolTag<__half>{}, PoolTag<__half>{});
+            default: break;
+        }
+    } else if (a_dtype == GFE_F32) {
+        if (r_dtype == GFE_BF16) return f(PoolTag<float>{}, PoolTag<__nv_bfloat16>{});
+        if (r_dtype == GFE_F16) return f(PoolTag<float>{}, PoolTag<__half>{});
+    } else if (r_dtype == GFE_F32) {
+        if (a_dtype == GFE_BF16) return f(PoolTag<__nv_bfloat16>{}, PoolTag<float>{});
+        if (a_dtype == GFE_F16) return f(PoolTag<__half>{}, PoolTag<float>{});
+    }
+    set_error("%s: unsupported dtype pair (a %d, r %d)", what, a_dtype, r_dtype);
+    return GFE_ERR_DTYPE;
 }
 
 }  // namespace gfe
@@ -82,30 +103,50 @@ GFE_API size_t gfe_add_mean_pool_workspace_bytes(int B, int L, int D) {
     return (size_t)B * ((L + gfe::kPoolTile - 1) / gfe::kPoolTile) * D * sizeof(float);
 }
 
-GFE_API int gfe_add_mean_pool_fwd(const void *a, const void *r, void *out, int B, int L, int D, int dtype, void *ws, size_t ws_bytes,
-                                  void *stream) {
+GFE_API int gfe_add_mean_pool_fwd_mixed(const void *a, const void *r, void *out, int B, int L, int D, int a_dtype, int r_dtype,
+                                        void *ws, size_t ws_bytes, void *stream) {
     using namespace gfe;
     if (!a || !out || B <= 0 || L <= 0 || D <= 0 || B > 65535) { set_error("add_mean_pool_fwd: bad argument"); return GFE_ERR_ARG; }
     if (!ws || ws_bytes < gfe_add_mean_pool_workspace_bytes(B, L, D)) { set_error("add_mean_pool_fwd: workspace too small"); return GFE_ERR_WORKSPACE; }
+    if (!r) r_dtype = a_dtype;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    switch (dtype) {
-        case GFE_F32: return pool_fwd_t<float>(a, r, out, B, L, D, reinterpret_cast<float *>(ws), st);
-        case GFE_BF16: return pool_fwd_t<__nv_bfloat16>(a, r, out, B, L, D, reinterpret_cast<float *>(ws), st);
-        case GFE_F16: return pool_fwd_t<__half>(a, r, out, B, L, D, reinterpret_cast<float *>(ws), st);
-        default: set_error("add_mean_pool_fwd: bad dtype %d", dtype); return GFE_ERR_DTYPE;
-    }
+    float *part = reinterpret_cast<float *>(ws);
+    const int ntile = (L + kPoolTile - 1) / kPoolTile;
+    return pool_dispatch(a_dtype, r_dtype, "add_mean_pool_fwd", [&](auto ta, auto tr) {
+        using TA = typename decltype(ta)::type;
+        using TR = typename decltype(tr)::type;
+        using TO = typename PoolOut<TA, TR>::type;
+        { ScopedKernelTimer tm(K_POOL_FWD, st);
+          add_mean_pool_partial_kernel<TA, TR><<<dim3((D + kPoolNT - 1) / kPoolNT, ntile, B), kPoolNT, 0, st>>>(
+              reinterpret_cast<const TA *>(a), reinterpret_cast<const TR *>(r), part, L, D, ntile);
+          add_mean_pool_final_kernel<TO><<<dim3((D + kPoolNT - 1) / kPoolNT, B), kPoolNT, 0, st>>>(part, reinterpret_cast<TO *>(out), L, D, ntile); }
+        return check_launch("add_mean_pool_fwd");
+    });
 }
 
-GFE_API int gfe_mean_pool_bwd(const void *dout, void *da, int B, int L, int D, int dtype, void *stream) {
+GFE_API int gfe_add_mean_pool_fwd(const void *a, const void *r, void *out, int B, int L, int D, int dtype, void *ws, size_t ws_bytes,
+                                  void *stream) {
+    return gfe_add_mean_pool_fwd_mixed(a, r, out, B, L, D, dtype, dtype, ws, ws_bytes, stream);
+}
+
+GFE_API int gfe_mean_pool_bwd_mixed(const void *dout, void *da, void *dr, int B, int L, int D, int a_dtype, int r_dtype, void *stream) {
     using namespace gfe;
     if (!dout || !da || B <= 0 || L <= 0 || D <= 0 || B > 65535) { set_error("mean_pool_bwd: bad argument"); return GFE_ERR_ARG; }
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    switch (dtype) {
-        case GFE_F32: return pool_bwd_t<float>(dout, da, B, L, D, st);
-        case GFE_BF16: return pool_bwd_t<__nv_bfloat16>(dout, da, B, L, D, st);
-        case GFE_F16: return pool_bwd_t<__half>(dout, da, B, L, D, st);
-        default: set_error("mean_pool_bwd: bad dtype %d", dtype); return GFE_ERR_DTYPE;
-    }
+    const int ntile = (L + kPoolTile - 1) / kPoolTile;
+    return pool_dispatch(a_dtype, r_dtype, "mean_pool_bwd", [&](auto ta, auto tr) {
+        using TA = typename decltype(ta)::type;
+        using TR = typename decltype(tr)::type;
+        using TO = typename PoolOut<TA, TR>::type;
+        { ScopedKernelTimer tm(K_POOL_BWD, st);
+          mean_pool_bwd_kernel<TA, TR><<<dim3((D + kPoolNT - 1) / kPoolNT, ntile, B), kPoolNT, 0, st>>>(
+              reinterpret_cast<const TO *>(dout), reinterpret_cast<TA *>(da), reinterpret_cast<TR *>(dr), L, D); }
+        return check_launch("mean_pool_bwd");
+    });
+}
+
+GFE_API int gfe_mean_pool_bwd(const void *dout, void *da, int B, int L, int D, int dtype, void *stream) {
+    return gfe_mean_pool_bwd_mixed(dout, da, nullptr, B, L, D, dtype, dtype, stream);
 }
 
 }  // extern "C"

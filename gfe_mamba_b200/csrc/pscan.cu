@@ -13,6 +13,8 @@
 // paying a second pass.  Only when even
 // that cannot fill the GPU (B*D*N below ~25 k elements, e.g. one long sequence with few channels) is L split into segments:
 // pass 1 reduces each segment to its (product of A, local end state) pair, pass 2 starts each segment from the combined carry.
+// The split only ever follows the fall to (1, 32), so the summary passes exist as (1, 32) alone; misaligned operands also run
+// (1, 32).  Compiled: forward (4, 16), (1, 32), (1, 32) summary; backward (4, 8), (2, 16), (1, 32), (1, 32) summary.
 #include "common.cuh"
 
 namespace gfe {
@@ -387,16 +389,14 @@ GFE_API int gfe_pscan_fwd(const float *A, const float *X, float *H, int B, int L
     p.segS = reinterpret_cast<float *>(reinterpret_cast<char *>(ws) + need / 2);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     const bool al = aligned16(A) && aligned16(X) && aligned16(H) && (need == 0 || aligned16(ws));
-    const int V = al ? pl.V : 1;                                  // rows of D*N fp32 keep 8 / 16-byte alignment when DN % V == 0
+    // The plan only splits L once it has fallen to (1, 32), so the split runs the scalar kernels whatever the alignment;
+    // otherwise (4, 16) when the operands allow it (rows of D*N fp32 keep 16-byte alignment when DN % 4 == 0)
+    const int V = (al && pl.nseg == 1) ? pl.V : 1;
     const int64_t nvec = DN / V;
     const dim3 block(128), grid((unsigned)ceil_div64(nvec, 128), pl.nseg, B);
-    const bool deep = pl.U == 16;   // (4, 16): twice the loads in flight at the widest request
     if (pl.nseg > 1) {
         { ScopedKernelTimer tm(K_PSCAN_FWD_SUMMARY, st);
-          if (V == 4 && deep) pscan_fwd_kernel<4, 16, true><<<grid, block, 0, st>>>(p);
-          else if (V == 4) pscan_fwd_kernel<4, 8, true><<<grid, block, 0, st>>>(p);
-          else if (V == 2) pscan_fwd_kernel<2, 16, true><<<grid, block, 0, st>>>(p);
-          else pscan_fwd_kernel<1, 32, true><<<grid, block, 0, st>>>(p); }
+          pscan_fwd_kernel<1, 32, true><<<grid, block, 0, st>>>(p); }
         rc = check_launch("pscan_fwd_summary");
         if (rc != GFE_OK) return rc;
     }
@@ -409,9 +409,7 @@ GFE_API int gfe_pscan_fwd(const float *A, const float *X, float *H, int B, int L
         return check_launch("pscan_fwd (chained)");
     }
     { ScopedKernelTimer tm(K_PSCAN_FWD, st);
-      if (V == 4 && deep) pscan_fwd_kernel<4, 16, false><<<grid, block, 0, st>>>(p);
-      else if (V == 4) pscan_fwd_kernel<4, 8, false><<<grid, block, 0, st>>>(p);
-      else if (V == 2) pscan_fwd_kernel<2, 16, false><<<grid, block, 0, st>>>(p);
+      if (V == 4) pscan_fwd_kernel<4, 16, false><<<grid, block, 0, st>>>(p);
       else pscan_fwd_kernel<1, 32, false><<<grid, block, 0, st>>>(p); }
     return check_launch("pscan_fwd");
 }
@@ -432,15 +430,13 @@ GFE_API int gfe_pscan_bwd(const float *A, const float *H, const float *dH, float
     p.segS = reinterpret_cast<float *>(reinterpret_cast<char *>(ws) + need / 2);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     const bool al = aligned16(A) && aligned16(H) && aligned16(dH) && aligned16(dA) && aligned16(dX) && (need == 0 || aligned16(ws));
-    const int V = al ? pl.V : 1;
+    const int V = (al && pl.nseg == 1) ? pl.V : 1;   // as forward: the L-split only follows the fall to (1, 32)
     const int64_t nvec = DN / V;
     const dim3 block(128);
     if (pl.nseg > 1) {
         const dim3 grid((unsigned)ceil_div64(nvec, 128), pl.nseg - 1, B);
         { ScopedKernelTimer tm(K_PSCAN_BWD_SUMMARY, st);
-          if (V == 4) pscan_bwd_kernel<4, 8, true><<<grid, block, 0, st>>>(p);
-          else if (V == 2) pscan_bwd_kernel<2, 16, true><<<grid, block, 0, st>>>(p);
-          else pscan_bwd_kernel<1, 32, true><<<grid, block, 0, st>>>(p); }
+          pscan_bwd_kernel<1, 32, true><<<grid, block, 0, st>>>(p); }
         rc = check_launch("pscan_bwd_summary");
         if (rc != GFE_OK) return rc;
     }

@@ -451,6 +451,9 @@ class _AddRMSNormFn(torch.autograd.Function):
             nat.check(l.gfe_add_rmsnorm_fwd_mixed(_ptr(x_), _ptr(a_), _ptr(w_), _ptr(resid if a_ is not None else None), _ptr(y),
                                                   _ptr(rstd), rows, D, float(eps), _DT[x.dtype], _DT[io_dtype], _stream(dev)),
                       "add_rmsnorm_fwd")
+        # an output nothing downstream used arrives in backward as None, not as a zero-filled (rows, D) tensor: an unused
+        # resid runs the kernels without the dres stream, an unused y reads zeros
+        ctx.set_materialize_grads(False)
         if need_grad:
             ctx.save_for_backward(resid, w_, rstd)
             ctx.a_dtype = None if a is None else a.dtype
@@ -507,42 +510,57 @@ def add_rmsnorm(x: torch.Tensor, a: Optional[torch.Tensor], weight: torch.Tensor
 # --------------------------------------------------------- final residual add + mean over L
 class _AddMeanPoolFn(torch.autograd.Function):
     """mean over dim 1 of (a + r) -- the last residual add of the stack (cross_atten/mamba.py:103) fused with the head's
-    pooling (cross_atten/mamba_transformer.py:123).  SURVEY 8f rank 4."""
+    pooling (cross_atten/mamba_transformer.py:123).  SURVEY 8f rank 4.
+
+    a and r may differ in dtype as torch allows: fp32 next to bf16 / fp16, in either order (the stack under autocast: a 16-bit
+    last branch on the fp32 residual stream).  Each operand is read in its own dtype, the output is fp32 like ``a + r`` in torch,
+    and each operand's gradient comes out in its own dtype from one backward pass."""
 
     @staticmethod
     def forward(ctx, a, r):
         dev = _require_cuda(a, r)
         if a.dim() != 3 or (r is not None and r.shape != a.shape):
             raise ValueError("add_mean_pool: (B, L, D) operands of identical shape expected")
-        if a.dtype not in _DT:
-            raise TypeError(f"add_mean_pool: unsupported dtype {a.dtype}")
+        rdt = a.dtype if r is None else r.dtype
+        if a.dtype not in _DT or rdt not in _DT:
+            raise TypeError(f"add_mean_pool: unsupported dtype {a.dtype if a.dtype not in _DT else rdt}")
+        if rdt != a.dtype and torch.float32 not in (a.dtype, rdt):
+            raise TypeError(f"add_mean_pool: operands in {a.dtype} and {rdt}: only fp32 may meet a 16-bit dtype")
+        out_dt = torch.promote_types(a.dtype, rdt)
         B, L, D = a.shape
         a_ = a.detach().contiguous()
-        r_ = None if r is None else r.detach().to(a.dtype).contiguous()
-        out = torch.empty((B, 1, D), dtype=a.dtype, device=dev)
+        r_ = None if r is None else r.detach().contiguous()
+        out = torch.empty((B, 1, D), dtype=out_dt, device=dev)
         l = nat.lib()
         with torch.cuda.device(dev):
             nws = l.gfe_add_mean_pool_workspace_bytes(B, L, D)
             ws = _bytes(nws, dev)
-            nat.check(l.gfe_add_mean_pool_fwd(_ptr(a_), _ptr(r_), _ptr(out), B, L, D, _DT[a.dtype], _ptr(ws), nws, _stream(dev)),
-                      "add_mean_pool_fwd")
-        ctx.shape, ctx.has_r = (B, L, D), r is not None
+            nat.check(l.gfe_add_mean_pool_fwd_mixed(_ptr(a_), _ptr(r_), _ptr(out), B, L, D, _DT[a.dtype], _DT[rdt], _ptr(ws), nws,
+                                                    _stream(dev)), "add_mean_pool_fwd")
+        ctx.shape, ctx.has_r, ctx.dtypes = (B, L, D), r is not None, (a.dtype, rdt, out_dt)
         return out
 
     @staticmethod
     def backward(ctx, dout):
         B, L, D = ctx.shape
+        adt, rdt, out_dt = ctx.dtypes
         dev = dout.device
-        d_ = dout.detach().contiguous()
-        da = torch.empty((B, L, D), dtype=d_.dtype, device=dev)
+        d_ = dout.detach().to(out_dt).contiguous()
+        da = torch.empty((B, L, D), dtype=adt, device=dev)
+        # equal dtypes: both operands share one gradient tensor; else r's own, written by the same pass
+        dr = torch.empty((B, L, D), dtype=rdt, device=dev) if (ctx.has_r and rdt != adt and ctx.needs_input_grad[1]) else None
         l = nat.lib()
         with torch.cuda.device(dev):
-            nat.check(l.gfe_mean_pool_bwd(_ptr(d_), _ptr(da), B, L, D, _DT[d_.dtype], _stream(dev)), "mean_pool_bwd")
-        return da, (da if ctx.has_r else None)
+            nat.check(l.gfe_mean_pool_bwd_mixed(_ptr(d_), _ptr(da), _ptr(dr), B, L, D, _DT[adt], _DT[rdt], _stream(dev)),
+                      "mean_pool_bwd")
+        if not ctx.has_r:
+            return da, None
+        return da, (dr if rdt != adt else da)
 
 
 def add_mean_pool(a: torch.Tensor, r: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """(B, 1, D) = mean over L of (a + r); a, r: (B, L, D).  Equals ``torch.mean(a + r, dim=1, keepdim=True)``."""
+    """(B, 1, D) = mean over L of (a + r); a, r: (B, L, D).  Equals ``torch.mean(a + r, dim=1, keepdim=True)``, dtype included:
+    fp32 with bf16 / fp16 gives fp32; other dtype mixes raise TypeError."""
     return _AddMeanPoolFn.apply(a, r)
 
 

@@ -11,6 +11,10 @@ Host-side mirror of the reference training loop's tail (classify_mamba.py:64, 10
 
 ``ClipAdam(all_params, lr=1e-4, max_norm=1.0).step()`` does all of it in three kernel launches for the whole list,
 whatever the number of parameter tensors, and is CUDA-graph capturable (the step counter lives on the device).
+
+``state_dict()`` / ``load_state_dict()`` use torch.optim.Adam's format (``exp_avg``, ``exp_avg_sq`` and a float32 ``step`` per
+parameter), so a run resumes with its moments and bias corrections, and the state dicts of the two optimisers load into each
+other.
 """
 from __future__ import annotations
 
@@ -42,7 +46,14 @@ class ClipAdam(torch.optim.Optimizer):
         defaults = dict(lr=lr, betas=betas, eps=eps, max_norm=max_norm, per_parameter_clip=per_parameter_clip,
                         zero_grad=zero_grad)
         super().__init__(params, defaults)
-        self._tables = {}   # group index -> (key, table dict)
+        self._tables = {}        # group index -> (key, table dict)
+        self._loaded_steps = {}  # group index -> step counter loaded before the group's table existed
+
+    def __setstate__(self, state):
+        super().__setstate__(state)
+        for group in self.param_groups:   # groups of a torch.optim.Adam state dict lack ClipAdam's own settings
+            for k, v in self.defaults.items():
+                group.setdefault(k, v)
 
     # ------------------------------------------------------------------------------------------------
     @staticmethod
@@ -56,8 +67,15 @@ class ClipAdam(torch.optim.Optimizer):
             tensor_chunk0.append(len(chunk_tensor))
         return chunk_tensor, chunk_start, tensor_chunk0
 
+    def _key(self, params: List[torch.Tensor]):
+        """The addresses a table holds: parameters, gradients and -- so that a table never writes through the addresses of
+        replaced state tensors -- the moment buffers."""
+        return tuple((p.data_ptr(), p.grad.data_ptr(), p.numel(),
+                      *(t.data_ptr() if t is not None else 0 for t in (self.state[p].get("exp_avg"), self.state[p].get("exp_avg_sq"))))
+                     for p in params)
+
     def _table(self, gi: int, params: List[torch.Tensor]):
-        key = tuple((p.data_ptr(), p.grad.data_ptr(), p.numel()) for p in params)
+        key = self._key(params)
         cached = self._tables.get(gi)
         if cached is not None and cached[0] == key:
             return cached[1]
@@ -70,9 +88,10 @@ class ClipAdam(torch.optim.Optimizer):
                     or not p.is_contiguous() or not p.grad.is_contiguous():
                 raise RuntimeError("ClipAdam: parameters and gradients must be contiguous fp32 CUDA tensors on one device")
             st = self.state[p]
-            if len(st) == 0:
+            if "exp_avg" not in st:
                 st["exp_avg"] = torch.zeros_like(p, memory_format=torch.preserve_format)
                 st["exp_avg_sq"] = torch.zeros_like(p, memory_format=torch.preserve_format)
+        key = self._key(params)   # with the moment buffers just created
         chunk = nat.lib().gfe_clip_adam_chunk_elems()
         numels = [p.numel() for p in params]
         ct, cs, tc0 = self.plan_chunks(numels, chunk)
@@ -92,10 +111,70 @@ class ClipAdam(torch.optim.Optimizer):
             coef=torch.empty(len(params), dtype=torch.float32, device=dev),
             ntensors=len(params), nchunks=len(ct), dev=dev,
         )
-        cached_step = None if cached is None else cached[1]["step"]
-        tb["step"] = cached_step if cached_step is not None else torch.zeros(1, dtype=torch.int32, device=dev)
+        if gi in self._loaded_steps:
+            tb["step"] = torch.full((1,), self._loaded_steps.pop(gi), dtype=torch.int32, device=dev)
+        elif cached is not None:
+            tb["step"] = cached[1]["step"]
+        else:
+            tb["step"] = torch.zeros(1, dtype=torch.int32, device=dev)
         self._tables[gi] = (key, tb)
         return tb
+
+    def _group_step(self, gi: int) -> int:
+        cached = self._tables.get(gi)
+        if cached is not None:
+            return int(cached[1]["step"].item())
+        return self._loaded_steps.get(gi, 0)
+
+    def state_dict(self):
+        """torch.optim.Adam's layout: every parameter with state carries its group's step counter as a float32 CPU scalar
+        ``step``, and every group ``weight_decay = 0`` (ClipAdam has none), so that torch.optim.Adam can load the dict."""
+        sd = super().state_dict()
+        for gi, g in enumerate(sd["param_groups"]):
+            g.setdefault("weight_decay", 0.0)
+            step = None
+            for i in g["params"]:
+                if i in sd["state"]:
+                    if step is None:
+                        step = torch.tensor(float(self._group_step(gi)), dtype=torch.float32)
+                    sd["state"][i] = {**sd["state"][i], "step": step.clone()}   # a copy: the live state keeps no "step"
+        return sd
+
+    @torch.no_grad()
+    def load_state_dict(self, state_dict):
+        """Loads a ClipAdam or torch.optim.Adam state dict.  The moments are copied INTO the existing buffers and the device
+        step counter is overwritten, so the device tables -- and a CUDA graph captured over ``step`` -- stay valid.  The
+        parameters of one group share one step counter: a group whose parameters carry different steps raises ValueError.  A
+        group without any saved ``step`` restarts its bias correction."""
+        for g in state_dict["param_groups"]:
+            if g.get("weight_decay", 0) or g.get("amsgrad", False) or g.get("maximize", False):
+                raise ValueError("ClipAdam: weight decay, amsgrad and maximize are not supported")
+        steps = []
+        for g in state_dict["param_groups"]:
+            vals = {float(state_dict["state"][i]["step"]) for i in g["params"] if "step" in state_dict["state"].get(i, {})}
+            if len(vals) > 1:
+                raise ValueError(f"ClipAdam: one step counter serves a whole parameter group, but its parameters carry the "
+                                 f"steps {sorted(vals)}")
+            steps.append(int(vals.pop()) if vals else 0)
+        old = {p: (st["exp_avg"], st["exp_avg_sq"]) for p, st in self.state.items() if "exp_avg" in st}
+        super().load_state_dict(state_dict)
+        for p, (m, v) in old.items():
+            st = self.state[p]
+            for buf, new in ((m, st.get("exp_avg")), (v, st.get("exp_avg_sq"))):
+                if new is None:
+                    buf.zero_()
+                elif new is not buf:
+                    buf.copy_(new)
+            self.state[p] = {"exp_avg": m, "exp_avg_sq": v}
+        for st in self.state.values():
+            st.pop("step", None)
+        for gi, step in enumerate(steps):
+            cached = self._tables.get(gi)
+            if cached is not None:
+                cached[1]["step"].fill_(step)
+                self._loaded_steps.pop(gi, None)
+            else:
+                self._loaded_steps[gi] = step
 
     @torch.no_grad()
     def step(self, closure=None):

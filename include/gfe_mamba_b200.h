@@ -179,6 +179,14 @@ GFE_API size_t gfe_add_mean_pool_workspace_bytes(int B, int L, int D);
 GFE_API int gfe_add_mean_pool_fwd(const void *a, const void *r, void *out, int B, int L, int D, int dtype, void *ws, size_t ws_bytes,
                                   void *stream);
 GFE_API int gfe_mean_pool_bwd(const void *dout, void *da, int B, int L, int D, int dtype, void *stream);
+/* The same with an element type per operand: a in a_dtype, r in r_dtype (ignored when r is NULL).  The pairs are equal types,
+ * or GFE_F32 with GFE_BF16 / GFE_F16 in either order -- the stack under autocast, whose last branch is 16-bit next to the
+ * fp32 residual stream; any other pair returns GFE_ERR_DTYPE.  out and dout are in the promoted type (torch's a + r):
+ * GFE_F32 when the two differ.  bwd writes da in a_dtype and, when dr is not NULL, dr in r_dtype from the same pass. */
+GFE_API int gfe_add_mean_pool_fwd_mixed(const void *a, const void *r, void *out, int B, int L, int D, int a_dtype, int r_dtype,
+                                        void *ws, size_t ws_bytes, void *stream);
+GFE_API int gfe_mean_pool_bwd_mixed(const void *dout, void *da, void *dr, int B, int L, int D, int a_dtype, int r_dtype,
+                                    void *stream);
 
 /* ------------------------------------------- multi-tensor clip + Adam step --
  * One optimiser step for a whole parameter list in three launches; replaces the per-parameter loop

@@ -92,6 +92,19 @@ def test_add_rmsnorm_mixed_argument_validation_without_gpu():
                                          fake, 1 << 20, None) == -2
 
 
+def test_add_mean_pool_mixed_argument_validation_without_gpu():
+    """Pooling takes fp32 next to a 16-bit operand in either order; two different 16-bit dtypes are refused before any launch."""
+    from gfe_mamba_b200 import _native
+    lib = _native.lib()
+    fake = ctypes.c_void_p(4096)
+    ws = lib.gfe_add_mean_pool_workspace_bytes(2, 5, 8)
+    assert lib.gfe_add_mean_pool_fwd_mixed(fake, fake, fake, 2, 5, 8, _native.GFE_BF16, _native.GFE_F16, fake, ws, None) == -2
+    assert b"dtype pair" in lib.gfe_last_error_string()
+    assert lib.gfe_mean_pool_bwd_mixed(fake, fake, fake, 2, 5, 8, _native.GFE_F16, _native.GFE_BF16, None) == -2
+    assert lib.gfe_mean_pool_bwd_mixed(fake, fake, fake, 2, 5, 8, 7, _native.GFE_F32, None) == -2
+    assert lib.gfe_add_mean_pool_fwd_mixed(fake, None, fake, 2, 5, 8, _native.GFE_F32, _native.GFE_BF16, fake, ws - 4, None) == -4
+
+
 def test_argument_validation_without_gpu():
     """Bad arguments are rejected before any launch, with a message."""
     from gfe_mamba_b200 import _native

@@ -17,8 +17,13 @@ def _params(seed, shapes, scale):
 @pytest.mark.parametrize("max_norm", [1.0, None])
 def test_clip_adam_matches_torch(per_param, max_norm):
     from gfe_mamba_b200.optim import ClipAdam
-    shapes = [(1024, 16), (1024,), (2048, 512), (1024, 1, 4), (7,), (48 + 32, 1024), (4097,), (3, 5, 7)]
-    scale = [10.0, 1e-3, 1.0, 0.1, 5.0, 1e-2, 1.0, 100.0]   # some tensors clipped hard, some not at all
+    shapes = [(1024, 16), (1024,), (2048, 512), (1024, 1, 4), (7,), (48 + 32, 1024), (4097,), (3, 5, 7),
+              (0,), (1,), (33,), (5, 3), (8193,), (64, 64), (2,), (130, 3), (4096,)]
+    scale = [10.0, 1e-3, 1.0, 0.1, 5.0, 1e-2, 1.0, 100.0,   # some tensors clipped hard, some not at all
+             1.0, 50.0, 1e-4, 2.0, 0.5, 30.0, 1.0, 1e-2, 3.0]
+    # the per-tensor coef kernel runs one warp per tensor, 8 per CTA: 17 tensors need 3 CTAs (an empty one and a
+    # one-element one among them)
+    assert len(shapes) == len(scale) and -(-len(shapes) // 8) == 3
     ours, grads = _params(3, shapes, scale)
     ref = [torch.nn.Parameter(p.detach().clone()) for p in ours]
     opt_ref = torch.optim.Adam(ref, lr=1e-2)
