@@ -31,7 +31,9 @@ struct ScopedKernelTimer {   // brackets one launch with events when timing is e
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-constexpr int kNState = 16;     // d_state the fused kernels are compiled for
+constexpr int kNState = 16;     // d_state of the chained kernels (the generic kernels and the decode kernel also take 32 and 64)
+// d_state values the fused scan and decode kernels are compiled for; every other value is GFE_ERR_UNSUPPORTED
+static inline bool fused_d_state(int N) { return N == 16 || N == 32 || N == 64; }
 constexpr int kChunk = 16;      // time steps per register chunk == checkpoint interval
 constexpr int kMaxSeg = 256;    // max L-split factor (one long sequence sharded over 8 GPUs: 128 channels, 256 segments of 256 steps)
 constexpr int kCkptV2 = 8;      // checkpoint interval of the chained kernels: halves the register-resident history of backward

@@ -52,10 +52,11 @@ ChainPlan chain_bwd_plan(int B, int L, int ED) {
     return pl;
 }
 
-// The chained kernels serve every shape with ED % 32 == 0 (other widths take the generic kernels in selscan.cu).
-bool chain_applicable(int B, int L, int ED) {
+// The chained kernels serve every shape with d_state = 16 and ED % 32 == 0 (other widths and state sizes take the generic
+// kernels in selscan.cu).
+bool chain_applicable(int B, int L, int ED, int N) {
     (void)B; (void)L;
-    return ED % 32 == 0;
+    return N == kNState && ED % 32 == 0;
 }
 
 struct ChainLayout {

@@ -16,9 +16,9 @@ struct ScanParams {
     void *out;
     int64_t o_bs, o_rs;
     float *last_state;
-    float2 *ckpt;   // [B][nchunks][8][ED]
+    float2 *ckpt;   // [B][nchunks][N / 2][ED]
     void *ysave;    // [B][L][ED] activation dtype: y before the gate, lives behind ckpt (written by the chained kernels only)
-    float2 *seg_h;  // [B][nseg][8][ED]  segment-local end state (fwd) / start carry (bwd)
+    float2 *seg_h;  // [B][nseg][N / 2][ED]  segment-local end state (fwd) / start carry (bwd)
     float *seg_sd;  // [B][nseg][ED]     sum of delta over the segment
     // backward
     const void *dout;
@@ -26,14 +26,13 @@ struct ScanParams {
     void *du, *ddelta, *dz, *dBm, *dCm;
     int64_t du_bs, du_rs, dd_bs, dd_rs, dz_bs, dz_rs, dB_bs, dB_rs, dC_bs, dC_rs;
     float *dA_log, *dD, *ddt_bias;
-    float *part_bc;   // [G][B][L][32]   per-warp dB|dC rows
-    float *part_par;  // [B][nseg][18][ED]
+    float *part_bc;   // [G][B][L][2 N]   per-warp dB|dC rows
+    float *part_par;  // [B][nseg][N + 2][ED]
     int G;            // ceil(ED / 32)
-    int bc_interleaved;   // part_bc rows: 1 = {dB[n], dC[n]} pairs (chained backward), 0 = dB[16] | dC[16] (generic backward)
+    int bc_interleaved;   // part_bc rows: 1 = {dB[n], dC[n]} pairs (chained backward), 0 = dB[N] | dC[N] (generic backward)
 };
 
 constexpr int kPairs = kNState / 2;
-constexpr int kRedStride = 34;  // padded row of the reduced dB|dC tile (bank-conflict free float2 writes)
 
 // Dynamic chaining of L-segments (chained kernels): persistent CTAs draw (segment, batch row, channel block) units from an
 // atomic counter in segment-major order; a unit waits for the flag of its predecessor segment, reads the carried
@@ -221,7 +220,7 @@ struct ChainPlan {
 };
 ChainPlan chain_fwd_plan(int B, int L, int ED);
 ChainPlan chain_bwd_plan(int B, int L, int ED);
-bool chain_applicable(int B, int L, int ED);              // shape-only: both directions take the same decision
+bool chain_applicable(int B, int L, int ED, int N);       // shape-only: both directions take the same decision
 size_t chain_ckpt_state_bytes(int B, int L, int ED, int dtype);
 size_t chain_fwd_workspace_bytes(int B, int L, int ED);
 size_t chain_bwd_workspace_bytes(int B, int L, int ED);

@@ -29,7 +29,7 @@ __global__ void __launch_bounds__(128) conv1d_step_kernel(const T *xin, int64_t 
     if (K >= 2) cache[K - 2] = xnew;
 }
 
-template <typename T>
+template <typename T, int N>
 __global__ void __launch_bounds__(128) ssm_step_kernel(const T *u, int64_t u_bs, const T *delta, int64_t d_bs,
                                                        const T *z, int64_t z_bs, const T *Bm, int64_t B_bs,
                                                        const T *Cm, int64_t C_bs, const float *A_log, const float *D,
@@ -42,12 +42,12 @@ __global__ void __launch_bounds__(128) ssm_step_kernel(const T *u, int64_t u_bs,
     if (flags & GFE_FLAG_DELTA_SOFTPLUS) dl = softplus_only(dl);
     const float uj = to_f(u[(int64_t)b * u_bs + c]);
     const float du = dl * uj;
-    float4 *hrow = reinterpret_cast<float4 *>(h + ((size_t)b * ED + c) * kNState);
-    const float4 *arow = reinterpret_cast<const float4 *>(A_log + (size_t)c * kNState);
+    float4 *hrow = reinterpret_cast<float4 *>(h + ((size_t)b * ED + c) * N);
+    const float4 *arow = reinterpret_cast<const float4 *>(A_log + (size_t)c * N);
     const T *Bb = Bm + (int64_t)b * B_bs, *Cb = Cm + (int64_t)b * C_bs;
     float y = 0.f;
 #pragma unroll
-    for (int q = 0; q < kNState / 4; ++q) {
+    for (int q = 0; q < N / 4; ++q) {
         float4 hv = hrow[q];
         const float4 al = __ldg(arow + q);
         const float a0 = -expf(al.x) * kLog2e, a1 = -expf(al.y) * kLog2e, a2 = -expf(al.z) * kLog2e, a3 = -expf(al.w) * kLog2e;
@@ -85,18 +85,31 @@ static int conv_step_launch(const void *xin, int64_t x_bs, void *inputs, const f
     return check_launch("conv1d_step");
 }
 
-template <typename T>
+template <typename T, int N>
 static int ssm_step_launch(const void *u, int64_t u_bs, const void *delta, int64_t d_bs, const void *z, int64_t z_bs,
                            const void *Bm, int64_t B_bs, const void *Cm, int64_t C_bs, const float *A_log,
                            const float *D, const float *dt_bias, float *h, void *out, int64_t o_bs, int B, int ED,
                            uint32_t flags, cudaStream_t st) {
     const dim3 block(128), grid((ED + 127) / 128, B);
     ScopedKernelTimer tm(K_SSM_STEP, st);
-    ssm_step_kernel<T><<<grid, block, 0, st>>>(reinterpret_cast<const T *>(u), u_bs, reinterpret_cast<const T *>(delta), d_bs,
-                                               reinterpret_cast<const T *>(z), z_bs, reinterpret_cast<const T *>(Bm), B_bs,
-                                               reinterpret_cast<const T *>(Cm), C_bs, A_log, D, dt_bias, h,
-                                               reinterpret_cast<T *>(out), o_bs, B, ED, flags);
+    ssm_step_kernel<T, N><<<grid, block, 0, st>>>(reinterpret_cast<const T *>(u), u_bs, reinterpret_cast<const T *>(delta), d_bs,
+                                                  reinterpret_cast<const T *>(z), z_bs, reinterpret_cast<const T *>(Bm), B_bs,
+                                                  reinterpret_cast<const T *>(Cm), C_bs, A_log, D, dt_bias, h,
+                                                  reinterpret_cast<T *>(out), o_bs, B, ED, flags);
     return check_launch("ssm_step");
+}
+
+// by state size (gfe_ssm_step has checked fused_d_state)
+template <typename T>
+static int ssm_step_launch_n(int N, const void *u, int64_t u_bs, const void *delta, int64_t d_bs, const void *z, int64_t z_bs,
+                             const void *Bm, int64_t B_bs, const void *Cm, int64_t C_bs, const float *A_log,
+                             const float *D, const float *dt_bias, float *h, void *out, int64_t o_bs, int B, int ED,
+                             uint32_t flags, cudaStream_t st) {
+    switch (N) {
+        case 16: return ssm_step_launch<T, 16>(u, u_bs, delta, d_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, o_bs, B, ED, flags, st);
+        case 32: return ssm_step_launch<T, 32>(u, u_bs, delta, d_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, o_bs, B, ED, flags, st);
+        default: return ssm_step_launch<T, 64>(u, u_bs, delta, d_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, o_bs, B, ED, flags, st);
+    }
 }
 
 }  // namespace gfe
@@ -124,12 +137,12 @@ GFE_API int gfe_ssm_step(const void *u, int64_t u_bs, const void *delta, int64_t
     using namespace gfe;
     if (!u || !delta || !Bm || !Cm || !A_log || !D || !h || !out) { set_error("ssm_step: NULL pointer"); return GFE_ERR_ARG; }
     if (B <= 0 || ED <= 0 || B > 65535) { set_error("ssm_step: bad shape"); return GFE_ERR_ARG; }
-    if (N != kNState) { set_error("ssm_step: d_state=%d unsupported (compiled for %d)", N, kNState); return GFE_ERR_UNSUPPORTED; }
+    if (!fused_d_state(N)) { set_error("ssm_step: d_state=%d unsupported (compiled for 16, 32 and 64)", N); return GFE_ERR_UNSUPPORTED; }
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     switch (dtype) {
-        case GFE_F32: return ssm_step_launch<float>(u, u_bs, delta, delta_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, out_bs, B, ED, flags, st);
-        case GFE_BF16: return ssm_step_launch<__nv_bfloat16>(u, u_bs, delta, delta_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, out_bs, B, ED, flags, st);
-        case GFE_F16: return ssm_step_launch<__half>(u, u_bs, delta, delta_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, out_bs, B, ED, flags, st);
+        case GFE_F32: return ssm_step_launch_n<float>(N, u, u_bs, delta, delta_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, out_bs, B, ED, flags, st);
+        case GFE_BF16: return ssm_step_launch_n<__nv_bfloat16>(N, u, u_bs, delta, delta_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, out_bs, B, ED, flags, st);
+        case GFE_F16: return ssm_step_launch_n<__half>(N, u, u_bs, delta, delta_bs, z, z_bs, Bm, B_bs, Cm, C_bs, A_log, D, dt_bias, h, out, out_bs, B, ED, flags, st);
         default: set_error("ssm_step: bad dtype %d", dtype); return GFE_ERR_DTYPE;
     }
 }

@@ -197,7 +197,7 @@ class MambaBlock(nn.Module):
         """The one-node inner path serves the shapes the fused kernels are compiled for and the plain configuration (no
         inner layernorms); everything else takes the op-by-op composition below."""
         cfg = self.config
-        return (xz.is_cuda and xz.dim() == 3 and cfg.d_state == 16 and 2 <= cfg.d_conv <= 4 and not cfg.inner_layernorms
+        return (xz.is_cuda and xz.dim() == 3 and cfg.d_state in ops.FUSED_D_STATES and 2 <= cfg.d_conv <= 4 and not cfg.inner_layernorms
                 and xz.dtype in (torch.float32, torch.bfloat16, torch.float16) and self.x_proj.bias is None)
 
     def _project(self, x):
@@ -211,7 +211,7 @@ class MambaBlock(nn.Module):
 
     def _ssm_fused(self, x, z):
         delta, B, C = self._project(x)
-        if self.config.d_state == 16:
+        if self.config.d_state in ops.FUSED_D_STATES:
             return ops.selective_scan_fn(x, delta, self.A_log, B, C, self.D, z=z, dt_bias=self.dt_proj.bias,
                                          delta_softplus=True)
         # other state sizes: the reference's own composition on top of the CUDA pscan kernel
@@ -227,7 +227,7 @@ class MambaBlock(nn.Module):
     def selective_scan(self, x, delta, A, B, C, D):
         """mamba.py:265-286: x, delta (B, L, ED) with delta already softplus'ed; A (ED, N) negative; B, C (B, L, N);
         D (ED) -> y (B, L, ED) without gate."""
-        if A.shape[1] == 16:
+        if A.shape[1] in ops.FUSED_D_STATES:
             return ops.selective_scan_fn(x, delta, torch.log(-A), B, C, D, z=None, dt_bias=None, delta_softplus=False)
         deltaA = torch.exp(delta.unsqueeze(-1) * A)           # (B, L, ED, N)
         BX = (delta.unsqueeze(-1) * B.unsqueeze(2)) * x.unsqueeze(-1)
@@ -269,7 +269,7 @@ class MambaBlock(nn.Module):
         delta, B, C = torch.split(deltaBC, [self.config.dt_rank, self.config.d_state, self.config.d_state], dim=-1)
         delta, B, C = self._apply_layernorms(delta, B, C)
         delta = F.linear(delta, self.dt_proj.weight)
-        if self.config.d_state == 16 and self._step_kernels_usable(x, h, z):
+        if self.config.d_state in ops.FUSED_D_STATES and self._step_kernels_usable(x, h, z):
             return ops.ssm_step(x, delta, self.A_log, B, C, self.D, h, z=z, dt_bias=self.dt_proj.bias, delta_softplus=True)
         # other state sizes, or a caller that differentiates through the step: the reference's composition (:391-403)
         A = -torch.exp(self.A_log.float())

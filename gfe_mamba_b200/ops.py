@@ -14,6 +14,10 @@ from . import _native as nat
 
 _DT = {torch.float32: nat.GFE_F32, torch.bfloat16: nat.GFE_BF16, torch.float16: nat.GFE_F16}
 
+# d_state values the fused scan, the one-node inner path and the decode kernel are compiled for (fused_d_state in
+# csrc/common.cuh); MambaBlock takes the reference's composition on top of the pscan kernel for every other value
+FUSED_D_STATES = (16, 32, 64)
+
 
 def _require_cuda(*ts: Optional[torch.Tensor]) -> torch.device:
     dev = None
@@ -415,7 +419,8 @@ class _MambaInnerFn(torch.autograd.Function):
 
 def mamba_inner_fn(xz: torch.Tensor, conv_w: torch.Tensor, conv_b: Optional[torch.Tensor], x_proj_w: torch.Tensor,
                    dt_proj_w: torch.Tensor, dt_bias: Optional[torch.Tensor], A_log: torch.Tensor, D: torch.Tensor) -> torch.Tensor:
-    """y (B, L, ED) = gate(scan(conv(xz[..., :ED]), ...), xz[..., ED:]) for d_state = 16, d_conv in 2..4; see _MambaInnerFn."""
+    """y (B, L, ED) = gate(scan(conv(xz[..., :ED]), ...), xz[..., ED:]) for d_state in FUSED_D_STATES, d_conv in 2..4; see
+    _MambaInnerFn."""
     return _MambaInnerFn.apply(xz, conv_w, conv_b, x_proj_w, dt_proj_w, dt_bias, A_log, D, torch.is_grad_enabled())
 
 

@@ -23,7 +23,10 @@
  *     are fp32; `dtype` names the activation type;
  *   - return value: GFE_OK (0) or a negative gfe_status; gfe_last_error_string()
  *     returns a thread-local description of the last failure;
- *   - stateless and re-entrant: safe from any host thread (e.g. autograd's).
+ *   - stateless and re-entrant: safe from any host thread (e.g. autograd's);
+ *   - the selective scan (gfe_selscan_*) and the decode step (gfe_ssm_step) are compiled
+ *     for d_state N in {16, 32, 64}; the size queries return 0 and the entry points
+ *     GFE_ERR_UNSUPPORTED for any other N.
  */
 #ifndef GFE_MAMBA_B200_H
 #define GFE_MAMBA_B200_H
@@ -49,7 +52,7 @@ enum gfe_status {
     GFE_OK = 0,
     GFE_ERR_ARG = -1,         /* null pointer / non-positive size / bad flag            */
     GFE_ERR_DTYPE = -2,       /* dtype not one of gfe_dtype                              */
-    GFE_ERR_UNSUPPORTED = -3, /* shape outside the compiled envelope (e.g. d_state != 16) */
+    GFE_ERR_UNSUPPORTED = -3, /* shape outside the compiled envelope (e.g. d_state outside {16, 32, 64}) */
     GFE_ERR_WORKSPACE = -4,   /* workspace / checkpoint buffer missing or too small      */
     GFE_ERR_CUDA = -5         /* launch failed (cudaPeekAtLastError)                      */
 };
