@@ -6,8 +6,8 @@ or, as a drop-in for the reference's module names, put this repository ahead of 
 ``sys.path`` and keep ``from cross_atten.mamba import Mamba, MambaConfig`` unchanged.
 """
 from .mamba import Mamba, MambaBlock, MambaConfig, ResidualBlock, RMSNorm  # noqa: F401
-from .ops import (add_mean_pool, add_rmsnorm, causal_conv1d_silu, conv1d_step, mamba_inner_fn, selective_scan_fn,  # noqa: F401
-                  ssm_step)
+from .ops import (add_mean_pool, add_rmsnorm, causal_conv1d_silu, conv1d_prefill, conv1d_step, mamba_inner_fn,  # noqa: F401
+                  selective_scan_fn, ssm_prefill, ssm_step)
 from .optim import ClipAdam  # noqa: F401
 from .pscan import PScan, npo2, pad_npo2, pscan  # noqa: F401
 

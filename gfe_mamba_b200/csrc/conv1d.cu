@@ -24,6 +24,10 @@ struct ConvParams {
     float *dw, *dbias, *part;   // part: [B*ntiles][K+1][ED]
     int64_t x_bs, x_rs, u_bs, u_rs, du_bs, du_rs, dx_bs, dx_rs;
     int B, L, ED, ntiles;
+    // forward continuing a decode cache (gfe_conv1d_silu_fwd_state): rows t < 0 are read from cin (B, ED, K-1) instead of
+    // being zeros, and the last tile writes the last K-1 rows of cat(cin, xin) to cout (B, ED, K-1); either may be NULL
+    const void *cin;
+    void *cout;
 };
 
 // V adjacent channels per lane, moved as ONE load / store of V * sizeof(T) bytes (8 bytes when the layout allows it: 4
@@ -57,13 +61,14 @@ __global__ void __launch_bounds__(128) conv1d_silu_fwd_kernel(ConvParams p) {
         bias[i] = p.bias ? __ldg(p.bias + c + i) : 0.f;
     }
     float win[V][K];   // win[.][k] = xin[t - (K-1) + k]
+    const T *cin = reinterpret_cast<const T *>(p.cin) + ((size_t)b * p.ED + c) * (K - 1);   // row t < 0: cin[t + K - 1]
 #pragma unroll
     for (int k = 0; k < K - 1; ++k) {
         const int t = t0 - (K - 1) + k;
         ChanVec<T, V> xv{};
         if (t >= 0) xv = ChanVec<T, V>::load(x + (int64_t)t * p.x_rs);
 #pragma unroll
-        for (int i = 0; i < V; ++i) win[i][k + 1] = t >= 0 ? xv.get(i) : 0.f;
+        for (int i = 0; i < V; ++i) win[i][k + 1] = t >= 0 ? xv.get(i) : (p.cin != nullptr ? to_f(cin[i * (K - 1) + k]) : 0.f);
     }
     constexpr int U = 8;
     // rows of the next group, in flight while the current group is computed (measured on both directions: fp32 backward 14 %
@@ -95,6 +100,14 @@ __global__ void __launch_bounds__(128) conv1d_silu_fwd_kernel(ConvParams p) {
                 }
                 o.store(u + (int64_t)(tb + j) * p.u_rs);
             }
+        }
+    }
+    if (p.cout != nullptr && blockIdx.y == gridDim.y - 1) {   // last tile: the window holds the last K-1 rows of cat(cin, xin)
+        T *cout = reinterpret_cast<T *>(p.cout) + ((size_t)blockIdx.z * p.ED + (blockIdx.x * blockDim.x + threadIdx.x) * V) * (K - 1);
+#pragma unroll
+        for (int i = 0; i < V; ++i) {
+#pragma unroll
+            for (int k = 0; k < K - 1; ++k) cout[i * (K - 1) + k] = from_f<T>(win[i][k + 1]);
         }
     }
 }
@@ -267,13 +280,19 @@ __global__ void __launch_bounds__(128) conv1d_silu_fwd_pk_kernel(ConvParams p) {
         for (int k = 0; k < K; ++k) w[i][k] = make_float2(__ldg(p.w + (size_t)(c + 2 * i) * K + k), __ldg(p.w + (size_t)(c + 2 * i + 1) * K + k));
         bias[i] = p.bias ? make_float2(__ldg(p.bias + c + 2 * i), __ldg(p.bias + c + 2 * i + 1)) : make_float2(0.f, 0.f);
     }
+    const T *cin = reinterpret_cast<const T *>(p.cin) + ((size_t)b * p.ED + c) * (K - 1);   // row t < 0: cin[t + K - 1]
 #pragma unroll
     for (int k = 0; k < K - 1; ++k) {
         const int t = t0 - (K - 1) + k;
         float2 v[NP];
 #pragma unroll
         for (int i = 0; i < NP; ++i) v[i] = make_float2(0.f, 0.f);
-        if (t >= 0) PV::unpack(__ldcs(reinterpret_cast<const Raw *>(xp + (int64_t)(k - (K - 1)) * xs)), v);
+        if (t >= 0) {
+            PV::unpack(__ldcs(reinterpret_cast<const Raw *>(xp + (int64_t)(k - (K - 1)) * xs)), v);
+        } else if (p.cin != nullptr) {
+#pragma unroll
+            for (int i = 0; i < NP; ++i) v[i] = make_float2(to_f(cin[2 * i * (K - 1) + k]), to_f(cin[(2 * i + 1) * (K - 1) + k]));
+        }
 #pragma unroll
         for (int i = 0; i < NP; ++i) win[i][k + 1] = v[i];
     }
@@ -308,6 +327,17 @@ __global__ void __launch_bounds__(128) conv1d_silu_fwd_pk_kernel(ConvParams p) {
     int tb = t0;
     for (; tb + U <= t1; tb += U) group(std::true_type{}, U);
     if (tb < t1) group(std::false_type{}, t1 - tb);
+    if (p.cout != nullptr && blockIdx.y == gridDim.y - 1) {   // last tile: the window holds the last K-1 rows of cat(cin, xin)
+        T *cout = reinterpret_cast<T *>(p.cout) + ((size_t)blockIdx.z * p.ED + (blockIdx.x * blockDim.x + threadIdx.x) * V) * (K - 1);
+#pragma unroll
+        for (int i = 0; i < NP; ++i) {
+#pragma unroll
+            for (int k = 0; k < K - 1; ++k) {
+                cout[2 * i * (K - 1) + k] = from_f<T>(win[i][k + 1].x);
+                cout[(2 * i + 1) * (K - 1) + k] = from_f<T>(win[i][k + 1].y);
+            }
+        }
+    }
 }
 
 template <typename T, int K, int NP>
@@ -500,11 +530,22 @@ extern "C" {
 GFE_API int gfe_conv1d_silu_fwd(const void *xin, int64_t x_bs, int64_t x_rs, const float *w, const float *bias,
                                 void *u, int64_t u_bs, int64_t u_rs, int B, int L, int ED, int K, int dtype,
                                 void *stream) {
+    return gfe_conv1d_silu_fwd_state(xin, x_bs, x_rs, w, bias, nullptr, nullptr, u, u_bs, u_rs, B, L, ED, K, dtype, stream);
+}
+
+GFE_API int gfe_conv1d_silu_fwd_state(const void *xin, int64_t x_bs, int64_t x_rs, const float *w, const float *bias,
+                                      const void *inputs, void *new_inputs, void *u, int64_t u_bs, int64_t u_rs,
+                                      int B, int L, int ED, int K, int dtype, void *stream) {
     using namespace gfe;
     if (!xin || !w || !u) { set_error("conv1d_fwd: NULL pointer"); return GFE_ERR_ARG; }
     if (B <= 0 || L <= 0 || ED <= 0 || B > 65535) { set_error("conv1d_fwd: bad shape"); return GFE_ERR_ARG; }
+    if (inputs != nullptr && new_inputs != nullptr && K >= 2) {
+        const size_t bytes = (size_t)B * ED * (K - 1) * (dtype == GFE_F32 ? 4 : 2);
+        const char *a = reinterpret_cast<const char *>(inputs), *c = reinterpret_cast<const char *>(new_inputs);
+        if (a < c + bytes && c < a + bytes) { set_error("conv1d_fwd: inputs and new_inputs overlap"); return GFE_ERR_ARG; }
+    }
     ConvParams p{};
-    p.xin = xin; p.u = u; p.w = w; p.bias = bias;
+    p.xin = xin; p.u = u; p.w = w; p.bias = bias; p.cin = inputs; p.cout = new_inputs;
     p.x_bs = x_bs; p.x_rs = x_rs; p.u_bs = u_bs; p.u_rs = u_rs;
     p.B = B; p.L = L; p.ED = ED; p.ntiles = (L + kConvTile - 1) / kConvTile;
     return conv_dispatch(false, K, dtype, p, reinterpret_cast<cudaStream_t>(stream));

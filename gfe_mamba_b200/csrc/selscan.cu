@@ -235,10 +235,17 @@ __global__ void __launch_bounds__(128) selscan_fwd_kernel(ScanParams p) {
     Decay<N> A2;
     float2 h[P];
     A2.load(p.A_log, c, sA2, lane);
+    if (p.h0 != nullptr) {   // the caller's state before token 0 (same layout as last_state)
+        const float2 *src = reinterpret_cast<const float2 *>(p.h0 + ((size_t)b * p.ED + c) * N);
 #pragma unroll
-    for (int q = 0; q < P; ++q) h[q] = make_float2(0.f, 0.f);
+        for (int q = 0; q < P; ++q) h[q] = src[q];
+    } else {
+#pragma unroll
+        for (int q = 0; q < P; ++q) h[q] = make_float2(0.f, 0.f);
+    }
 
-    // carry-in: combine the summaries of all earlier segments (exp of a delta prefix sum per state)
+    // carry-in: combine the summaries of all earlier segments (exp of a delta prefix sum per state); the summaries are
+    // zero-start locals, so a state h0 is carried through them like any other
 #pragma unroll 4
     for (int s = 0; s < seg; ++s) {
         const float sd = p.seg_sd[(size_t)(b * p.nseg + s) * p.ED + c];
@@ -870,7 +877,7 @@ static void launch_fast(K kernel, dim3 grid, dim3 block, size_t smem, cudaStream
 }
 
 template <typename T, int N>
-static int launch_fwd(const gfe_selscan_args *a, cudaStream_t st) {
+static int launch_fwd(const gfe_selscan_args *a, const float *h0, cudaStream_t st) {
     const SegPlan sp = plan_segments(a->batch, a->seqlen, a->d_inner);
     const WsLayout wl = fwd_ws_layout(a->batch, a->seqlen, a->d_inner, N, sp);
     if (wl.total > 0 && (a->ws == nullptr || a->ws_bytes < wl.total)) {
@@ -879,7 +886,7 @@ static int launch_fwd(const gfe_selscan_args *a, cudaStream_t st) {
     }
     ScanParams p{};
     fill_common(p, a, sp);
-    p.out = a->out; p.o_bs = a->out_bs; p.o_rs = a->out_rs; p.last_state = a->last_state;
+    p.out = a->out; p.o_bs = a->out_bs; p.o_rs = a->out_rs; p.last_state = a->last_state; p.h0 = h0;
     char *ws = reinterpret_cast<char *>(a->ws);
     p.seg_h = reinterpret_cast<float2 *>(ws + wl.seg_h);
     p.seg_sd = reinterpret_cast<float *>(ws + wl.seg_sd);
@@ -975,11 +982,11 @@ static int launch_bwd(const gfe_selscan_args *a, cudaStream_t st) {
 
 // generic kernels by state size (validate_common has checked fused_d_state)
 template <typename T>
-static int launch_fwd_n(const gfe_selscan_args *a, cudaStream_t st) {
+static int launch_fwd_n(const gfe_selscan_args *a, const float *h0, cudaStream_t st) {
     switch (a->d_state) {
-        case 16: return launch_fwd<T, 16>(a, st);
-        case 32: return launch_fwd<T, 32>(a, st);
-        default: return launch_fwd<T, 64>(a, st);
+        case 16: return launch_fwd<T, 16>(a, h0, st);
+        case 32: return launch_fwd<T, 32>(a, h0, st);
+        default: return launch_fwd<T, 64>(a, h0, st);
     }
 }
 
@@ -989,6 +996,16 @@ static int launch_bwd_n(const gfe_selscan_args *a, cudaStream_t st) {
         case 16: return launch_bwd<T, 16>(a, st);
         case 32: return launch_bwd<T, 32>(a, st);
         default: return launch_bwd<T, 64>(a, st);
+    }
+}
+
+// forward dispatch of gfe_selscan_fwd / gfe_selscan_fwd_state (arguments validated); h0 NULL = zero start
+static int launch_fwd_any(const gfe_selscan_args *a, const float *h0, cudaStream_t st) {
+    if (chain_applicable(a->batch, a->seqlen, a->d_inner, a->d_state)) return chain_launch_fwd(a, h0, st);
+    switch (a->dtype) {
+        case GFE_F32: return launch_fwd_n<float>(a, h0, st);
+        case GFE_BF16: return launch_fwd_n<__nv_bfloat16>(a, h0, st);
+        default: return launch_fwd_n<__half>(a, h0, st);
     }
 }
 
@@ -1024,13 +1041,25 @@ GFE_API size_t gfe_selscan_bwd_workspace_bytes(int B, int L, int ED, int N) {
 GFE_API int gfe_selscan_fwd(const gfe_selscan_args *a, void *stream) {
     int rc = gfe::validate_common(a, false);
     if (rc != GFE_OK) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    if (gfe::chain_applicable(a->batch, a->seqlen, a->d_inner, a->d_state)) return gfe::chain_launch_fwd(a, st);
-    switch (a->dtype) {
-        case GFE_F32: return gfe::launch_fwd_n<float>(a, st);
-        case GFE_BF16: return gfe::launch_fwd_n<__nv_bfloat16>(a, st);
-        default: return gfe::launch_fwd_n<__half>(a, st);
+    return gfe::launch_fwd_any(a, nullptr, reinterpret_cast<cudaStream_t>(stream));
+}
+
+GFE_API int gfe_selscan_fwd_state(const gfe_selscan_args *a, const float *h0, void *stream) {
+    if (a != nullptr && a->ckpt != nullptr) {
+        gfe::set_error("selscan_fwd_state: ckpt must be NULL (a forward from a carried state has no backward)");
+        return GFE_ERR_ARG;
     }
+    int rc = gfe::validate_common(a, false);
+    if (rc != GFE_OK) return rc;
+    if (h0 != nullptr) {
+        if ((reinterpret_cast<uintptr_t>(h0) & 15) != 0) { gfe::set_error("selscan_fwd_state: h0 must be 16-byte aligned"); return GFE_ERR_ARG; }
+        const size_t n = (size_t)a->batch * a->d_inner * a->d_state;
+        if (a->last_state != nullptr && a->last_state < h0 + n && h0 < a->last_state + n) {
+            gfe::set_error("selscan_fwd_state: h0 and last_state overlap");
+            return GFE_ERR_ARG;
+        }
+    }
+    return gfe::launch_fwd_any(a, h0, reinterpret_cast<cudaStream_t>(stream));
 }
 
 GFE_API int gfe_selscan_bwd(const gfe_selscan_args *a, void *stream) {

@@ -165,7 +165,7 @@ bool chain_pair_stores(const gfe_selscan_args *a, bool bwd) {
 }
 
 template <typename T>
-static int launch_fwd_chain_t(const gfe_selscan_args *a, cudaStream_t st) {
+static int launch_fwd_chain_t(const gfe_selscan_args *a, const float *h0, cudaStream_t st) {
     const ChainPlan pl = chain_fwd_plan(a->batch, a->seqlen, a->d_inner);
     const size_t need = chain_bytes(a->batch, a->d_inner, pl);
     if (a->ws == nullptr || a->ws_bytes < need) {
@@ -176,7 +176,7 @@ static int launch_fwd_chain_t(const gfe_selscan_args *a, cudaStream_t st) {
     if (rc != GFE_OK) return rc;
     ScanParams p{};
     chain_fill_params(p, a);
-    p.out = a->out; p.o_bs = a->out_bs; p.o_rs = a->out_rs; p.last_state = a->last_state;
+    p.out = a->out; p.o_bs = a->out_bs; p.o_rs = a->out_rs; p.last_state = a->last_state; p.h0 = h0;
     ChainSched cs{};
     rc = chain_fill_sched(cs, reinterpret_cast<char *>(a->ws), a->batch, a->d_inner, pl, st);
     if (rc != GFE_OK) return rc;
@@ -193,11 +193,11 @@ static int launch_fwd_chain_t(const gfe_selscan_args *a, cudaStream_t st) {
     return check_launch("selscan_fwd (chained)");
 }
 
-int chain_launch_fwd(const gfe_selscan_args *a, cudaStream_t st) {
+int chain_launch_fwd(const gfe_selscan_args *a, const float *h0, cudaStream_t st) {
     switch (a->dtype) {
-        case GFE_F32: return launch_fwd_chain_t<float>(a, st);
-        case GFE_BF16: return launch_fwd_chain_t<__nv_bfloat16>(a, st);
-        default: return launch_fwd_chain_t<__half>(a, st);
+        case GFE_F32: return launch_fwd_chain_t<float>(a, h0, st);
+        case GFE_BF16: return launch_fwd_chain_t<__nv_bfloat16>(a, h0, st);
+        default: return launch_fwd_chain_t<__half>(a, h0, st);
     }
 }
 

@@ -10,7 +10,8 @@
 //      segment.  No C.h, no outputs, no checkpoints, no cross-lane reduction: 2 packed FP32 ops and 2 exp2 per state pair
 //      and step; one exp2 pair of four runs as a polynomial on the FMA pipe, because this loop is MUFU-bound.
 //   2. combine pass: carry[s + 1] = exp2(A sum_delta[s]) carry[s] + local[s] over the segments, as a two-level scan (32 runs of
-//      up to 8 segments per (b, c, n) element, chained through shared memory).
+//      up to 8 segments per (b, c, n) element, chained through shared memory); carry[0] is the caller's state h0 (forward from
+//      a carried state, gfe_selscan_fwd_state) or zero.
 //   3. main pass: the chained kernels with ChainSched::independent = 1 (selscan_v4_fwd.cu, selscan_chain_bwd.cu).
 #include "common.cuh"
 #include "selscan_shared.cuh"
@@ -212,13 +213,15 @@ __global__ void __launch_bounds__(2 * CPC, 4 * (64 / CPC)) selscan_seg_summary_k
 }
 
 // carry[slot] <- exp2(A sum_delta[slot]) carry[previous slot] + local[slot], in place; forward: slots ascending (the result is
-// the carry-in of segment slot + 1), reverse: slots descending (the reverse carry-in of segment slot).
+// the carry-in of segment slot + 1), reverse: slots descending (the reverse carry-in of segment slot).  The carry before the
+// first slot is h0[(b, c, n)] ((B, ED, 16), the element index) when h0 is not NULL (forward only), else zero.
 // A CTA of 32 x 32 threads serves 32 consecutive (b, c, n) elements: thread (x, y) owns element x and the y-th run of K <= 8
 // consecutive slots (in processing order).  It loads its run (all loads in flight at once), reduces it to one (P, S) pair,
 // row y = 0 chains the 32 pairs through shared memory, and every thread replays its run from the carry it was handed.
 constexpr int kCombK = (kMaxSeg + 31) / 32;
 __global__ void __launch_bounds__(1024) selscan_seg_combine_kernel(float *__restrict__ segc, const float *__restrict__ segsd,
-                                                                   const float *__restrict__ A_log, int nslots, int B, int ED, int rev) {
+                                                                   const float *__restrict__ A_log, const float *__restrict__ h0,
+                                                                   int nslots, int B, int ED, int rev) {
     __shared__ float sP[32][33], sS[32][33];
     const int x = threadIdx.x, y = threadIdx.y;
     const int64_t n_el = (int64_t)B * ED * kNState;
@@ -246,7 +249,7 @@ __global__ void __launch_bounds__(1024) selscan_seg_combine_kernel(float *__rest
     sP[y][x] = P; sS[y][x] = H;
     __syncthreads();
     if (y == 0) {
-        float h = 0.f;
+        float h = h0 != nullptr ? __ldg(h0 + ic) : 0.f;
         for (int r = 0; r < 32; ++r) {          // carry INTO run r
             const float pr = sP[r][x], sr = sS[r][x];
             sS[r][x] = h;
@@ -270,13 +273,14 @@ __global__ void __launch_bounds__(1024) selscan_seg_combine_kernel(float *__rest
 
 // The same for a few segments (<= 32, e.g. the production shape): one thread per element walks the slots, 8 loads in flight.
 __global__ void __launch_bounds__(256) selscan_seg_combine_seq_kernel(float *__restrict__ segc, const float *__restrict__ segsd,
-                                                                      const float *__restrict__ A_log, int nslots, int B, int ED, int rev) {
+                                                                      const float *__restrict__ A_log, const float *__restrict__ h0,
+                                                                      int nslots, int B, int ED, int rev) {
     const int64_t n_el = (int64_t)B * ED * kNState;
     const int64_t idx = (int64_t)blockIdx.x * 256 + threadIdx.x;
     if (idx >= n_el) return;
     const int64_t bc = idx >> 4;
     const float a2 = -expf(__ldg(A_log + (size_t)(bc % ED) * kNState + (idx & 15))) * kLog2e;
-    float H = 0.f;
+    float H = h0 != nullptr ? __ldg(h0 + idx) : 0.f;
     constexpr int U = 8;
     for (int s0 = 0; s0 < nslots; s0 += U) {
         float S[U], sd[U];
@@ -344,10 +348,11 @@ int seg_launch_carries(const ScanParams &p, const ChainSched &cs, int dtype, int
     int rc = check_launch(rev ? "selscan_bwd segment summary" : "selscan_fwd segment summary");
     if (rc != GFE_OK) return rc;
     const int64_t n_el = (int64_t)p.B * p.ED * kNState;
+    const float *h0 = rev ? nullptr : p.h0;
     if (cs.nseg - 1 <= 32)
-        selscan_seg_combine_seq_kernel<<<(unsigned)ceil_div64(n_el, 256), 256, 0, st>>>(cs.segc, cs.segsd, p.A_log, cs.nseg - 1, p.B, p.ED, rev ? 1 : 0);
+        selscan_seg_combine_seq_kernel<<<(unsigned)ceil_div64(n_el, 256), 256, 0, st>>>(cs.segc, cs.segsd, p.A_log, h0, cs.nseg - 1, p.B, p.ED, rev ? 1 : 0);
     else
-        selscan_seg_combine_kernel<<<(unsigned)ceil_div64(n_el, 32), dim3(32, 32), 0, st>>>(cs.segc, cs.segsd, p.A_log, cs.nseg - 1, p.B, p.ED, rev ? 1 : 0);
+        selscan_seg_combine_kernel<<<(unsigned)ceil_div64(n_el, 32), dim3(32, 32), 0, st>>>(cs.segc, cs.segsd, p.A_log, h0, cs.nseg - 1, p.B, p.ED, rev ? 1 : 0);
     return check_launch("selscan segment combine");
 }
 

@@ -30,6 +30,7 @@ struct ScanParams {
     float *part_par;  // [B][nseg][N + 2][ED]
     int G;            // ceil(ED / 32)
     int bc_interleaved;   // part_bc rows: 1 = {dB[n], dC[n]} pairs (chained backward), 0 = dB[N] | dC[N] (generic backward)
+    const float *h0;      // forward: (B, ED, N) state before token 0 (gfe_selscan_fwd_state), or NULL: zeros
 };
 
 constexpr int kPairs = kNState / 2;
@@ -224,7 +225,7 @@ bool chain_applicable(int B, int L, int ED, int N);       // shape-only: both di
 size_t chain_ckpt_state_bytes(int B, int L, int ED, int dtype);
 size_t chain_fwd_workspace_bytes(int B, int L, int ED);
 size_t chain_bwd_workspace_bytes(int B, int L, int ED);
-int chain_launch_fwd(const gfe_selscan_args *a, cudaStream_t st);
+int chain_launch_fwd(const gfe_selscan_args *a, const float *h0, cudaStream_t st);   // h0: state before token 0, or NULL
 int chain_launch_bwd(const gfe_selscan_args *a, cudaStream_t st);
 
 }  // namespace gfe

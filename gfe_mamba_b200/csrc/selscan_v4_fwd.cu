@@ -235,6 +235,13 @@ __global__ void __launch_bounds__(2 * CPC, kFwdMinBlocks * (64 / CPC)) selscan_f
                 h[ch][0] = make_float2(v.x, v.y);
                 h[ch][1] = make_float2(v.z, v.w);
             }
+        } else if (p.h0 != nullptr) {   // the caller's state before token 0, in the lane layout of the last_state store below
+#pragma unroll
+            for (int ch = 0; ch < 2; ++ch) {
+                const float4 v = __ldg(reinterpret_cast<const float4 *>(p.h0 + ((size_t)b * p.ED + c0 + 2 * rp + ch) * kNState) + rq);
+                h[ch][0] = make_float2(v.x, v.y);
+                h[ch][1] = make_float2(v.z, v.w);
+            }
         } else {
 #pragma unroll
             for (int ch = 0; ch < 2; ++ch) h[ch][0] = h[ch][1] = make_float2(0.f, 0.f);

@@ -19,7 +19,12 @@ class GraphedDecoder:
     """decoder = GraphedDecoder(model, batch);  y = decoder.step(x)  with x: (batch, d_model) on the model's device.
 
     ``caches`` start as the reference's initial cache (h = zeros, conv window = zeros, mamba.py:342-373 with h=None) or can
-    be seeded from a prefill with ``load_caches``."""
+    be seeded from a prefill with ``load_caches``: a P-token prompt costs one ``Mamba.prefill`` instead of P steps,
+
+        _, caches = model.prefill(prompt)      # prompt: (batch, P, d_model)
+        decoder.load_caches(caches)
+        y = decoder.step(next_token)           # continues exactly where the prompt ended
+    """
 
     def __init__(self, model: Mamba, batch: int, dtype: Optional[torch.dtype] = None, warmup: int = 3):
         p = next(model.parameters())

@@ -112,6 +112,39 @@ class Mamba(nn.Module):
             x, caches[idx] = self.layers[idx].step(x, caches[idx])
         return x, caches
 
+    def prefill(self, x, caches=None):
+        """Many tokens of decoding at once.  x: (B, L, D); caches: [(h (B, ED, N) fp32 or None, inputs (B, ED, d_conv-1))] per
+        layer in the convention of ``step``, or None for the reference's initial cache (h = None, a zero conv window in the
+        activation dtype).  Returns (y (B, L, D), caches).
+
+        Gives the same output rows and the same caches as ``x.shape[1]`` calls of ``step`` from ``caches``; when ``caches`` is
+        what a prefix left, ``y`` equals the last rows of ``forward`` over prefix + ``x``.  So a prompt can be prefilled in one
+        call (``_, caches = model.prefill(prompt)``, then ``step`` or ``GraphedDecoder.load_caches(caches)``), in chunks of
+        bounded memory, or continued after decoding.  Extension of the reference API (like ``forward_mean``); the layers take
+        the scan and conv kernels from the carried state where they are compiled and fall back to ``step`` token by token
+        otherwise (see ``MambaBlock.prefill``).  ``caches`` is not modified."""
+        if not x.is_cuda:
+            raise RuntimeError("gfe_mamba_b200.Mamba: CUDA tensors required (this library has no CPU fallback); "
+                               f"got input on {x.device}")
+        cfg = self.config
+        if caches is None:
+            dt = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else x.dtype
+            caches = [(None, torch.zeros(x.shape[0], cfg.d_inner, cfg.d_conv - 1, dtype=dt, device=x.device))
+                      for _ in self.layers]
+        caches = list(caches)
+        if len(self.layers) == 0:
+            return x, caches
+        if not _fusable_norm(x, cfg):
+            for i, layer in enumerate(self.layers):
+                x, caches[i] = layer.prefill(x, caches[i])
+            return x, caches
+        # the add + RMSNorm structure of forward
+        resid, branch = x, None
+        for i, layer in enumerate(self.layers):
+            resid, normed = add_rmsnorm(resid, branch, layer.norm.weight, layer.norm.eps)
+            branch, caches[i] = layer.mixer.prefill(normed, caches[i])
+        return branch + resid, caches
+
 
 class ResidualBlock(nn.Module):
     """mamba.py:91-117: output = mixer(norm(x)) + x."""
@@ -126,6 +159,11 @@ class ResidualBlock(nn.Module):
 
     def step(self, x, cache):
         y, cache = self.mixer.step(self.norm(x), cache)
+        return y + x, cache
+
+    def prefill(self, x, cache):
+        """x: (B, L, D); ``step`` over the L tokens (see Mamba.prefill)."""
+        y, cache = self.mixer.prefill(self.norm(x), cache)
         return y + x, cache
 
 
@@ -255,6 +293,33 @@ class MambaBlock(nn.Module):
         y, h = self.ssm_step(u, h, z=z)
         output = self.out_proj(y)
         return output, (h, inputs)
+
+    def prefill(self, x, cache):
+        """x: (B, L, D); cache: (h, inputs) as for ``step``.  Returns (y (B, L, D), cache): the outputs and the cache of L
+        calls of ``step`` from ``cache``.  Where the kernels are compiled (d_state in ops.FUSED_D_STATES, 2 <= d_conv <= 4) and
+        no gradient is asked for, the forward path runs once over the L tokens from the carried state: in_proj ->
+        conv1d_prefill -> x_proj / dt_proj (inner layernorms included) -> ssm_prefill (gate fused) -> out_proj.  Otherwise
+        ``step`` runs token by token: the reference's semantics, differentiable, any configuration."""
+        h, inputs = cache
+        cfg = self.config
+        if cfg.d_state in ops.FUSED_D_STATES and 2 <= cfg.d_conv <= 4 and self._step_kernels_usable(x, h, inputs):
+            y, cache = self._prefill_inner(x, h, inputs)
+            return self.out_proj(y), cache
+        ys = []
+        for t in range(x.shape[1]):
+            y, cache = self.step(x[:, t], cache)
+            ys.append(y)
+        return torch.stack(ys, 1), cache
+
+    def _prefill_inner(self, x, h, inputs):
+        """prefill between in_proj and out_proj: (y (B, L, ED), (h, inputs)).  A function of its own so that xz, u, delta and
+        x_proj's output are freed before out_proj runs: the peak stays that of forward (whose inner node frees them too)."""
+        xz = self.in_proj(x)                                  # (B, L, 2*ED)
+        xin, z = xz.chunk(2, dim=-1)                          # strided halves, consumed in place
+        u, inputs = ops.conv1d_prefill(xin, inputs, self.conv1d.weight, self.conv1d.bias)
+        delta, B, C = self._project(u)
+        y, h = ops.ssm_prefill(u, delta, self.A_log, B, C, self.D, h, z=z, dt_bias=self.dt_proj.bias, delta_softplus=True)
+        return y, (h, inputs)
 
     def _step_kernels_usable(self, *tensors):
         """The decode kernels are inference-only: a caller that backpropagates through ``step`` (the reference's step is

@@ -571,8 +571,8 @@ def add_mean_pool(a: torch.Tensor, r: Optional[torch.Tensor] = None) -> torch.Te
 
 # ------------------------------------------------------------------------------- decode step
 def _no_autograd(name: str, *ts):
-    """The decode kernels have no backward: refuse to silently detach a graph (MambaBlock.step falls back to the
-    reference's differentiable torch composition in that case)."""
+    """The decode and prefill kernels have no backward: refuse to silently detach a graph (MambaBlock.step / .prefill fall
+    back to the reference's differentiable torch composition in that case)."""
     if torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in ts):
         raise RuntimeError(f"gfe_mamba_b200.{name}: inputs require grad but the decode kernels are inference-only; "
                            "call under torch.no_grad() or use MambaBlock.step, which falls back to torch ops")
@@ -598,6 +598,76 @@ def conv1d_step(xin: torch.Tensor, inputs: torch.Tensor, weight: torch.Tensor, b
         nat.check(l.gfe_conv1d_step(_ptr(x_), x_.stride(0), _ptr(new_inputs), _ptr(w_), _ptr(b_), _ptr(u), u.stride(0),
                                     B, ED, K, _DT[dt], _stream(dev)), "conv1d_step")
     return u, new_inputs
+
+
+def conv1d_prefill(xin: torch.Tensor, inputs: Optional[torch.Tensor], weight: torch.Tensor, bias: Optional[torch.Tensor]
+                   ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """L tokens of the causal conv continuing a decode cache: the multi-token ``conv1d_step``.  xin: (B, L, ED) (any
+    batch / row strides, unit channel stride); inputs: (B, ED, K-1) or None (zeros).  Returns (u (B, L, ED),
+    new_inputs (B, ED, K-1)): u equals causal_conv1d_silu over cat(inputs, xin) without its first K-1 rows, new_inputs is
+    the cache L calls of ``conv1d_step`` would leave.  Inference only; ``inputs`` is not modified."""
+    dev = _require_cuda(xin, inputs, weight, bias)
+    _no_autograd("conv1d_prefill", xin, inputs, weight, bias)
+    if xin.dim() != 3:
+        raise ValueError(f"conv1d_prefill: x must be (B, L, ED); got {tuple(xin.shape)}")
+    B, L, ED = xin.shape
+    K = weight.shape[-1]
+    dt = xin.dtype
+    if dt not in _DT:
+        raise TypeError(f"conv1d_prefill: unsupported activation dtype {dt}")
+    if weight.numel() != ED * K or (inputs is not None and tuple(inputs.shape) != (B, ED, K - 1)):
+        raise ValueError("conv1d_prefill: weight must be (ED, 1, K) / (ED, K) and inputs (B, ED, K-1)")
+    x_ = _rows(xin.detach())
+    in_ = None if inputs is None else inputs.detach().to(dt).contiguous()
+    w_ = weight.detach().float().reshape(ED, K).contiguous()
+    b_ = _f32(bias)
+    u = torch.empty((B, L, ED), dtype=dt, device=dev)
+    new_inputs = torch.empty((B, ED, K - 1), dtype=dt, device=dev)
+    l = nat.lib()
+    with torch.cuda.device(dev):
+        nat.check(l.gfe_conv1d_silu_fwd_state(_ptr(x_), x_.stride(0), x_.stride(1), _ptr(w_), _ptr(b_), _ptr(in_), _ptr(new_inputs),
+                                              _ptr(u), u.stride(0), u.stride(1), B, L, ED, K, _DT[dt], _stream(dev)),
+                  "conv1d_silu_fwd_state")
+    return u, new_inputs
+
+
+def ssm_prefill(u, delta, A_log, Bm, Cm, D, h, z=None, dt_bias=None, delta_softplus: bool = True):
+    """L tokens of the selective scan from a carried state: the multi-token ``ssm_step``.  u, delta, z: (B, L, ED); Bm, Cm:
+    (B, L, N) (any batch / row strides, unit channel stride: the halves of in_proj's and the slices of x_proj's output are
+    read in place); h: (B, ED, N) or None (zeros).  Returns (out (B, L, ED), h_new (B, ED, N) fp32): the outputs and final
+    state of ``selective_scan_fn`` over the L tokens started from h instead of zero -- what L calls of ``ssm_step`` give.
+    Inference only (no checkpoints are written); ``h`` is not modified."""
+    dev = _require_cuda(u, delta, A_log, Bm, Cm, D, h, z, dt_bias)
+    _no_autograd("ssm_prefill", u, delta, A_log, Bm, Cm, D, h, z, dt_bias)
+    if u.dim() != 3:
+        raise ValueError(f"ssm_prefill: u must be (B, L, ED); got {tuple(u.shape)}")
+    B, L, ED = u.shape
+    N = A_log.shape[1]
+    dt = u.dtype
+    if dt not in _DT:
+        raise TypeError(f"ssm_prefill: unsupported activation dtype {dt}")
+    if tuple(delta.shape) != (B, L, ED) or tuple(Bm.shape) != (B, L, N) or tuple(Cm.shape) != (B, L, N) \
+            or tuple(A_log.shape) != (ED, N) or tuple(D.shape) != (ED,) or (h is not None and tuple(h.shape) != (B, ED, N)):
+        raise ValueError("ssm_prefill: inconsistent shapes")
+    u_, delta_, Bm_, Cm_ = (_as(t, dt) for t in (u, delta, Bm, Cm))
+    z_ = None if z is None else _as(z, dt)
+    A_log_, D_, bias_ = _f32(A_log), _f32(D), _f32(dt_bias)
+    h_ = None if h is None else _f32(h)
+    if h_ is not None and h_.data_ptr() % 16:   # the kernels read the state as 16-byte vectors
+        h_ = h_.clone()
+    out = torch.empty((B, L, ED), dtype=dt, device=dev)
+    h_new = torch.empty((B, ED, N), dtype=torch.float32, device=dev)
+    l = nat.lib()
+    a = nat.SelscanArgs()
+    _fill_common(a, u_, delta_, z_, Bm_, Cm_, A_log_, D_, bias_, delta_softplus)
+    a.out, a.out_bs, a.out_rs = out.data_ptr(), out.stride(0), out.stride(1)
+    a.last_state = h_new.data_ptr()
+    with torch.cuda.device(dev):
+        nws = _sizes(B, L, ED, N, dev, _DT[dt])[1]
+        ws = _bytes(nws, dev)
+        a.ws, a.ws_bytes = (0 if ws is None else ws.data_ptr()), nws
+        nat.check(l.gfe_selscan_fwd_state(ctypes.byref(a), _ptr(h_), _stream(dev)), "selscan_fwd_state")
+    return out, h_new
 
 
 def ssm_step(u, delta, A_log, Bm, Cm, D, h, z=None, dt_bias=None, delta_softplus: bool = True):

@@ -11,6 +11,8 @@
  *                                        i.e. the contract of the selective_scan_fn call at :251)
  *   gfe_conv1d_silu_fwd / _bwd           cross_atten/mamba.py:128-131,208-212 (causal depthwise conv + SiLU)
  *   gfe_conv1d_step / gfe_ssm_step       cross_atten/mamba.py:357-358,370 and :375-405 (decode step)
+ *   gfe_conv1d_silu_fwd_state /          the same forwards continuing a decode cache (prefill: many tokens
+ *   gfe_selscan_fwd_state                at once from a (h, conv window) cache, the multi-token decode step)
  *
  * Conventions
  *   - every pointer is a DEVICE pointer owned by the caller; the library never
@@ -120,14 +122,25 @@ GFE_API size_t gfe_selscan_fwd_workspace_bytes(int B, int L, int ED, int N);
 GFE_API size_t gfe_selscan_bwd_workspace_bytes(int B, int L, int ED, int N);
 GFE_API int gfe_selscan_fwd(const gfe_selscan_args *args, void *stream);
 GFE_API int gfe_selscan_bwd(const gfe_selscan_args *args, void *stream);
+/* Forward from a carried state (inference, prefill from a decode cache): gfe_selscan_fwd with h[-1] = h0 instead of 0.
+ * h0: (B, ED, N) fp32, contiguous, 16-byte aligned, or NULL (= zeros) -- the layout of last_state and of gfe_ssm_step's h.
+ * args->ckpt must be NULL (no backward from here).  args->last_state may be NULL; it must not overlap h0.
+ * Same workspace query (gfe_selscan_fwd_workspace_bytes). */
+GFE_API int gfe_selscan_fwd_state(const gfe_selscan_args *args, const float *h0, void *stream);
 
 /* ------------------------------------------------ causal depthwise conv1d --
  * u[b,t,c] = silu(bias[c] + sum_k w[c,k] xin[b, t-(K-1)+k, c]),  xin = 0 for t < 0.
- * w: (ED, K) fp32 (= conv1d.weight viewed (ED,1,K)), bias: (ED) fp32 or NULL.  K <= 8.
+ * w: (ED, K) fp32 (= conv1d.weight viewed (ED,1,K)), bias: (ED) fp32 or NULL.  K in 2..4 (GFE_ERR_UNSUPPORTED otherwise).
  */
 GFE_API int gfe_conv1d_silu_fwd(const void *xin, int64_t x_bs, int64_t x_rs, const float *w, const float *bias,
                                 void *u, int64_t u_bs, int64_t u_rs, int B, int L, int ED, int K, int dtype,
                                 void *stream);
+/* Causal conv + SiLU continuing a decode cache: xin[t < 0] is read from inputs (B, ED, K-1) in the activation dtype
+ * (NULL = zeros); new_inputs (B, ED, K-1), may be NULL, receives the last K-1 rows of cat(inputs, xin) along time -- the
+ * cache gfe_conv1d_step would hold after the same tokens.  inputs and new_inputs must not overlap.  K in 2..4. */
+GFE_API int gfe_conv1d_silu_fwd_state(const void *xin, int64_t x_bs, int64_t x_rs, const float *w, const float *bias,
+                                      const void *inputs, void *new_inputs, void *u, int64_t u_bs, int64_t u_rs,
+                                      int B, int L, int ED, int K, int dtype, void *stream);
 GFE_API size_t gfe_conv1d_bwd_workspace_bytes(int B, int L, int ED, int K);
 GFE_API int gfe_conv1d_silu_bwd(const void *xin, int64_t x_bs, int64_t x_rs, const float *w, const float *bias,
                                 const void *du, int64_t du_bs, int64_t du_rs,
