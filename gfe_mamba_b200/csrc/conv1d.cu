@@ -25,9 +25,12 @@ struct ConvParams {
     int64_t x_bs, x_rs, u_bs, u_rs, du_bs, du_rs, dx_bs, dx_rs;
     int B, L, ED, ntiles;
     // forward continuing a decode cache (gfe_conv1d_silu_fwd_state): rows t < 0 are read from cin (B, ED, K-1) instead of
-    // being zeros, and the last tile writes the last K-1 rows of cat(cin, xin) to cout (B, ED, K-1); either may be NULL
+    // being zeros, and the last tile writes the last K-1 rows of cat(cin, xin) to cout (B, ED, K-1); either may be NULL.
+    // The backward (gfe_conv1d_silu_bwd_carry) reads rows t < 0 from cin too, and tile 0 writes the gradient of those rows,
+    // the dxin sum evaluated at t = j - (K-1), to dcin (B, ED, K-1) unless it is NULL
     const void *cin;
     void *cout;
+    void *dcin;
 };
 
 // V adjacent channels per lane, moved as ONE load / store of V * sizeof(T) bytes (8 bytes when the layout allows it: 4
@@ -129,6 +132,7 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_kernel(ConvParams p) {
         bias[i] = p.bias ? __ldg(p.bias + c + i) : 0.f;
     }
     float win[V][K], dvw[V][K], dw[V][K], db[V];   // dvw[.][k] = dv[t - (K-1) + k]
+    const T *cin = reinterpret_cast<const T *>(p.cin) + ((size_t)b * p.ED + c) * (K - 1);   // row t < 0: cin[t + K - 1]
 #pragma unroll
     for (int i = 0; i < V; ++i) {
         db[i] = 0.f;
@@ -141,7 +145,7 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_kernel(ConvParams p) {
         ChanVec<T, V> xv{};
         if (t >= 0) xv = ChanVec<T, V>::load(x + (int64_t)t * p.x_rs);
 #pragma unroll
-        for (int i = 0; i < V; ++i) win[i][k + 1] = t >= 0 ? xv.get(i) : 0.f;
+        for (int i = 0; i < V; ++i) win[i][k + 1] = t >= 0 ? xv.get(i) : (p.cin != nullptr ? to_f(cin[i * (K - 1) + k]) : 0.f);
     }
     // dv is needed K-1 steps past the tile to finish dxin of the tile's last steps
     const int tend = t1 + (K - 1);
@@ -195,7 +199,13 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_kernel(ConvParams p) {
                     for (int k = 0; k < K; ++k) acc = fmaf(w[i][k], dvw[i][K - 1 - k], acc);
                     o.set(i, acc);
                 }
-                if (s_out >= t0 && s_out < t1) o.store(dx + (int64_t)s_out * p.dx_rs);
+                if (s_out >= t0 && s_out < t1) {
+                    o.store(dx + (int64_t)s_out * p.dx_rs);
+                } else if (s_out < 0 && p.dcin != nullptr) {   // tile 0: a row of the caller's window
+                    T *dcin = reinterpret_cast<T *>(p.dcin) + ((size_t)b * p.ED + c) * (K - 1) + s_out + (K - 1);
+#pragma unroll
+                    for (int i = 0; i < V; ++i) dcin[i * (K - 1)] = from_f<T>(o.get(i));
+                }
             }
         }
     }
@@ -355,6 +365,7 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_pk_kernel(ConvParams p) {
     // dxin[s] is complete when dv[s + K - 1] is known: the row stored while step t is processed is t - (K - 1)
     char *dp = reinterpret_cast<char *>(reinterpret_cast<T *>(p.dxin) + (int64_t)b * p.dx_bs + c) + (int64_t)(t0 - (K - 1)) * ds;
     float2 w[NP][K], bias[NP], win[NP][K], dvw[NP][K], dw[NP][K], db[NP];   // dvw[.][k] = dv[t - (K-1) + k]
+    const T *cin = reinterpret_cast<const T *>(p.cin) + ((size_t)b * p.ED + c) * (K - 1);   // row t < 0: cin[t + K - 1]
 #pragma unroll
     for (int i = 0; i < NP; ++i) {
 #pragma unroll
@@ -371,7 +382,12 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_pk_kernel(ConvParams p) {
         float2 v[NP];
 #pragma unroll
         for (int i = 0; i < NP; ++i) v[i] = make_float2(0.f, 0.f);
-        if (t >= 0) PV::unpack(__ldcs(reinterpret_cast<const Raw *>(xp + (int64_t)(k - (K - 1)) * xs)), v);
+        if (t >= 0) {
+            PV::unpack(__ldcs(reinterpret_cast<const Raw *>(xp + (int64_t)(k - (K - 1)) * xs)), v);
+        } else if (p.cin != nullptr) {
+#pragma unroll
+            for (int i = 0; i < NP; ++i) v[i] = make_float2(to_f(cin[2 * i * (K - 1) + k]), to_f(cin[(2 * i + 1) * (K - 1) + k]));
+        }
 #pragma unroll
         for (int i = 0; i < NP; ++i) win[i][k + 1] = v[i];
     }
@@ -423,7 +439,16 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_pk_kernel(ConvParams p) {
                     o[i] = acc;
                 }
                 const int s_out = t - (K - 1);
-                if (s_out >= t0 && s_out < t1) __stcs(reinterpret_cast<Raw *>(dp + j * ds), PV::pack(o));
+                if (s_out >= t0 && s_out < t1) {
+                    __stcs(reinterpret_cast<Raw *>(dp + j * ds), PV::pack(o));
+                } else if (!MAIN && s_out < 0 && p.dcin != nullptr) {   // tile 0: a row of the caller's window
+                    T *dcin = reinterpret_cast<T *>(p.dcin) + ((size_t)b * p.ED + c) * (K - 1) + s_out + (K - 1);
+#pragma unroll
+                    for (int i = 0; i < NP; ++i) {
+                        dcin[2 * i * (K - 1)] = from_f<T>(o[i].x);
+                        dcin[(2 * i + 1) * (K - 1)] = from_f<T>(o[i].y);
+                    }
+                }
             }
         }
         xp += U * xs;
@@ -431,6 +456,10 @@ __global__ void __launch_bounds__(128) conv1d_silu_bwd_pk_kernel(ConvParams p) {
         dp += U * ds;
     };
     int tb = t0;
+    if (tile == 0 && p.dcin != nullptr) {   // the rows whose outputs include the window's gradient: the general group
+        group(std::false_type{}, tb);
+        tb += U;
+    }
     for (; tb + U <= t1; tb += U) group(std::true_type{}, tb);
     for (; tb < tend; tb += U) group(std::false_type{}, tb);
     float *part = p.part + ((size_t)(b * p.ntiles + tile) * (K + 1)) * p.ED + c;
@@ -561,13 +590,26 @@ GFE_API int gfe_conv1d_silu_bwd(const void *xin, int64_t x_bs, int64_t x_rs, con
                                 const void *du, int64_t du_bs, int64_t du_rs,
                                 void *dxin, int64_t dx_bs, int64_t dx_rs, float *dw, float *dbias,
                                 int B, int L, int ED, int K, int dtype, void *ws, size_t ws_bytes, void *stream) {
+    return gfe_conv1d_silu_bwd_carry(xin, x_bs, x_rs, w, bias, nullptr, du, du_bs, du_rs, dxin, dx_bs, dx_rs, dw, dbias, nullptr,
+                                     B, L, ED, K, dtype, ws, ws_bytes, stream);
+}
+
+GFE_API int gfe_conv1d_silu_bwd_carry(const void *xin, int64_t x_bs, int64_t x_rs, const float *w, const float *bias,
+                                      const void *inputs, const void *du, int64_t du_bs, int64_t du_rs,
+                                      void *dxin, int64_t dx_bs, int64_t dx_rs, float *dw, float *dbias, void *dinputs,
+                                      int B, int L, int ED, int K, int dtype, void *ws, size_t ws_bytes, void *stream) {
     using namespace gfe;
     if (!xin || !w || !du || !dxin || !dw) { set_error("conv1d_bwd: NULL pointer"); return GFE_ERR_ARG; }
     if (B <= 0 || L <= 0 || ED <= 0 || B > 65535) { set_error("conv1d_bwd: bad shape"); return GFE_ERR_ARG; }
     const size_t need = gfe_conv1d_bwd_workspace_bytes(B, L, ED, K);
     if (!ws || ws_bytes < need) { set_error("conv1d_bwd: workspace too small (%zu < %zu)", ws ? ws_bytes : (size_t)0, need); return GFE_ERR_WORKSPACE; }
+    if (inputs != nullptr && dinputs != nullptr && K >= 2) {
+        const size_t bytes = (size_t)B * ED * (K - 1) * (dtype == GFE_F32 ? 4 : 2);
+        const char *a = reinterpret_cast<const char *>(inputs), *c = reinterpret_cast<const char *>(dinputs);
+        if (a < c + bytes && c < a + bytes) { set_error("conv1d_bwd: inputs and dinputs overlap"); return GFE_ERR_ARG; }
+    }
     ConvParams p{};
-    p.xin = xin; p.du = du; p.dxin = dxin; p.w = w; p.bias = bias; p.dw = dw; p.dbias = dbias;
+    p.xin = xin; p.du = du; p.dxin = dxin; p.w = w; p.bias = bias; p.dw = dw; p.dbias = dbias; p.cin = inputs; p.dcin = dinputs;
     p.part = reinterpret_cast<float *>(ws);
     p.x_bs = x_bs; p.x_rs = x_rs; p.du_bs = du_bs; p.du_rs = du_rs; p.dx_bs = dx_bs; p.dx_rs = dx_rs;
     p.B = B; p.L = L; p.ED = ED; p.ntiles = (L + kConvTile - 1) / kConvTile;

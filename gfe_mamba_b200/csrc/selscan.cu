@@ -565,13 +565,16 @@ __global__ void __launch_bounds__(128) selscan_bwd_kernel(ScanParams p) {
             sA[(2 * q) * 32 + lane] = make_float2(-expf(v.x), -expf(v.y));
             sA[(2 * q + 1) * 32 + lane] = make_float2(-expf(v.z), -expf(v.w));
         }
+        // the carry after the last token: the gradient of the final state (gfe_selscan_bwd_carry) or zero
+        const float2 *dlast = p.dlast != nullptr ? reinterpret_cast<const float2 *>(p.dlast + ((size_t)b * p.ED + c) * N) : nullptr;
 #pragma unroll
         for (int q = 0; q < P; ++q) {
-            sG[q * 32 + lane] = make_float2(0.f, 0.f);
+            sG[q * 32 + lane] = dlast != nullptr ? dlast[q] : make_float2(0.f, 0.f);
             sdA[q * 32 + lane] = make_float2(0.f, 0.f);
         }
         // carry-in from the later segments: G = P[s] * G + Gloc[s], s = nseg-1 .. seg+1 (N = 64: one segment's 32 pairs of
-        // loads at a time, four would take the whole register file)
+        // loads at a time, four would take the whole register file); Gloc are zero-start locals, so dlast is carried through
+        // them like any other carry
 #pragma unroll(N > 32 ? 1 : 4)
         for (int s = p.nseg - 1; s > seg; --s) {
             const float sd = p.seg_sd[(size_t)(b * p.nseg + s) * p.ED + c];
@@ -754,6 +757,11 @@ __global__ void __launch_bounds__(128) selscan_bwd_kernel(ScanParams p) {
         }
         dst[(size_t)N * p.ED] = dD_acc;
         dst[(size_t)(N + 1) * p.ED] = dbias_acc;
+        if (seg == 0 && p.dh0 != nullptr) {   // a[0] g[0]: the gradient of the state before token 0
+            float2 *dh0 = reinterpret_cast<float2 *>(p.dh0 + ((size_t)b * p.ED + c) * N);
+#pragma unroll
+            for (int q = 0; q < P; ++q) dh0[q] = sG[q * 32 + lane];
+        }
     }
 }
 
@@ -955,7 +963,7 @@ void launch_bwd_finalize(const gfe_selscan_args *a, ScanParams &p, cudaStream_t 
 }
 
 template <typename T, int N>
-static int launch_bwd(const gfe_selscan_args *a, cudaStream_t st) {
+static int launch_bwd(const gfe_selscan_args *a, const float *dlast, float *dh0, cudaStream_t st) {
     const SegPlan sp = plan_segments(a->batch, a->seqlen, a->d_inner);
     const WsLayout wl = bwd_ws_layout(a->batch, a->seqlen, a->d_inner, N, sp);
     if (a->ws == nullptr || a->ws_bytes < wl.total) {
@@ -976,6 +984,7 @@ static int launch_bwd(const gfe_selscan_args *a, cudaStream_t st) {
     p.dBm = a->dBm; p.dB_bs = a->dB_bs; p.dB_rs = a->dB_rs;
     p.dCm = a->dCm; p.dC_bs = a->dC_bs; p.dC_rs = a->dC_rs;
     p.dA_log = a->dA_log; p.dD = a->dD; p.ddt_bias = a->ddt_bias;
+    p.dlast = dlast; p.dh0 = dh0;
     if (a->z != nullptr) return launch_bwd_z<T, true, N>(a, p, sp, st);
     return launch_bwd_z<T, false, N>(a, p, sp, st);
 }
@@ -991,11 +1000,11 @@ static int launch_fwd_n(const gfe_selscan_args *a, const float *h0, cudaStream_t
 }
 
 template <typename T>
-static int launch_bwd_n(const gfe_selscan_args *a, cudaStream_t st) {
+static int launch_bwd_n(const gfe_selscan_args *a, const float *dlast, float *dh0, cudaStream_t st) {
     switch (a->d_state) {
-        case 16: return launch_bwd<T, 16>(a, st);
-        case 32: return launch_bwd<T, 32>(a, st);
-        default: return launch_bwd<T, 64>(a, st);
+        case 16: return launch_bwd<T, 16>(a, dlast, dh0, st);
+        case 32: return launch_bwd<T, 32>(a, dlast, dh0, st);
+        default: return launch_bwd<T, 64>(a, dlast, dh0, st);
     }
 }
 
@@ -1007,6 +1016,30 @@ static int launch_fwd_any(const gfe_selscan_args *a, const float *h0, cudaStream
         case GFE_BF16: return launch_fwd_n<__nv_bfloat16>(a, h0, st);
         default: return launch_fwd_n<__half>(a, h0, st);
     }
+}
+
+// backward dispatch of gfe_selscan_bwd / gfe_selscan_bwd_carry (arguments validated); dlast NULL = zero end carry
+static int launch_bwd_any(const gfe_selscan_args *a, const float *dlast, float *dh0, cudaStream_t st) {
+    if (chain_applicable(a->batch, a->seqlen, a->d_inner, a->d_state)) return chain_launch_bwd(a, dlast, dh0, st);
+    switch (a->dtype) {
+        case GFE_F32: return launch_bwd_n<float>(a, dlast, dh0, st);
+        case GFE_BF16: return launch_bwd_n<__nv_bfloat16>(a, dlast, dh0, st);
+        default: return launch_bwd_n<__half>(a, dlast, dh0, st);
+    }
+}
+
+static bool overlaps(const void *x, size_t nx, const void *y, size_t ny) {   // byte ranges [x, x + nx) and [y, y + ny)
+    const char *a = reinterpret_cast<const char *>(x), *b = reinterpret_cast<const char *>(y);
+    return a != nullptr && b != nullptr && a < b + ny && b < a + nx;
+}
+
+// h0 of the forwards from a carried state: 16-byte aligned, apart from last_state
+static int validate_h0(const gfe_selscan_args *a, const float *h0, const char *who) {
+    if (h0 == nullptr) return GFE_OK;
+    if ((reinterpret_cast<uintptr_t>(h0) & 15) != 0) { set_error("%s: h0 must be 16-byte aligned", who); return GFE_ERR_ARG; }
+    const size_t n = (size_t)a->batch * a->d_inner * a->d_state * sizeof(float);
+    if (overlaps(a->last_state, n, h0, n)) { set_error("%s: h0 and last_state overlap", who); return GFE_ERR_ARG; }
+    return GFE_OK;
 }
 
 }  // namespace gfe
@@ -1051,27 +1084,47 @@ GFE_API int gfe_selscan_fwd_state(const gfe_selscan_args *a, const float *h0, vo
     }
     int rc = gfe::validate_common(a, false);
     if (rc != GFE_OK) return rc;
-    if (h0 != nullptr) {
-        if ((reinterpret_cast<uintptr_t>(h0) & 15) != 0) { gfe::set_error("selscan_fwd_state: h0 must be 16-byte aligned"); return GFE_ERR_ARG; }
-        const size_t n = (size_t)a->batch * a->d_inner * a->d_state;
-        if (a->last_state != nullptr && a->last_state < h0 + n && h0 < a->last_state + n) {
-            gfe::set_error("selscan_fwd_state: h0 and last_state overlap");
-            return GFE_ERR_ARG;
-        }
-    }
+    rc = gfe::validate_h0(a, h0, "selscan_fwd_state");
+    if (rc != GFE_OK) return rc;
+    return gfe::launch_fwd_any(a, h0, reinterpret_cast<cudaStream_t>(stream));
+}
+
+GFE_API int gfe_selscan_fwd_carry(const gfe_selscan_args *a, const float *h0, void *stream) {
+    int rc = gfe::validate_common(a, false);
+    if (rc != GFE_OK) return rc;
+    rc = gfe::validate_h0(a, h0, "selscan_fwd_carry");
+    if (rc != GFE_OK) return rc;
     return gfe::launch_fwd_any(a, h0, reinterpret_cast<cudaStream_t>(stream));
 }
 
 GFE_API int gfe_selscan_bwd(const gfe_selscan_args *a, void *stream) {
+    return gfe_selscan_bwd_carry(a, nullptr, nullptr, stream);
+}
+
+GFE_API int gfe_selscan_bwd_carry(const gfe_selscan_args *a, const float *dlast, float *dh0, void *stream) {
+    using gfe::overlaps;
     int rc = gfe::validate_common(a, true);
     if (rc != GFE_OK) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    if (gfe::chain_applicable(a->batch, a->seqlen, a->d_inner, a->d_state)) return gfe::chain_launch_bwd(a, st);
-    switch (a->dtype) {
-        case GFE_F32: return gfe::launch_bwd_n<float>(a, st);
-        case GFE_BF16: return gfe::launch_bwd_n<__nv_bfloat16>(a, st);
-        default: return gfe::launch_bwd_n<__half>(a, st);
+    if ((reinterpret_cast<uintptr_t>(dlast) & 15) != 0 || (reinterpret_cast<uintptr_t>(dh0) & 15) != 0) {
+        gfe::set_error("selscan_bwd_carry: dlast and dh0 must be 16-byte aligned");
+        return GFE_ERR_ARG;
     }
+    if (dh0 != nullptr) {
+        const size_t B = a->batch, L = a->seqlen, ED = a->d_inner, N = a->d_state;
+        const size_t es = a->dtype == GFE_F32 ? 4 : 2, ns = B * ED * N * sizeof(float);
+        auto act = [&](int64_t bs, int64_t rs, size_t w) {   // bytes from the base of a (B, L, w) strided tensor to its end
+            return ((B - 1) * (size_t)bs + (L - 1) * (size_t)rs + w) * es;
+        };
+        if (overlaps(dlast, ns, dh0, ns) || overlaps(a->du, act(a->du_bs, a->du_rs, ED), dh0, ns) ||
+            overlaps(a->ddelta, act(a->ddelta_bs, a->ddelta_rs, ED), dh0, ns) || overlaps(a->dz, act(a->dz_bs, a->dz_rs, ED), dh0, ns) ||
+            overlaps(a->dBm, act(a->dB_bs, a->dB_rs, N), dh0, ns) || overlaps(a->dCm, act(a->dC_bs, a->dC_rs, N), dh0, ns) ||
+            overlaps(a->dA_log, ED * N * sizeof(float), dh0, ns) || overlaps(a->dD, ED * sizeof(float), dh0, ns) ||
+            overlaps(a->ddt_bias, ED * sizeof(float), dh0, ns)) {
+            gfe::set_error("selscan_bwd_carry: dh0 overlaps dlast or another output");
+            return GFE_ERR_ARG;
+        }
+    }
+    return gfe::launch_bwd_any(a, dlast, dh0, reinterpret_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

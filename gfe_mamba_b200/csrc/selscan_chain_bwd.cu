@@ -23,6 +23,8 @@
 //   phase C  (warp-local item mapping, right after each reverse sweep: only __syncwarp, packed FP32): du, ddelta from the
 //            four quads' partials; dD / ddt_bias accumulation;
 //   then the warps' dB|dC rows are added and leave as one row per (CTA, t) for selscan_bwd_finalize_bc.
+// Backward through a carried state (gfe_selscan_bwd_carry): the last segment starts its reverse carry from dlast instead of
+// zero, and segment 0 stores the carry it ends with, a[0] g[0] = d loss / d h0, to dh0.
 #include <type_traits>
 
 #include "common.cuh"
@@ -245,19 +247,24 @@ __global__ void __launch_bounds__(2 * CPC, kBwdMinBlocks * (64 / CPC)) selscan_b
         const float2 Dc = __ldg(reinterpret_cast<const float2 *>(p.D + c0) + cp);                                                // phase C pair
         float2 dD_acc = make_float2(0.f, 0.f), dbias_acc = make_float2(0.f, 0.f);
 
-        float *carry = cs.independent ? cs.segc + (((size_t)(rseg > 0 ? seg : 0) * p.B + b) * p.ED + c0 + 2 * rp) * kNState + 4 * rq
-                                      : cs.carry + ((size_t)b * p.ED + c0 + 2 * rp) * kNState + 4 * rq;
-        if (rseg > 0) {
-            if (!cs.independent) {
-                if (tid == 0) {
-                    const int *f = cs.flags + (unit - per_seg);
-                    while (ld_acquire(f) == 0) __nanosleep(100);
-                }
-                __syncthreads();
+        // reverse carry in / out of this unit, all (B, ED, 16) states at the same element: in = the later segment's carry-out,
+        // or dlast (the gradient of the final state) for the last segment; out = this segment's carry-out on the waiting
+        // schedule, or dh0 (the gradient of the state before token 0) for segment 0.  NULL: zeros in / nothing out.
+        const size_t off = ((size_t)b * p.ED + c0 + 2 * rp) * kNState + 4 * rq;
+        float *carry = cs.independent ? cs.segc + (size_t)(rseg > 0 ? seg : 0) * p.B * p.ED * kNState + off : cs.carry + off;
+        const float *gin = rseg > 0 ? carry : (p.dlast != nullptr ? p.dlast + off : nullptr);
+        float *gout = seg > 0 ? (cs.independent ? nullptr : carry) : (p.dh0 != nullptr ? p.dh0 + off : nullptr);
+        if (rseg > 0 && !cs.independent) {
+            if (tid == 0) {
+                const int *f = cs.flags + (unit - per_seg);
+                while (ld_acquire(f) == 0) __nanosleep(100);
             }
+            __syncthreads();
+        }
+        if (gin != nullptr) {
 #pragma unroll
             for (int ch = 0; ch < 2; ++ch) {
-                const float4 v = __ldcg(reinterpret_cast<const float4 *>(carry + ch * kNState));
+                const float4 v = __ldcg(reinterpret_cast<const float4 *>(gin + ch * kNState));
                 G[ch][0] = sw ? make_float2(v.y, v.x) : make_float2(v.x, v.y);
                 G[ch][1] = sw ? make_float2(v.w, v.z) : make_float2(v.z, v.w);
             }
@@ -560,16 +567,18 @@ __global__ void __launch_bounds__(2 * CPC, kBwdMinBlocks * (64 / CPC)) selscan_b
             *reinterpret_cast<float2 *>(dst + (size_t)16 * p.ED) = dD_acc;
             *reinterpret_cast<float2 *>(dst + (size_t)17 * p.ED) = dbias_acc;
         }
-        if (seg > 0 && !cs.independent) {
+        if (gout != nullptr) {   // uniform over the CTA
 #pragma unroll
             for (int ch = 0; ch < 2; ++ch) {
                 const float4 gv = sw ? make_float4(G[ch][0].y, G[ch][0].x, G[ch][1].y, G[ch][1].x)
                                      : make_float4(G[ch][0].x, G[ch][0].y, G[ch][1].x, G[ch][1].y);
-                __stcg(reinterpret_cast<float4 *>(carry + ch * kNState), gv);
+                __stcg(reinterpret_cast<float4 *>(gout + ch * kNState), gv);
             }
-            __threadfence();
-            __syncthreads();
-            if (tid == 0) st_release(cs.flags + unit, 1);
+            if (seg > 0) {
+                __threadfence();
+                __syncthreads();
+                if (tid == 0) st_release(cs.flags + unit, 1);
+            }
         }
         cp_async_wait<0>();
         GFE_CLK(0);
@@ -625,7 +634,7 @@ static void launch_bwd_chain_cpc(const ScanParams &p, const ChainSched &cs, bool
 }
 
 template <typename T>
-static int launch_bwd_chain_t(const gfe_selscan_args *a, cudaStream_t st) {
+static int launch_bwd_chain_t(const gfe_selscan_args *a, const float *dlast, float *dh0, cudaStream_t st) {
     const ChainPlan pl = chain_bwd_plan(a->batch, a->seqlen, a->d_inner);
     const int cpc = pl.cpc, nblk = pl.nblk, nseg = pl.nseg;
     const BwdWs w = bwd_ws(a->batch, a->seqlen, a->d_inner);
@@ -647,6 +656,7 @@ static int launch_bwd_chain_t(const gfe_selscan_args *a, cudaStream_t st) {
     p.dBm = a->dBm; p.dB_bs = a->dB_bs; p.dB_rs = a->dB_rs;
     p.dCm = a->dCm; p.dC_bs = a->dC_bs; p.dC_rs = a->dC_rs;
     p.dA_log = a->dA_log; p.dD = a->dD; p.ddt_bias = a->ddt_bias;
+    p.dlast = dlast; p.dh0 = dh0;
     p.nseg = nseg;   // finalize_par sums over B * nseg partial rows
     p.G = nblk;      // finalize_bc sums one row per channel block
     p.bc_interleaved = 1;
@@ -671,11 +681,11 @@ static int launch_bwd_chain_t(const gfe_selscan_args *a, cudaStream_t st) {
     return rc;
 }
 
-int chain_launch_bwd(const gfe_selscan_args *a, cudaStream_t st) {
+int chain_launch_bwd(const gfe_selscan_args *a, const float *dlast, float *dh0, cudaStream_t st) {
     switch (a->dtype) {
-        case GFE_F32: return launch_bwd_chain_t<float>(a, st);
-        case GFE_BF16: return launch_bwd_chain_t<__nv_bfloat16>(a, st);
-        default: return launch_bwd_chain_t<__half>(a, st);
+        case GFE_F32: return launch_bwd_chain_t<float>(a, dlast, dh0, st);
+        case GFE_BF16: return launch_bwd_chain_t<__nv_bfloat16>(a, dlast, dh0, st);
+        default: return launch_bwd_chain_t<__half>(a, dlast, dh0, st);
     }
 }
 

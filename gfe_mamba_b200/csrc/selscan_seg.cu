@@ -11,7 +11,8 @@
 //      and step; one exp2 pair of four runs as a polynomial on the FMA pipe, because this loop is MUFU-bound.
 //   2. combine pass: carry[s + 1] = exp2(A sum_delta[s]) carry[s] + local[s] over the segments, as a two-level scan (32 runs of
 //      up to 8 segments per (b, c, n) element, chained through shared memory); carry[0] is the caller's state h0 (forward from
-//      a carried state, gfe_selscan_fwd_state) or zero.
+//      a carried state, gfe_selscan_fwd_state / _fwd_carry) or zero; in reverse the chain starts from the gradient of the
+//      final state, dlast (gfe_selscan_bwd_carry), or zero.
 //   3. main pass: the chained kernels with ChainSched::independent = 1 (selscan_v4_fwd.cu, selscan_chain_bwd.cu).
 #include "common.cuh"
 #include "selscan_shared.cuh"
@@ -214,7 +215,8 @@ __global__ void __launch_bounds__(2 * CPC, 4 * (64 / CPC)) selscan_seg_summary_k
 
 // carry[slot] <- exp2(A sum_delta[slot]) carry[previous slot] + local[slot], in place; forward: slots ascending (the result is
 // the carry-in of segment slot + 1), reverse: slots descending (the reverse carry-in of segment slot).  The carry before the
-// first slot is h0[(b, c, n)] ((B, ED, 16), the element index) when h0 is not NULL (forward only), else zero.
+// first slot in processing order is h0[(b, c, n)] ((B, ED, 16), the element index) when h0 is not NULL, else zero: the
+// caller's initial state (forward) or the gradient of the final state, dlast (reverse).
 // A CTA of 32 x 32 threads serves 32 consecutive (b, c, n) elements: thread (x, y) owns element x and the y-th run of K <= 8
 // consecutive slots (in processing order).  It loads its run (all loads in flight at once), reduces it to one (P, S) pair,
 // row y = 0 chains the 32 pairs through shared memory, and every thread replays its run from the carry it was handed.
@@ -348,7 +350,7 @@ int seg_launch_carries(const ScanParams &p, const ChainSched &cs, int dtype, int
     int rc = check_launch(rev ? "selscan_bwd segment summary" : "selscan_fwd segment summary");
     if (rc != GFE_OK) return rc;
     const int64_t n_el = (int64_t)p.B * p.ED * kNState;
-    const float *h0 = rev ? nullptr : p.h0;
+    const float *h0 = rev ? p.dlast : p.h0;   // the carry entering the first slot in processing order
     if (cs.nseg - 1 <= 32)
         selscan_seg_combine_seq_kernel<<<(unsigned)ceil_div64(n_el, 256), 256, 0, st>>>(cs.segc, cs.segsd, p.A_log, h0, cs.nseg - 1, p.B, p.ED, rev ? 1 : 0);
     else

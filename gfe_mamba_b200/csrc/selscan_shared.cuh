@@ -31,6 +31,10 @@ struct ScanParams {
     int G;            // ceil(ED / 32)
     int bc_interleaved;   // part_bc rows: 1 = {dB[n], dC[n]} pairs (chained backward), 0 = dB[N] | dC[N] (generic backward)
     const float *h0;      // forward: (B, ED, N) state before token 0 (gfe_selscan_fwd_state), or NULL: zeros
+    // backward through a carried state (gfe_selscan_bwd_carry), (B, ED, N) like last_state, or NULL: dlast seeds the reverse
+    // carry of the last token (NULL: zeros), dh0 receives the reverse carry left after token 0 (NULL: not written)
+    const float *dlast;
+    float *dh0;
 };
 
 constexpr int kPairs = kNState / 2;
@@ -226,6 +230,6 @@ size_t chain_ckpt_state_bytes(int B, int L, int ED, int dtype);
 size_t chain_fwd_workspace_bytes(int B, int L, int ED);
 size_t chain_bwd_workspace_bytes(int B, int L, int ED);
 int chain_launch_fwd(const gfe_selscan_args *a, const float *h0, cudaStream_t st);   // h0: state before token 0, or NULL
-int chain_launch_bwd(const gfe_selscan_args *a, cudaStream_t st);
+int chain_launch_bwd(const gfe_selscan_args *a, const float *dlast, float *dh0, cudaStream_t st);   // NULL, NULL: zero end carry
 
 }  // namespace gfe

@@ -122,7 +122,11 @@ class Mamba(nn.Module):
         call (``_, caches = model.prefill(prompt)``, then ``step`` or ``GraphedDecoder.load_caches(caches)``), in chunks of
         bounded memory, or continued after decoding.  Extension of the reference API (like ``forward_mean``); the layers take
         the scan and conv kernels from the carried state where they are compiled and fall back to ``step`` token by token
-        otherwise (see ``MambaBlock.prefill``).  ``caches`` is not modified."""
+        otherwise (see ``MambaBlock.prefill``).  ``caches`` is not modified.
+
+        Under grad the result is differentiable in the parameters, ``x`` and ``caches``: chunks of a long sequence trained with
+        the returned caches passed on as they are give the gradients of ``forward`` over the whole sequence, and with the
+        caches detached between chunks, truncated backpropagation through time."""
         if not x.is_cuda:
             raise RuntimeError("gfe_mamba_b200.Mamba: CUDA tensors required (this library has no CPU fallback); "
                                f"got input on {x.device}")
@@ -296,14 +300,20 @@ class MambaBlock(nn.Module):
 
     def prefill(self, x, cache):
         """x: (B, L, D); cache: (h, inputs) as for ``step``.  Returns (y (B, L, D), cache): the outputs and the cache of L
-        calls of ``step`` from ``cache``.  Where the kernels are compiled (d_state in ops.FUSED_D_STATES, 2 <= d_conv <= 4) and
-        no gradient is asked for, the forward path runs once over the L tokens from the carried state: in_proj ->
-        conv1d_prefill -> x_proj / dt_proj (inner layernorms included) -> ssm_prefill (gate fused) -> out_proj.  Otherwise
-        ``step`` runs token by token: the reference's semantics, differentiable, any configuration."""
+        calls of ``step`` from ``cache``.  Where the kernels are compiled (d_state in ops.FUSED_D_STATES, 2 <= d_conv <= 4) the
+        forward path runs once over the L tokens from the carried state: in_proj -> conv from the cache -> x_proj / dt_proj
+        (inner layernorms included) -> scan from the state (gate fused) -> out_proj.  With no gradient asked for it takes the
+        inference ops (conv1d_prefill, ssm_prefill: no checkpoints); under grad the differentiable ones
+        (causal_conv1d_silu_state, selective_scan_state), and the returned cache carries gradient back to ``cache``: chunked
+        training passes it on as it is, truncated backpropagation through time detaches it.  Other configurations run
+        ``step`` token by token: the reference's semantics, differentiable."""
         h, inputs = cache
         cfg = self.config
-        if cfg.d_state in ops.FUSED_D_STATES and 2 <= cfg.d_conv <= 4 and self._step_kernels_usable(x, h, inputs):
-            y, cache = self._prefill_inner(x, h, inputs)
+        if cfg.d_state in ops.FUSED_D_STATES and 2 <= cfg.d_conv <= 4:
+            if self._step_kernels_usable(x, h, inputs):
+                y, cache = self._prefill_inner(x, h, inputs, ops.conv1d_prefill, ops.ssm_prefill)
+            else:
+                y, cache = self._prefill_inner(x, h, inputs, ops.causal_conv1d_silu_state, ops.selective_scan_state)
             return self.out_proj(y), cache
         ys = []
         for t in range(x.shape[1]):
@@ -311,14 +321,15 @@ class MambaBlock(nn.Module):
             ys.append(y)
         return torch.stack(ys, 1), cache
 
-    def _prefill_inner(self, x, h, inputs):
+    def _prefill_inner(self, x, h, inputs, conv, scan):
         """prefill between in_proj and out_proj: (y (B, L, ED), (h, inputs)).  A function of its own so that xz, u, delta and
-        x_proj's output are freed before out_proj runs: the peak stays that of forward (whose inner node frees them too)."""
+        x_proj's output are freed before out_proj runs: the peak stays that of forward (whose inner node frees them too).
+        ``conv`` / ``scan``: the inference or the differentiable ops from a carried state (same signatures)."""
         xz = self.in_proj(x)                                  # (B, L, 2*ED)
         xin, z = xz.chunk(2, dim=-1)                          # strided halves, consumed in place
-        u, inputs = ops.conv1d_prefill(xin, inputs, self.conv1d.weight, self.conv1d.bias)
+        u, inputs = conv(xin, inputs, self.conv1d.weight, self.conv1d.bias)
         delta, B, C = self._project(u)
-        y, h = ops.ssm_prefill(u, delta, self.A_log, B, C, self.D, h, z=z, dt_bias=self.dt_proj.bias, delta_softplus=True)
+        y, h = scan(u, delta, self.A_log, B, C, self.D, h, z=z, dt_bias=self.dt_proj.bias, delta_softplus=True)
         return y, (h, inputs)
 
     def _step_kernels_usable(self, *tensors):

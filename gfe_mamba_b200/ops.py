@@ -670,6 +670,181 @@ def ssm_prefill(u, delta, A_log, Bm, Cm, D, h, z=None, dt_bias=None, delta_softp
     return out, h_new
 
 
+# ------------------------------------------------------------ training from a carried state
+def _state16(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    """A (B, ED, N) state as the kernels read it: fp32, contiguous, 16-byte aligned."""
+    t = _f32(t)
+    return t.clone() if (t is not None and t.data_ptr() % 16) else t
+
+
+class _SelectiveScanStateFn(torch.autograd.Function):
+    """selective_scan_fn from a carried state h0 with the final state as a second output, differentiable in both: the
+    forward keeps checkpoints that start from h0, the backward seeds its reverse carry with d h_last and returns d h0."""
+
+    @staticmethod
+    def forward(ctx, u, delta, A_log, Bm, Cm, D, h0, z, dt_bias, softplus: bool, grad_mode: bool):
+        dev = _require_cuda(u, delta, A_log, Bm, Cm, D, h0, z, dt_bias)
+        if u.dim() != 3:
+            raise ValueError(f"selective_scan_state: u must be (B, L, ED); got {tuple(u.shape)}")
+        B, L, ED = u.shape
+        N = A_log.shape[1]
+        dt = u.dtype
+        if dt not in _DT:
+            raise TypeError(f"selective_scan_state: unsupported activation dtype {dt}")
+        if tuple(delta.shape) != (B, L, ED) or tuple(Bm.shape) != (B, L, N) or tuple(Cm.shape) != (B, L, N) \
+                or tuple(A_log.shape) != (ED, N) or tuple(D.shape) != (ED,) or (h0 is not None and tuple(h0.shape) != (B, ED, N)):
+            raise ValueError("selective_scan_state: inconsistent shapes")
+        u_, delta_, Bm_, Cm_ = (_as(t, dt) for t in (u, delta, Bm, Cm))
+        z_ = None if z is None else _as(z, dt)
+        A_log_, D_, bias_ = _f32(A_log), _f32(D), _f32(dt_bias)
+        h0_ = _state16(h0)
+        out = torch.empty((B, L, ED), dtype=dt, device=dev)
+        last = torch.empty((B, ED, N), dtype=torch.float32, device=dev)
+        need_grad = grad_mode and any(ctx.needs_input_grad)
+        l = nat.lib()
+        a = nat.SelscanArgs()
+        _fill_common(a, u_, delta_, z_, Bm_, Cm_, A_log_, D_, bias_, softplus)
+        a.out, a.out_bs, a.out_rs = out.data_ptr(), out.stride(0), out.stride(1)
+        a.last_state = last.data_ptr()
+        with torch.cuda.device(dev):
+            sz = _sizes(B, L, ED, N, dev, _DT[dt])
+            nck = sz[0] if need_grad else 0
+            ckpt = _bytes(nck, dev)
+            ws = _bytes(sz[1], dev)
+            a.ckpt, a.ckpt_bytes = (0 if ckpt is None else ckpt.data_ptr()), nck
+            a.ws, a.ws_bytes = (0 if ws is None else ws.data_ptr()), sz[1]
+            nat.check(l.gfe_selscan_fwd_carry(ctypes.byref(a), _ptr(h0_), _stream(dev)), "selscan_fwd_carry")
+        # an unused output arrives in backward as None: an unused h_last runs the backward with dlast = NULL
+        ctx.set_materialize_grads(False)
+        if need_grad:
+            ctx.save_for_backward(u_, delta_, A_log_, Bm_, Cm_, D_, z_, bias_, ckpt)
+            ctx.softplus = softplus
+            ctx.in_dtypes = tuple(None if t is None else t.dtype for t in (u, delta, A_log, Bm, Cm, D, h0, z, dt_bias))
+        return out, last
+
+    @staticmethod
+    def backward(ctx, dout, dlast):
+        u, delta, A_log, Bm, Cm, D, z, bias, ckpt = ctx.saved_tensors
+        dev = u.device
+        B, L, ED = u.shape
+        N = A_log.shape[1]
+        dt = u.dtype
+        dout = torch.zeros((B, L, ED), dtype=dt, device=dev) if dout is None else _as(dout, dt)
+        dlast = _state16(dlast)
+        du = torch.empty((B, L, ED), dtype=dt, device=dev)
+        ddelta = torch.empty((B, L, ED), dtype=dt, device=dev)
+        dz = None if z is None else torch.empty((B, L, ED), dtype=dt, device=dev)
+        dBm = torch.empty((B, L, N), dtype=dt, device=dev)
+        dCm = torch.empty((B, L, N), dtype=dt, device=dev)
+        dA_log = torch.empty((ED, N), dtype=torch.float32, device=dev)
+        dD = torch.empty((ED,), dtype=torch.float32, device=dev)
+        dbias = None if bias is None else torch.empty((ED,), dtype=torch.float32, device=dev)
+        dh0 = torch.empty((B, ED, N), dtype=torch.float32, device=dev) if ctx.needs_input_grad[6] else None
+        l = nat.lib()
+        a = nat.SelscanArgs()
+        _fill_common(a, u, delta, z, Bm, Cm, A_log, D, bias, ctx.softplus)
+        a.ckpt, a.ckpt_bytes = ckpt.data_ptr(), ckpt.numel()
+        a.dout, a.dout_bs, a.dout_rs = dout.data_ptr(), dout.stride(0), dout.stride(1)
+        a.du, a.du_bs, a.du_rs = du.data_ptr(), du.stride(0), du.stride(1)
+        a.ddelta, a.ddelta_bs, a.ddelta_rs = ddelta.data_ptr(), ddelta.stride(0), ddelta.stride(1)
+        if dz is not None:
+            a.dz, a.dz_bs, a.dz_rs = dz.data_ptr(), dz.stride(0), dz.stride(1)
+        a.dBm, a.dB_bs, a.dB_rs = dBm.data_ptr(), dBm.stride(0), dBm.stride(1)
+        a.dCm, a.dC_bs, a.dC_rs = dCm.data_ptr(), dCm.stride(0), dCm.stride(1)
+        a.dA_log, a.dD = dA_log.data_ptr(), dD.data_ptr()
+        a.ddt_bias = 0 if dbias is None else dbias.data_ptr()
+        with torch.cuda.device(dev):
+            nws = _sizes(B, L, ED, N, dev, _DT[dt])[2]
+            ws = _bytes(nws, dev)
+            a.ws, a.ws_bytes = (0 if ws is None else ws.data_ptr()), nws
+            nat.check(l.gfe_selscan_bwd_carry(ctypes.byref(a), _ptr(dlast), _ptr(dh0), _stream(dev)), "selscan_bwd_carry")
+        dts = ctx.in_dtypes
+
+        def cast(g, i):
+            return None if (g is None or dts[i] is None) else (g if g.dtype == dts[i] else g.to(dts[i]))
+
+        return (cast(du, 0), cast(ddelta, 1), cast(dA_log, 2), cast(dBm, 3), cast(dCm, 4), cast(dD, 5), cast(dh0, 6),
+                cast(dz, 7), cast(dbias, 8), None, None)
+
+
+def selective_scan_state(u, delta, A_log, Bm, Cm, D, h0, z=None, dt_bias=None, delta_softplus: bool = True):
+    """selective_scan_fn started from a carried state, for training in chunks.  h0: (B, ED, N) or None (zeros); the other
+    arguments as for selective_scan_fn.  Returns (out (B, L, ED), h_last (B, ED, N) fp32), both differentiable, h0 included:
+    feeding one chunk's h_last (not detached) as the next chunk's h0 gives the gradients of one pass over the whole sequence,
+    detaching it gives truncated backpropagation through time.  Under no_grad no checkpoint is allocated.  ``h0`` is not
+    modified."""
+    return _SelectiveScanStateFn.apply(u, delta, A_log, Bm, Cm, D, h0, z, dt_bias, bool(delta_softplus), torch.is_grad_enabled())
+
+
+class _CausalConv1dSiluStateFn(torch.autograd.Function):
+    """causal_conv1d_silu over cat(inputs, xin) without its first K-1 rows: the conv from a carried window, differentiable in
+    the window too."""
+
+    @staticmethod
+    def forward(ctx, xin, inputs, weight, bias):
+        dev = _require_cuda(xin, inputs, weight, bias)
+        B, L, ED = xin.shape
+        K = weight.shape[-1]
+        x_ = _rows(xin.detach())
+        in_ = None if inputs is None else inputs.detach().contiguous()
+        w_ = weight.detach().float().reshape(ED, K).contiguous()
+        b_ = _f32(bias)
+        u = torch.empty((B, L, ED), dtype=xin.dtype, device=dev)
+        l = nat.lib()
+        with torch.cuda.device(dev):
+            nat.check(l.gfe_conv1d_silu_fwd_state(_ptr(x_), x_.stride(0), x_.stride(1), _ptr(w_), _ptr(b_), _ptr(in_), None,
+                                                  _ptr(u), u.stride(0), u.stride(1), B, L, ED, K, _DT[xin.dtype], _stream(dev)),
+                      "conv1d_silu_fwd_state")
+        ctx.save_for_backward(x_, in_, w_, b_)
+        ctx.meta = (weight.shape, weight.dtype, None if bias is None else bias.dtype)
+        return u
+
+    @staticmethod
+    def backward(ctx, du):
+        x_, in_, w_, b_ = ctx.saved_tensors
+        dev = x_.device
+        B, L, ED = x_.shape
+        K = w_.shape[1]
+        du = _rows(du.detach().to(x_.dtype))
+        dx = torch.empty((B, L, ED), dtype=x_.dtype, device=dev)
+        dw = torch.empty((ED, K), dtype=torch.float32, device=dev)
+        db = None if b_ is None else torch.empty((ED,), dtype=torch.float32, device=dev)
+        din = torch.empty((B, ED, K - 1), dtype=x_.dtype, device=dev) if ctx.needs_input_grad[1] else None
+        l = nat.lib()
+        with torch.cuda.device(dev):
+            nws = l.gfe_conv1d_bwd_workspace_bytes(B, L, ED, K)
+            ws = _bytes(nws, dev)
+            nat.check(l.gfe_conv1d_silu_bwd_carry(_ptr(x_), x_.stride(0), x_.stride(1), _ptr(w_), _ptr(b_), _ptr(in_), _ptr(du),
+                                                  du.stride(0), du.stride(1), _ptr(dx), dx.stride(0), dx.stride(1), _ptr(dw),
+                                                  _ptr(db), _ptr(din), B, L, ED, K, _DT[x_.dtype], _ptr(ws), nws, _stream(dev)),
+                      "conv1d_silu_bwd_carry")
+        wshape, wdt, bdt = ctx.meta
+        return dx, din, dw.reshape(wshape).to(wdt), (None if db is None else db.to(bdt))
+
+
+def causal_conv1d_silu_state(xin: torch.Tensor, inputs: Optional[torch.Tensor], weight: torch.Tensor,
+                             bias: Optional[torch.Tensor]) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The causal conv + SiLU continuing a carried window, for training in chunks.  xin: (B, L, ED) (any batch / row strides,
+    unit channel stride); inputs: (B, ED, K-1) or None (zeros).  Returns (u (B, L, ED), new_inputs (B, ED, K-1)) as
+    conv1d_prefill does, differentiable in xin, inputs, weight and bias.  ``inputs`` is read in xin's dtype; new_inputs, the
+    last K-1 rows of cat(inputs, xin) along time, is a torch gather, so its gradient reaches both."""
+    _require_cuda(xin, inputs, weight, bias)
+    if xin.dim() != 3:
+        raise ValueError(f"causal_conv1d_silu_state: x must be (B, L, ED); got {tuple(xin.shape)}")
+    B, L, ED = xin.shape
+    K = weight.shape[-1]
+    if xin.dtype not in _DT:
+        raise TypeError(f"causal_conv1d_silu_state: unsupported activation dtype {xin.dtype}")
+    if weight.numel() != ED * K or (inputs is not None and tuple(inputs.shape) != (B, ED, K - 1)):
+        raise ValueError("causal_conv1d_silu_state: weight must be (ED, 1, K) / (ED, K) and inputs (B, ED, K-1)")
+    if inputs is not None:
+        inputs = inputs.to(xin.dtype)
+    u = _CausalConv1dSiluStateFn.apply(xin, inputs, weight, bias)
+    window = inputs if inputs is not None else xin.new_zeros((B, ED, K - 1))
+    new_inputs = torch.cat([window, xin[:, max(0, L - (K - 1)):].transpose(1, 2)], dim=2)[:, :, -(K - 1):].contiguous()
+    return u, new_inputs
+
+
 def ssm_step(u, delta, A_log, Bm, Cm, D, h, z=None, dt_bias=None, delta_softplus: bool = True):
     """One token of the selective scan (mamba.py:375-405).  u, delta, z: (B, ED); Bm, Cm: (B, N); h: (B, ED, N) or None.
     Returns (out, h_new); ``h`` is not modified."""

@@ -13,6 +13,9 @@
  *   gfe_conv1d_step / gfe_ssm_step       cross_atten/mamba.py:357-358,370 and :375-405 (decode step)
  *   gfe_conv1d_silu_fwd_state /          the same forwards continuing a decode cache (prefill: many tokens
  *   gfe_selscan_fwd_state                at once from a (h, conv window) cache, the multi-token decode step)
+ *   gfe_selscan_fwd_carry / _bwd_carry / training from a carried state: the forwards with checkpoints, and the
+ *   gfe_conv1d_silu_bwd_carry            backwards that take the final state's gradient and return the initial
+ *                                        state's (chunked training, truncated BPTT, a trainable prompt cache)
  *
  * Conventions
  *   - every pointer is a DEVICE pointer owned by the caller; the library never
@@ -127,6 +130,15 @@ GFE_API int gfe_selscan_bwd(const gfe_selscan_args *args, void *stream);
  * args->ckpt must be NULL (no backward from here).  args->last_state may be NULL; it must not overlap h0.
  * Same workspace query (gfe_selscan_fwd_workspace_bytes). */
 GFE_API int gfe_selscan_fwd_state(const gfe_selscan_args *args, const float *h0, void *stream);
+/* Training from a carried state.  gfe_selscan_fwd_carry is gfe_selscan_fwd_state with args->ckpt allowed: the checkpoints
+ * then hold the states from h0 on, which is what gfe_selscan_bwd_carry needs.  gfe_selscan_bwd_carry is gfe_selscan_bwd
+ * of such a forward, plus the state gradients:
+ *   dlast: (B, ED, N) fp32 gradient of the loss w.r.t. last_state, or NULL (= zeros: the final state is not used);
+ *   dh0:   (B, ED, N) fp32, receives the gradient w.r.t. h0, or NULL (not computed).
+ * Both contiguous and 16-byte aligned; dh0 must not overlap dlast or any other output.  gfe_selscan_bwd is
+ * gfe_selscan_bwd_carry(args, NULL, NULL, stream).  Same workspace and checkpoint queries. */
+GFE_API int gfe_selscan_fwd_carry(const gfe_selscan_args *args, const float *h0, void *stream);
+GFE_API int gfe_selscan_bwd_carry(const gfe_selscan_args *args, const float *dlast, float *dh0, void *stream);
 
 /* ------------------------------------------------ causal depthwise conv1d --
  * u[b,t,c] = silu(bias[c] + sum_k w[c,k] xin[b, t-(K-1)+k, c]),  xin = 0 for t < 0.
@@ -146,6 +158,16 @@ GFE_API int gfe_conv1d_silu_bwd(const void *xin, int64_t x_bs, int64_t x_rs, con
                                 const void *du, int64_t du_bs, int64_t du_rs,
                                 void *dxin, int64_t dx_bs, int64_t dx_rs, float *dw, float *dbias,
                                 int B, int L, int ED, int K, int dtype, void *ws, size_t ws_bytes, void *stream);
+/* Backward of gfe_conv1d_silu_fwd_state: gfe_conv1d_silu_bwd with rows t < 0 read from inputs (B, ED, K-1) (NULL = zeros,
+ * as in the forward), and dinputs (B, ED, K-1), may be NULL, receiving the gradient w.r.t. inputs:
+ * dinputs[b, c, j] = sum_k w[c, k] dpre[b, j - k, c] over the rows j - k inside [0, L), dpre being the gradient of the
+ * pre-activation (window row j sits at time j - (K-1)).  Both in the activation dtype; they must not overlap.  The gradient of new_inputs is not taken here:
+ * new_inputs is a gather of rows of inputs and xin, which a caller differentiates by itself.  gfe_conv1d_silu_bwd is this
+ * call with inputs = dinputs = NULL. */
+GFE_API int gfe_conv1d_silu_bwd_carry(const void *xin, int64_t x_bs, int64_t x_rs, const float *w, const float *bias,
+                                      const void *inputs, const void *du, int64_t du_bs, int64_t du_rs,
+                                      void *dxin, int64_t dx_bs, int64_t dx_rs, float *dw, float *dbias, void *dinputs,
+                                      int B, int L, int ED, int K, int dtype, void *ws, size_t ws_bytes, void *stream);
 
 /* ------------------------------------------------------------ decode step --
  * gfe_conv1d_step: window = cat(inputs, xin[:, None]) (mamba.py:357); u = silu(conv(window)[K-1]);
