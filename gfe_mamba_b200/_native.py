@@ -62,6 +62,9 @@ SIGNATURES = {
     "gfe_selscan_fwd_state": (ctypes.c_int, [ctypes.POINTER(SelscanArgs), c_vp, c_vp]),
     "gfe_selscan_fwd_carry": (ctypes.c_int, [ctypes.POINTER(SelscanArgs), c_vp, c_vp]),
     "gfe_selscan_bwd_carry": (ctypes.c_int, [ctypes.POINTER(SelscanArgs), c_vp, c_vp, c_vp]),
+    "gfe_selscan_summary_workspace_bytes": (c_sz, [ctypes.c_int] * 4),
+    "gfe_selscan_summary_fwd": (ctypes.c_int, [ctypes.POINTER(SelscanArgs), c_vp, c_vp, c_vp]),
+    "gfe_selscan_summary_bwd": (ctypes.c_int, [ctypes.POINTER(SelscanArgs), c_vp, c_vp]),
     "gfe_conv1d_silu_fwd": (ctypes.c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_i64, c_i64] + [ctypes.c_int] * 5 + [c_vp]),
     "gfe_conv1d_silu_fwd_state": (ctypes.c_int, [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_i64]
                                   + [ctypes.c_int] * 5 + [c_vp]),

@@ -432,8 +432,8 @@ __device__ __forceinline__ void bwd_prep_step(float xraw, float uj, float zj, fl
 }
 
 // Pass A' (only when nseg > 1): reverse-scan carry a[t0]*g[t0] of a segment from a zero incoming carry,
-// plus sum(delta) of the segment.
-template <typename T, bool HAS_Z, int N>
+// plus sum(delta) of the segment.  SEG0 = 0: segment 0 too (the summary of a whole range, gfe_selscan_summary_bwd).
+template <typename T, bool HAS_Z, int N, int SEG0 = 1>
 __global__ void __launch_bounds__(128) selscan_bwd_summary_kernel(ScanParams p) {
     constexpr int P = N / 2;
     extern __shared__ float smem[];
@@ -443,7 +443,7 @@ __global__ void __launch_bounds__(128) selscan_bwd_summary_kernel(ScanParams p) 
     const int c_raw = g * 32 + lane;
     const bool active = c_raw < p.ED;
     const int c = active ? c_raw : p.ED - 1;
-    const int seg = blockIdx.y + 1, b = blockIdx.z;   // segment 0's carry-out is never needed
+    const int seg = blockIdx.y + SEG0, b = blockIdx.z;   // segment 0's carry-out is needed by a whole-range summary only
     const int t0 = seg * p.seg_len, t1 = min(p.L, t0 + p.seg_len);
     float *sBC = smem + warp * summary_smem_floats<N>();
     float2 *sA2 = reinterpret_cast<float2 *>(sBC + kChunk * row_stride<N>());
@@ -1042,6 +1042,89 @@ static int validate_h0(const gfe_selscan_args *a, const float *h0, const char *w
     return GFE_OK;
 }
 
+// ---- the summary of a whole range (gfe_selscan_summary_fwd / _bwd), generic family ----
+// Segments as plan_segments cuts them, every one from a zero carry: the summary kernels above over all nseg segments, then
+// the fold of selscan_seg.cu.  Workspace: seg_h [B][nseg][N / 2][ED] float2 and seg_sd [B][nseg][ED].
+static WsLayout summary_ws_layout(int B, int L, int ED, int N) {
+    const SegPlan sp = plan_segments(B, L, ED);
+    WsLayout w{};
+    w.seg_h = 0;
+    w.seg_sd = align_up((size_t)B * sp.nseg * N * ED * sizeof(float), 256);
+    w.total = w.seg_sd + align_up((size_t)B * sp.nseg * ED * sizeof(float), 256);
+    return w;
+}
+
+template <typename T, int N>
+static int launch_summary(const gfe_selscan_args *a, bool rev, float *out, float *sum_delta, cudaStream_t st) {
+    const SegPlan sp = plan_segments(a->batch, a->seqlen, a->d_inner);
+    const WsLayout wl = summary_ws_layout(a->batch, a->seqlen, a->d_inner, N);
+    if (a->ws == nullptr || a->ws_bytes < wl.total) {
+        set_error("%s: workspace too small (%zu < %zu)", rev ? "selscan_summary_bwd" : "selscan_summary_fwd",
+                  a->ws ? a->ws_bytes : (size_t)0, wl.total);
+        return GFE_ERR_WORKSPACE;
+    }
+    ScanParams p{};
+    fill_common(p, a, sp);
+    p.ckpt = nullptr; p.ysave = nullptr;
+    p.dout = a->dout; p.do_bs = a->dout_bs; p.do_rs = a->dout_rs;
+    char *ws = reinterpret_cast<char *>(a->ws);
+    p.seg_h = reinterpret_cast<float2 *>(ws + wl.seg_h);
+    p.seg_sd = reinterpret_cast<float *>(ws + wl.seg_sd);
+    const dim3 grid(p.G, sp.nseg, a->batch), block(32);
+    const size_t smem = summary_smem_floats<N>() * sizeof(float);
+    if (!rev) selscan_fwd_summary_kernel<T, N><<<grid, block, smem, st>>>(p);
+    else if (a->z != nullptr) selscan_bwd_summary_kernel<T, true, N, 0><<<grid, block, smem, st>>>(p);
+    else selscan_bwd_summary_kernel<T, false, N, 0><<<grid, block, smem, st>>>(p);
+    int rc = check_launch(rev ? "selscan_bwd_summary" : "selscan_fwd_summary");
+    if (rc != GFE_OK) return rc;
+    return launch_summary_total(reinterpret_cast<const float *>(p.seg_h), p.seg_sd, a->A_log, out, sum_delta, sp.nseg, a->batch,
+                                a->d_inner, N, true, rev, st);
+}
+
+template <typename T>
+static int launch_summary_n(const gfe_selscan_args *a, bool rev, float *out, float *sum_delta, cudaStream_t st) {
+    switch (a->d_state) {
+        case 16: return launch_summary<T, 16>(a, rev, out, sum_delta, st);
+        case 32: return launch_summary<T, 32>(a, rev, out, sum_delta, st);
+        default: return launch_summary<T, 64>(a, rev, out, sum_delta, st);
+    }
+}
+
+// Arguments of gfe_selscan_summary_fwd / _bwd: only the inputs that direction reads are required (forward: u, delta, Bm;
+// reverse: dout, delta, Cm, z optional), A_log as in validate_common, the (B, ED, N) state output 16-byte aligned like
+// last_state and apart from sum_delta.
+static int validate_summary(const gfe_selscan_args *a, bool rev, const float *out, const float *sum_delta) {
+    const char *who = rev ? "selscan_summary_bwd" : "selscan_summary_fwd";
+    if (a == nullptr) { set_error("%s: args is NULL", who); return GFE_ERR_ARG; }
+    if (a->batch <= 0 || a->seqlen <= 0 || a->d_inner <= 0) { set_error("%s: non-positive shape", who); return GFE_ERR_ARG; }
+    if (!fused_d_state(a->d_state)) {
+        set_error("%s: d_state=%d unsupported by the fused kernel (compiled for 16, 32 and 64)", who, a->d_state);
+        return GFE_ERR_UNSUPPORTED;
+    }
+    if (a->dtype != GFE_F32 && a->dtype != GFE_BF16 && a->dtype != GFE_F16) { set_error("%s: bad dtype %d", who, a->dtype); return GFE_ERR_DTYPE; }
+    const bool missing = rev ? (!a->dout || !a->delta || !a->Cm) : (!a->u || !a->delta || !a->Bm);
+    if (missing || !a->A_log) { set_error("%s: NULL input pointer", who); return GFE_ERR_ARG; }
+    if ((reinterpret_cast<uintptr_t>(a->A_log) & 15) != 0) { set_error("%s: A_log must be 16-byte aligned", who); return GFE_ERR_ARG; }
+    if (out == nullptr || (!rev && sum_delta == nullptr)) { set_error("%s: NULL output pointer", who); return GFE_ERR_ARG; }
+    if ((reinterpret_cast<uintptr_t>(out) & 15) != 0 || (reinterpret_cast<uintptr_t>(sum_delta) & 3) != 0) {
+        set_error("%s: the state output must be 16-byte aligned and sum_delta 4-byte aligned", who);
+        return GFE_ERR_ARG;
+    }
+    const size_t ns = (size_t)a->batch * a->d_inner * a->d_state * sizeof(float), nd = (size_t)a->batch * a->d_inner * sizeof(float);
+    if (overlaps(out, ns, sum_delta, nd)) { set_error("%s: the state output and sum_delta overlap", who); return GFE_ERR_ARG; }
+    return GFE_OK;
+}
+
+static int launch_summary_any(const gfe_selscan_args *a, bool rev, float *out, float *sum_delta, cudaStream_t st) {
+    ScopedKernelTimer tm(rev ? K_SELSCAN_BWD_SUMMARY : K_SELSCAN_FWD_SUMMARY, st);
+    if (chain_applicable(a->batch, a->seqlen, a->d_inner, a->d_state)) return chain_launch_summary(a, rev, out, sum_delta, st);
+    switch (a->dtype) {
+        case GFE_F32: return launch_summary_n<float>(a, rev, out, sum_delta, st);
+        case GFE_BF16: return launch_summary_n<__nv_bfloat16>(a, rev, out, sum_delta, st);
+        default: return launch_summary_n<__half>(a, rev, out, sum_delta, st);
+    }
+}
+
 }  // namespace gfe
 
 extern "C" {
@@ -1095,6 +1178,24 @@ GFE_API int gfe_selscan_fwd_carry(const gfe_selscan_args *a, const float *h0, vo
     rc = gfe::validate_h0(a, h0, "selscan_fwd_carry");
     if (rc != GFE_OK) return rc;
     return gfe::launch_fwd_any(a, h0, reinterpret_cast<cudaStream_t>(stream));
+}
+
+GFE_API size_t gfe_selscan_summary_workspace_bytes(int B, int L, int ED, int N) {
+    if (B <= 0 || L <= 0 || ED <= 0 || !gfe::fused_d_state(N)) return 0;
+    if (gfe::chain_applicable(B, L, ED, N)) return gfe::chain_summary_workspace_bytes(B, L, ED);
+    return gfe::summary_ws_layout(B, L, ED, N).total;
+}
+
+GFE_API int gfe_selscan_summary_fwd(const gfe_selscan_args *a, float *h_loc, float *sum_delta, void *stream) {
+    int rc = gfe::validate_summary(a, false, h_loc, sum_delta);
+    if (rc != GFE_OK) return rc;
+    return gfe::launch_summary_any(a, false, h_loc, sum_delta, reinterpret_cast<cudaStream_t>(stream));
+}
+
+GFE_API int gfe_selscan_summary_bwd(const gfe_selscan_args *a, float *g_loc, void *stream) {
+    int rc = gfe::validate_summary(a, true, g_loc, nullptr);
+    if (rc != GFE_OK) return rc;
+    return gfe::launch_summary_any(a, true, g_loc, nullptr, reinterpret_cast<cudaStream_t>(stream));
 }
 
 GFE_API int gfe_selscan_bwd(const gfe_selscan_args *a, void *stream) {

@@ -11,6 +11,8 @@ template <typename T>
 void v4_launch_fwd_kernel(const ScanParams &p, const ChainSched &cs, int cpc, bool has_z, int cpb, cudaStream_t st);   // selscan_v4_fwd.cu
 
 int seg_launch_carries(const ScanParams &p, const ChainSched &cs, int dtype, int cpc, bool rev, bool has_z, int cpb, cudaStream_t st);   // selscan_seg.cu
+int seg_launch_total(const ScanParams &p, const ChainSched &cs, int dtype, int cpc, bool rev, bool has_z, int cpb, float *out,
+                     float *sum_delta, cudaStream_t st);   // selscan_seg.cu
 
 // L is cut into chained segments, ~12 units per resident CTA: the units of a chain interleave with those of the others and
 // hop between SMs, which evens out SMs that host 2 and 3 working CTAs (measured on cfg3, profiles/r02_chain_variants.txt:
@@ -199,6 +201,69 @@ int chain_launch_fwd(const gfe_selscan_args *a, const float *h0, cudaStream_t st
         case GFE_BF16: return launch_fwd_chain_t<__nv_bfloat16>(a, h0, st);
         default: return launch_fwd_chain_t<__half>(a, h0, st);
     }
+}
+
+// ---- the summary of a whole range (gfe_selscan_summary_fwd / _bwd) ----
+// Independent segments for every B * ED, cut as for the forward's summary pass; both directions take the same plan, so one
+// workspace query serves both.  Workspace: the unit counter, then nseg slots of local aggregates [nseg][B][ED][16] and of
+// sum(delta) [nseg][B][ED].
+static ChainPlan chain_summary_plan(int B, int L, int ED) {
+    ChainPlan pl{};
+    pl.cpc = chain_cpc(ED);
+    pl.nblk = ED / pl.cpc;
+    pl.independent = 1;
+    chain_plan(B, L, pl.nblk, kFwdMinBlocks * (64 / pl.cpc), true, pl.nseg, pl.seg_len);
+    return pl;
+}
+
+struct SummaryLayout {
+    size_t counter, segc, segsd, total;
+};
+static SummaryLayout chain_summary_layout(int B, int ED, const ChainPlan &pl) {
+    SummaryLayout c{};
+    size_t off = 256;   // counter
+    c.segc = off;
+    off += align_up((size_t)pl.nseg * B * ED * kNState * sizeof(float), 256);
+    c.segsd = off;
+    off += align_up((size_t)pl.nseg * B * ED * sizeof(float), 256);
+    c.total = off;
+    return c;
+}
+
+size_t chain_summary_workspace_bytes(int B, int L, int ED) { return chain_summary_layout(B, ED, chain_summary_plan(B, L, ED)).total; }
+
+int chain_launch_summary(const gfe_selscan_args *a, bool rev, float *out, float *sum_delta, cudaStream_t st) {
+    const ChainPlan pl = chain_summary_plan(a->batch, a->seqlen, a->d_inner);
+    const SummaryLayout cl = chain_summary_layout(a->batch, a->d_inner, pl);
+    const char *who = rev ? "selscan_summary_bwd" : "selscan_summary_fwd";
+    if (a->ws == nullptr || a->ws_bytes < cl.total) {
+        set_error("%s: workspace too small (%zu < %zu)", who, a->ws ? a->ws_bytes : (size_t)0, cl.total);
+        return GFE_ERR_WORKSPACE;
+    }
+    if (a->dt_bias && (reinterpret_cast<uintptr_t>(a->dt_bias) & 7) != 0) {   // read two channels at a time
+        set_error("%s: dt_bias must be 8-byte aligned", who);
+        return GFE_ERR_ARG;
+    }
+    ScanParams p{};
+    chain_fill_params(p, a);
+    if (rev) { p.dout = a->dout; p.do_bs = a->dout_bs; p.do_rs = a->dout_rs; }
+    else p.z = nullptr;   // the forward summary never reads z
+    char *ws = reinterpret_cast<char *>(a->ws);
+    ChainSched cs{};
+    cs.counter = reinterpret_cast<int *>(ws + cl.counter);
+    cs.segc = cs.carry = reinterpret_cast<float *>(ws + cl.segc);
+    cs.segsd = reinterpret_cast<float *>(ws + cl.segsd);
+    cs.nseg = pl.nseg;
+    cs.seg_len = pl.seg_len;
+    cs.nblk = pl.nblk;
+    cs.independent = 1;
+    if (cudaMemsetAsync(cs.counter, 0, sizeof(int), st) != cudaSuccess) return check_launch("selscan summary memset");
+    gfe_selscan_args b = *a;   // staging checks of the tensors this direction reads
+    if (rev) { b.u = nullptr; b.Bm = nullptr; }
+    else { b.z = nullptr; b.Cm = nullptr; }
+    b.ckpt = nullptr;
+    const int cpb = chain_cpb(&b, rev);
+    return seg_launch_total(p, cs, a->dtype, pl.cpc, rev, rev && a->z != nullptr, cpb, out, sum_delta, st);
 }
 
 }  // namespace gfe

@@ -33,7 +33,8 @@ struct SegSumSmem {
 
 // REV = false: forward aggregate of segments 0 .. nseg-2 (slot = segment);  v = delta u,        h = a h + v B
 // REV = true : reverse aggregate of segments 1 .. nseg-1 (slot = segment - 1);  v = dout silu(z), G = a (G + v C)
-template <typename T, bool HAS_Z, int CPB, int CPC, bool REV>
+// SLOT0 = 0 with REV: every segment, slot = segment (the summary of a whole range, seg_launch_total)
+template <typename T, bool HAS_Z, int CPB, int CPC, bool REV, int SLOT0 = REV ? 1 : 0>
 __global__ void __launch_bounds__(2 * CPC, 4 * (64 / CPC)) selscan_seg_summary_kernel(ScanParams p, ChainSched cs) {
     extern __shared__ __align__(16) unsigned char smem[];
     __shared__ int s_unit;
@@ -62,7 +63,7 @@ __global__ void __launch_bounds__(2 * CPC, 4 * (64 / CPC)) selscan_seg_summary_k
         const int unit = s_unit;
         if (unit >= cs.total) break;
         const int slot = unit / per_seg;
-        const int seg = REV ? slot + 1 : slot;
+        const int seg = slot + SLOT0;
         const int rem = unit - slot * per_seg;
         const int b = rem / cs.nblk;
         const int c0 = (rem - b * cs.nblk) * CPC;
@@ -305,26 +306,86 @@ __global__ void __launch_bounds__(256) selscan_seg_combine_seq_kernel(float *__r
     }
 }
 
-// ---------------------------------------------------------------------------------------------------- host
-template <typename T, bool HAS_Z, int CPB, int CPC, bool REV>
-static void launch_summary_inst(const ScanParams &p, const ChainSched &cs, cudaStream_t st) {
-    constexpr size_t smem = SegSumSmem<T, HAS_Z, CPC>::kTotal;
-    const int grid = persistent_grid<selscan_seg_summary_kernel<T, HAS_Z, CPB, CPC, REV>>(2 * CPC, smem, cs.total);
-    selscan_seg_summary_kernel<T, HAS_Z, CPB, CPC, REV><<<grid, 2 * CPC, smem, st>>>(p, cs);
+// Fold of per-segment summaries into the summary of a whole range (gfe_selscan_summary_fwd / _bwd): for every (b, c, n)
+// element, out = the carry chain over all nseg segments from a zero carry, carry = exp2(A sum_delta[s]) carry + local[s],
+// segments ascending (forward) or descending (reverse); sum_delta (may be NULL) = the sum over s of sum_delta[s].  The
+// segment summaries are in the chained layout (GEN = false: local [s][B][ED][16], sum_delta [s][B][ED]) or in the generic
+// one (GEN = true: local [B][s][N / 2][ED] float2, sum_delta [B][s][ED]).  out: (B, ED, N); sum_delta: (B, ED).
+template <int N, bool GEN>
+__global__ void __launch_bounds__(256) selscan_summary_total_kernel(const float *__restrict__ loc, const float *__restrict__ segsd,
+                                                                    const float *__restrict__ A_log, float *__restrict__ out,
+                                                                    float *__restrict__ sum_delta, int nseg, int B, int ED, int rev) {
+    const int64_t n_el = (int64_t)B * ED * N;
+    const int64_t idx = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (idx >= n_el) return;
+    const int n = (int)(idx % N);
+    const int64_t bc = idx / N;
+    const int64_t b = bc / ED, c = bc % ED;
+    const float a2 = -expf(__ldg(A_log + c * N + n)) * kLog2e;
+    float H = 0.f, S = 0.f;
+    for (int i = 0; i < nseg; ++i) {
+        const int64_t s = rev ? nseg - 1 - i : i;
+        const int64_t si = GEN ? (b * nseg + s) * ED + c : (s * B + b) * ED + c;
+        const int64_t li = GEN ? (((b * nseg + s) * (N / 2) + n / 2) * ED + c) * 2 + (n & 1) : s * n_el + idx;
+        const float sd = __ldcg(segsd + si);
+        H = fmaf(ex2_approx(a2 * sd), H, __ldcg(loc + li));
+        S += sd;
+    }
+    out[idx] = H;
+    if (sum_delta != nullptr && n == 0) sum_delta[bc] = S;
 }
 
-template <typename T, int CPC>
+int launch_summary_total(const float *loc, const float *segsd, const float *A_log, float *out, float *sum_delta, int nseg, int B,
+                         int ED, int N, bool generic, bool rev, cudaStream_t st) {
+    const unsigned grid = (unsigned)ceil_div64((int64_t)B * ED * N, 256);
+    const int r = rev ? 1 : 0;
+    if (!generic) selscan_summary_total_kernel<kNState, false><<<grid, 256, 0, st>>>(loc, segsd, A_log, out, sum_delta, nseg, B, ED, r);
+    else if (N == 16) selscan_summary_total_kernel<16, true><<<grid, 256, 0, st>>>(loc, segsd, A_log, out, sum_delta, nseg, B, ED, r);
+    else if (N == 32) selscan_summary_total_kernel<32, true><<<grid, 256, 0, st>>>(loc, segsd, A_log, out, sum_delta, nseg, B, ED, r);
+    else selscan_summary_total_kernel<64, true><<<grid, 256, 0, st>>>(loc, segsd, A_log, out, sum_delta, nseg, B, ED, r);
+    return check_launch("selscan summary total");
+}
+
+// ---------------------------------------------------------------------------------------------------- host
+template <typename T, bool HAS_Z, int CPB, int CPC, bool REV, int SLOT0>
+static void launch_summary_inst(const ScanParams &p, const ChainSched &cs, cudaStream_t st) {
+    constexpr size_t smem = SegSumSmem<T, HAS_Z, CPC>::kTotal;
+    const int grid = persistent_grid<selscan_seg_summary_kernel<T, HAS_Z, CPB, CPC, REV, SLOT0>>(2 * CPC, smem, cs.total);
+    selscan_seg_summary_kernel<T, HAS_Z, CPB, CPC, REV, SLOT0><<<grid, 2 * CPC, smem, st>>>(p, cs);
+}
+
+// RSLOT0: slot of segment 0 in reverse (1: segments 1 .. nseg-1 for the carries, 0: every segment for a total)
+template <typename T, int CPC, int RSLOT0>
 static void launch_summary_cpc(const ScanParams &p, const ChainSched &cs, bool rev, bool has_z, int cpb, cudaStream_t st) {
     if (!rev) {   // the forward aggregate never needs z
-        if (cpb == 16) launch_summary_inst<T, false, 16, CPC, false>(p, cs, st);
-        else launch_summary_inst<T, false, 0, CPC, false>(p, cs, st);
+        if (cpb == 16) launch_summary_inst<T, false, 16, CPC, false, 0>(p, cs, st);
+        else launch_summary_inst<T, false, 0, CPC, false, 0>(p, cs, st);
     } else if (has_z) {
-        if (cpb == 16) launch_summary_inst<T, true, 16, CPC, true>(p, cs, st);
-        else launch_summary_inst<T, true, 0, CPC, true>(p, cs, st);
+        if (cpb == 16) launch_summary_inst<T, true, 16, CPC, true, RSLOT0>(p, cs, st);
+        else launch_summary_inst<T, true, 0, CPC, true, RSLOT0>(p, cs, st);
     } else {
-        if (cpb == 16) launch_summary_inst<T, false, 16, CPC, true>(p, cs, st);
-        else launch_summary_inst<T, false, 0, CPC, true>(p, cs, st);
+        if (cpb == 16) launch_summary_inst<T, false, 16, CPC, true, RSLOT0>(p, cs, st);
+        else launch_summary_inst<T, false, 0, CPC, true, RSLOT0>(p, cs, st);
     }
+}
+
+template <int RSLOT0>
+static int launch_summaries(const ScanParams &p, const ChainSched &s, int dtype, int cpc, bool rev, bool has_z, int cpb, cudaStream_t st) {
+    switch (dtype) {
+        case GFE_F32:
+            if (cpc == 64) launch_summary_cpc<float, 64, RSLOT0>(p, s, rev, has_z, cpb, st);
+            else launch_summary_cpc<float, 32, RSLOT0>(p, s, rev, has_z, cpb, st);
+            break;
+        case GFE_BF16:
+            if (cpc == 64) launch_summary_cpc<__nv_bfloat16, 64, RSLOT0>(p, s, rev, has_z, cpb, st);
+            else launch_summary_cpc<__nv_bfloat16, 32, RSLOT0>(p, s, rev, has_z, cpb, st);
+            break;
+        default:
+            if (cpc == 64) launch_summary_cpc<__half, 64, RSLOT0>(p, s, rev, has_z, cpb, st);
+            else launch_summary_cpc<__half, 32, RSLOT0>(p, s, rev, has_z, cpb, st);
+            break;
+    }
+    return check_launch(rev ? "selscan_bwd segment summary" : "selscan_fwd segment summary");
 }
 
 // Summary + combine for the independent segments of `cs` (cs.nseg > 1): fills cs.segc with every segment's carry-in.
@@ -333,21 +394,7 @@ int seg_launch_carries(const ScanParams &p, const ChainSched &cs, int dtype, int
     ChainSched s = cs;
     s.counter = cs.counter + 16;
     s.total = (cs.nseg - 1) * p.B * cs.nblk;
-    switch (dtype) {
-        case GFE_F32:
-            if (cpc == 64) launch_summary_cpc<float, 64>(p, s, rev, has_z, cpb, st);
-            else launch_summary_cpc<float, 32>(p, s, rev, has_z, cpb, st);
-            break;
-        case GFE_BF16:
-            if (cpc == 64) launch_summary_cpc<__nv_bfloat16, 64>(p, s, rev, has_z, cpb, st);
-            else launch_summary_cpc<__nv_bfloat16, 32>(p, s, rev, has_z, cpb, st);
-            break;
-        default:
-            if (cpc == 64) launch_summary_cpc<__half, 64>(p, s, rev, has_z, cpb, st);
-            else launch_summary_cpc<__half, 32>(p, s, rev, has_z, cpb, st);
-            break;
-    }
-    int rc = check_launch(rev ? "selscan_bwd segment summary" : "selscan_fwd segment summary");
+    int rc = launch_summaries<1>(p, s, dtype, cpc, rev, has_z, cpb, st);
     if (rc != GFE_OK) return rc;
     const int64_t n_el = (int64_t)p.B * p.ED * kNState;
     const float *h0 = rev ? p.dlast : p.h0;   // the carry entering the first slot in processing order
@@ -356,6 +403,18 @@ int seg_launch_carries(const ScanParams &p, const ChainSched &cs, int dtype, int
     else
         selscan_seg_combine_kernel<<<(unsigned)ceil_div64(n_el, 32), dim3(32, 32), 0, st>>>(cs.segc, cs.segsd, p.A_log, h0, cs.nseg - 1, p.B, p.ED, rev ? 1 : 0);
     return check_launch("selscan segment combine");
+}
+
+// The summary of the whole range [0, L) (gfe_selscan_summary_fwd / _bwd) for the chained family: every segment of `cs`
+// from a zero carry (slot = segment; cs.segc / cs.segsd hold cs.nseg slots, *cs.counter is zero), folded into out (B, ED, 16)
+// and, forward, sum_delta (B, ED).
+int seg_launch_total(const ScanParams &p, const ChainSched &cs, int dtype, int cpc, bool rev, bool has_z, int cpb, float *out,
+                     float *sum_delta, cudaStream_t st) {
+    ChainSched s = cs;
+    s.total = cs.nseg * p.B * cs.nblk;
+    int rc = launch_summaries<0>(p, s, dtype, cpc, rev, has_z, cpb, st);
+    if (rc != GFE_OK) return rc;
+    return launch_summary_total(cs.segc, cs.segsd, p.A_log, out, sum_delta, cs.nseg, p.B, p.ED, kNState, false, rev, st);
 }
 
 }  // namespace gfe

@@ -231,5 +231,10 @@ size_t chain_fwd_workspace_bytes(int B, int L, int ED);
 size_t chain_bwd_workspace_bytes(int B, int L, int ED);
 int chain_launch_fwd(const gfe_selscan_args *a, const float *h0, cudaStream_t st);   // h0: state before token 0, or NULL
 int chain_launch_bwd(const gfe_selscan_args *a, const float *dlast, float *dh0, cudaStream_t st);   // NULL, NULL: zero end carry
+// the summary of a whole range (gfe_selscan_summary_fwd / _bwd): chained family, and the fold both families end with
+size_t chain_summary_workspace_bytes(int B, int L, int ED);
+int chain_launch_summary(const gfe_selscan_args *a, bool rev, float *out, float *sum_delta, cudaStream_t st);
+int launch_summary_total(const float *loc, const float *segsd, const float *A_log, float *out, float *sum_delta, int nseg, int B,
+                         int ED, int N, bool generic, bool rev, cudaStream_t st);   // selscan_seg.cu
 
 }  // namespace gfe

@@ -845,6 +845,70 @@ def causal_conv1d_silu_state(xin: torch.Tensor, inputs: Optional[torch.Tensor], 
     return u, new_inputs
 
 
+# ------------------------------------------------------------ summaries of a whole range
+def _summary_call(fn: str, x, delta, A_log, BC, z, dt_bias, softplus: bool, rev: bool):
+    """gfe_selscan_summary_fwd (x = u, BC = Bm) or _bwd (x = dout, BC = Cm): (state (B, ED, N) fp32, sum_delta (B, ED) fp32
+    or None)."""
+    dev = _require_cuda(x, delta, A_log, BC, z, dt_bias)
+    _no_autograd(fn, x, delta, A_log, BC, z, dt_bias)
+    if x.dim() != 3:
+        raise ValueError(f"{fn}: activations must be (B, L, ED); got {tuple(x.shape)}")
+    B, L, ED = x.shape
+    N = A_log.shape[1]
+    dt = x.dtype
+    if dt not in _DT:
+        raise TypeError(f"{fn}: unsupported activation dtype {dt}")
+    if tuple(delta.shape) != (B, L, ED) or tuple(BC.shape) != (B, L, N) or tuple(A_log.shape) != (ED, N) \
+            or (z is not None and tuple(z.shape) != (B, L, ED)):
+        raise ValueError(f"{fn}: inconsistent shapes")
+    x_, delta_, BC_ = (_as(t, dt) for t in (x, delta, BC))
+    z_ = None if z is None else _as(z, dt)
+    A_log_, bias_ = _f32(A_log), _f32(dt_bias)
+    state = torch.empty((B, ED, N), dtype=torch.float32, device=dev)
+    sd = None if rev else torch.empty((B, ED), dtype=torch.float32, device=dev)
+    l = nat.lib()
+    a = nat.SelscanArgs()
+    a.batch, a.seqlen, a.d_inner, a.d_state = B, L, ED, N
+    a.dtype = _DT[dt]
+    a.flags = nat.GFE_FLAG_DELTA_SOFTPLUS if softplus else 0
+    a.delta, a.delta_bs, a.delta_rs = delta_.data_ptr(), delta_.stride(0), delta_.stride(1)
+    if rev:
+        a.dout, a.dout_bs, a.dout_rs = x_.data_ptr(), x_.stride(0), x_.stride(1)
+        a.Cm, a.C_bs, a.C_rs = BC_.data_ptr(), BC_.stride(0), BC_.stride(1)
+        if z_ is not None:
+            a.z, a.z_bs, a.z_rs = z_.data_ptr(), z_.stride(0), z_.stride(1)
+    else:
+        a.u, a.u_bs, a.u_rs = x_.data_ptr(), x_.stride(0), x_.stride(1)
+        a.Bm, a.B_bs, a.B_rs = BC_.data_ptr(), BC_.stride(0), BC_.stride(1)
+    a.A_log = A_log_.data_ptr()
+    a.dt_bias = 0 if bias_ is None else bias_.data_ptr()
+    with torch.cuda.device(dev):
+        nws = l.gfe_selscan_summary_workspace_bytes(B, L, ED, N)
+        ws = _bytes(nws, dev)
+        a.ws, a.ws_bytes = (0 if ws is None else ws.data_ptr()), nws
+        if rev:
+            nat.check(l.gfe_selscan_summary_bwd(ctypes.byref(a), _ptr(state), _stream(dev)), "selscan_summary_bwd")
+        else:
+            nat.check(l.gfe_selscan_summary_fwd(ctypes.byref(a), _ptr(state), _ptr(sd), _stream(dev)), "selscan_summary_fwd")
+    return state, sd
+
+
+def selscan_summary(u, delta, A_log, Bm, dt_bias=None, delta_softplus: bool = True) -> Tuple[torch.Tensor, torch.Tensor]:
+    """What a range of tokens does to the scan state, for passing state between devices that each hold part of a sequence.
+    u, delta: (B, L, ED); Bm: (B, L, N) (any batch / row strides, unit channel stride); A_log: (ED, N).  Returns (h_loc
+    (B, ED, N) fp32, sum_delta (B, ED) fp32): the final state of ``selective_scan_fn`` over the L tokens started from zero, and
+    the sum over the tokens of the step size (softplus(delta + dt_bias) with ``delta_softplus``, else delta + dt_bias).  The
+    state after the range from a state h is exp(A sum_delta) h + h_loc per state, A = -exp(A_log).  Inference only."""
+    return _summary_call("selscan_summary", u, delta, A_log, Bm, None, dt_bias, delta_softplus, False)
+
+
+def selscan_summary_rev(dout, delta, A_log, Cm, z=None, dt_bias=None, delta_softplus: bool = True) -> torch.Tensor:
+    """The reverse counterpart of ``selscan_summary``: g_loc (B, ED, N) fp32, the gradient of the state before the range that
+    the output gradient ``dout`` (B, L, ED) alone produces -- d h0 of ``selective_scan_state`` with no gradient on its final
+    state.  With a final-state gradient dlast it is exp(A sum_delta) dlast + g_loc.  z: the gate, or None.  Inference only."""
+    return _summary_call("selscan_summary_rev", dout, delta, A_log, Cm, z, dt_bias, delta_softplus, True)[0]
+
+
 def ssm_step(u, delta, A_log, Bm, Cm, D, h, z=None, dt_bias=None, delta_softplus: bool = True):
     """One token of the selective scan (mamba.py:375-405).  u, delta, z: (B, ED); Bm, Cm: (B, N); h: (B, ED, N) or None.
     Returns (out, h_new); ``h`` is not modified."""

@@ -16,6 +16,8 @@
  *   gfe_selscan_fwd_carry / _bwd_carry / training from a carried state: the forwards with checkpoints, and the
  *   gfe_conv1d_silu_bwd_carry            backwards that take the final state's gradient and return the initial
  *                                        state's (chunked training, truncated BPTT, a trainable prompt cache)
+ *   gfe_selscan_summary_fwd / _bwd       a range's end state from zero and its reverse counterpart: what one
+ *                                        device of a sequence split over devices passes to the others
  *
  * Conventions
  *   - every pointer is a DEVICE pointer owned by the caller; the library never
@@ -139,6 +141,21 @@ GFE_API int gfe_selscan_fwd_state(const gfe_selscan_args *args, const float *h0,
  * gfe_selscan_bwd_carry(args, NULL, NULL, stream).  Same workspace and checkpoint queries. */
 GFE_API int gfe_selscan_fwd_carry(const gfe_selscan_args *args, const float *h0, void *stream);
 GFE_API int gfe_selscan_bwd_carry(const gfe_selscan_args *args, const float *dlast, float *dh0, void *stream);
+/* Summaries of a whole range, for a sequence split over several devices (each device scans its own range from the state the
+ * earlier ranges leave, and backpropagates from the state gradient the later ranges send back).  Both cut [0, L) into
+ * independent segments, summarise each from a zero carry and fold the segments; they write nothing but their outputs.
+ * gfe_selscan_summary_fwd: h_loc (B, ED, N) fp32 = the final state of a scan over [0, L) started from zero (what last_state
+ *   of gfe_selscan_fwd would hold); sum_delta (B, ED) fp32 = sum over t of delta_t (softplus(delta + dt_bias) when the
+ *   flag is set, else delta + dt_bias).  Reads u, delta, Bm, A_log, dt_bias, flags; z, Cm, D, out, ckpt, last_state are
+ *   ignored.  The state after [0, L) from a state h0 is then exp(A sum_delta) h0 + h_loc.
+ * gfe_selscan_summary_bwd: g_loc (B, ED, N) fp32 = the dh0 gfe_selscan_bwd_carry returns with dlast = NULL for the same
+ *   dout.  Reads dout, z (gate, may be NULL), delta, Cm, A_log, dt_bias, flags; u, Bm, D and the gradient outputs are
+ *   ignored.  With a final-state gradient dlast, dh0 = exp(A sum_delta) dlast + g_loc.
+ * h_loc / g_loc contiguous and 16-byte aligned, sum_delta contiguous; they must not overlap.  Workspace (args->ws):
+ * gfe_selscan_summary_workspace_bytes(), one size for both directions. */
+GFE_API size_t gfe_selscan_summary_workspace_bytes(int B, int L, int ED, int N);
+GFE_API int gfe_selscan_summary_fwd(const gfe_selscan_args *args, float *h_loc, float *sum_delta, void *stream);
+GFE_API int gfe_selscan_summary_bwd(const gfe_selscan_args *args, float *g_loc, void *stream);
 
 /* ------------------------------------------------ causal depthwise conv1d --
  * u[b,t,c] = silu(bias[c] + sum_k w[c,k] xin[b, t-(K-1)+k, c]),  xin = 0 for t < 0.
